@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # our arm (CUDA, through the C ABI)
     python bench.py --impl reference --gpus N --steps K ...   # the reference's CPU algorithm (oracle port)
+    python bench.py ... --dump-outputs DIR                    # also write what the last timed step computed (.npy)
 
 One STEP = one pass of the hot path over one batch of synthetic input of the BASELINE.json
 configs[1] shape (C2): extract 100 000 fg + 100 000 bg sequences x 500 bp, k = 1..8, revcomp-merged,
@@ -98,6 +99,31 @@ def algorithmic_bytes_extract(n, L, nnz, binarize):
 def algorithmic_bytes_iter(n, m, nnz, binarize):
     """nnz (4 + v) + (n+1) 8 + n + 3 (m+1) 8 per full-space prox-grad iteration"""
     return nnz * (4 + (0 if binarize else 4)) + (n + 1) * 8 + n + 3 * (m + 1) * 8
+
+
+def dump_outputs(out_dir, data, est, sample_rows=1024, seed=0, budget=64 << 20):
+    """what one step hands its caller, as out_dir/<name>.npy in float64: the estimator's theta and the hook's loss
+    at that theta, the class list (k, code), the entry count of every row of the count matrix, and the entries of
+    a fixed, seeded sample of its rows -- as many of the sampled rows as fit in `budget` bytes in all.  The hook's
+    loss_old is left out: a step runs one iteration, so it is still the NaN that stands for "no previous loss"."""
+    rowptr, col, val = data.rows()
+    k, code = data.Kmers()
+    out = {"theta": est.Theta, "loss": est.hook_state[1:], "kmers_k": k, "kmers_code": code, "row_nnz": np.diff(rowptr)}
+    left = budget - sum(8 * len(v) for v in out.values()) - 9 * 128 - 8      # 9 .npy headers, the first row pointer
+    pick = np.random.default_rng(seed).permutation(data.n)[:sample_rows]
+    # a row costs its row index, its row pointer and 16 bytes per entry
+    cost = np.cumsum(16 + 16 * (rowptr[pick + 1] - rowptr[pick]))
+    pick = np.sort(pick[:int(np.searchsorted(cost, max(left, 0), side="right"))])
+    ent = np.concatenate([np.arange(rowptr[r], rowptr[r + 1]) for r in pick]) if len(pick) else np.zeros(0, dtype=np.int64)
+    out.update(sample_rows=pick, sample_rowptr=np.concatenate([[0], np.cumsum(rowptr[pick + 1] - rowptr[pick])]),
+               sample_col=col[ent], sample_val=val[ent])
+    out = {name: np.asarray(v, dtype=np.float64) for name, v in out.items()}
+    bad = [name for name, v in out.items() if not np.all(np.isfinite(v))]
+    if bad:
+        raise ValueError("the last timed step computed non-finite values in: " + ", ".join(bad))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v)
 
 
 def canonical_classes(n_classes, M, N, seed=5):
@@ -438,7 +464,12 @@ def main():
     ap.add_argument("--short", action="store_true", help="profiling runs only: allow fewer than 3 warm-up steps")
     ap.add_argument("--legs", default="auto", help="extra legs on the same JSON line: comma list of c3,path,path100,c4,c5; "
                     "auto = all four on one GPU, c3,c5 on several; none = headline only")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step computed as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the CUDA path computed: it needs --impl ours")
     if args.warmup < 3 and args.impl == "ours" and not args.short:
         args.warmup = 3
 
@@ -485,8 +516,8 @@ def main():
             dist.barrier()
         torch.cuda.synchronize()
 
-    def step_resident():
-        """returns (device ms, matrix info)"""
+    def step_resident(keep=False):
+        """returns (device ms, matrix info, (matrix, estimator) if keep else None: the caller frees that matrix)"""
         ms = 0.0
         data = api._extract(counter, seqs, None, None, sharded)
         ms += K.last_device_ms()
@@ -498,8 +529,10 @@ def main():
         est.estimate_proximal(data, lam)
         ms += K.last_device_ms()
         info = (data.n, data.m, data.nnz)
+        if keep:
+            return ms, info, (data, est)
         data.free()
-        return ms, info
+        return ms, info, None
 
     def step_e2e():
         """the same step through the host-buffer C-ABI calls; returns wall seconds"""
@@ -528,14 +561,18 @@ def main():
     launches0 = K.launch_count()
     dev_ms, info = [], None
     t_wall0 = time.perf_counter()
-    for _ in range(args.steps):
-        ms, info = step_resident()
+    for i in range(args.steps):
+        ms, info, last = step_resident(keep=args.dump_outputs is not None and i == args.steps - 1)
         dev_ms.append(ms)
     barrier()
     t_wall = time.perf_counter() - t_wall0
     launches = K.launch_count() - launches0
     prof = K.api.profile_dump()
     K.api.profile(False)
+    if last is not None:
+        if rank == 0:
+            dump_outputs(args.dump_outputs, *last)
+        last[0].free()
 
     # full-space prox-grad iterations back to back on a resident matrix
     data = api._extract(counter, seqs, None, None, sharded)
@@ -588,7 +625,7 @@ def main():
 
     # e2e through host buffers
     e2e_s = []
-    for i in range(2 + max(3, args.steps)):          # 2 untimed (the arena settles), then the timed ones
+    for i in range(2 + args.steps):                  # 2 untimed (the arena settles), then the timed ones
         dt, m_e2e, _ = step_e2e()
         if i > 1:
             e2e_s.append(dt)

@@ -1,17 +1,19 @@
 """Generates tests/golden/ref_fixtures.npz from the reference's own test fixtures.
 
-Run in the dev container (needs /root/reference, which does not exist on the GPU box):
-    python tests/golden/make_fixtures.py
+It needs a checkout of the reference (pbenner/kmerLr), which the tests themselves do not:
+    python tests/golden/make_fixtures.py <reference checkout>
 The fixtures are DATA (FASTA sequences and score tables the reference's tests read,
 kmerLr_test.go / scoresLr_test.go), stored as uint8 / float64 arrays.  The golden numbers
-those tests assert are transcribed, with file:line, in golden_vectors.json.
+those tests assert are transcribed, with file:line, in tests/test_oracle_golden.py.
 """
 import os
 import sys
 
 import numpy as np
 
-REF = sys.argv[1] if len(sys.argv) > 1 else "/root/reference"
+if len(sys.argv) != 2:
+    sys.exit(__doc__)
+REF = sys.argv[1]
 OUT = os.path.join(os.path.dirname(os.path.abspath(__file__)), "ref_fixtures.npz")
 
 
