@@ -60,6 +60,18 @@ void arena_release_all() {
   g_free_blocks.clear();
 }
 
+void *host_staging(size_t bytes) {
+  KL_CUDA(cudaEventSynchronize(g_ctx.staging_ev));
+  if (bytes > g_ctx.staging_bytes) {
+    if (g_ctx.staging) KL_CUDA(cudaFreeHost(g_ctx.staging));
+    g_ctx.staging = nullptr; g_ctx.staging_bytes = 0;
+    const size_t want = (bytes + ARENA_GRAIN - 1) / ARENA_GRAIN * ARENA_GRAIN;
+    KL_CUDA(cudaMallocHost(&g_ctx.staging, want));
+    g_ctx.staging_bytes = want;
+  }
+  return g_ctx.staging;
+}
+
 // ---- per-kernel profiling ---------------------------------------------------------------------------
 namespace {
 struct ProfRec { std::string name; cudaEvent_t e0, e1; };
@@ -223,6 +235,7 @@ int kmerlr_init(int device) {
 
     KL_CUDA(cudaEventCreate(&g_ctx.ev0));
     KL_CUDA(cudaEventCreate(&g_ctx.ev1));
+    KL_CUDA(cudaEventCreateWithFlags(&g_ctx.staging_ev, cudaEventDisableTiming));
     g_ctx.ready = true;
   }, false);
 }
@@ -235,6 +248,8 @@ int kmerlr_shutdown(void) {
       arena_release_all();
       comm_destroy();
       cudaEventDestroy(g_ctx.ev0); cudaEventDestroy(g_ctx.ev1);
+      cudaEventDestroy(g_ctx.staging_ev);
+      if (g_ctx.staging) cudaFreeHost(g_ctx.staging);
       cudaStreamSynchronize(g_ctx.copy_stream);
       for (int i = 0; i < CTX_COPY_EVENTS; i++) cudaEventDestroy(g_ctx.copy_ev[i]);
       cudaStreamDestroy(g_ctx.copy_stream);

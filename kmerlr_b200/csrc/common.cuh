@@ -72,6 +72,7 @@ struct PeerBox {
 };
 
 constexpr int CTX_COPY_EVENTS = 11;   // chunks of a pipelined host feed + 1
+struct Numbering;
 struct Ctx {
   bool ready = false;
   int device = 0;
@@ -82,6 +83,12 @@ struct Ctx {
   cudaEvent_t join_ev[2] = {nullptr, nullptr};
   cudaEvent_t copy_ev[CTX_COPY_EVENTS] = {nullptr};
   cudaEvent_t ev0 = nullptr, ev1 = nullptr;
+  // pinned host staging of the small per-call transfers (labels, theta, iteration state): see host_staging()
+  void *staging = nullptr;
+  size_t staging_bytes = 0;
+  cudaEvent_t staging_ev = nullptr;              // recorded after the last transfer that used the staging buffer
+  // numbering sets of every class a configuration can produce, one per (M, N, strand op) seen (extract.cu)
+  std::vector<std::shared_ptr<const Numbering>> numbering;
   int64_t launches = 0;
   double last_ms = 0.0;
   bool profiling = false;
@@ -122,6 +129,13 @@ void profile_end();
   } while (0)
 
 inline void sync_stream() { KL_CUDA(cudaStreamSynchronize(ctx().stream)); }
+
+// Pinned host buffer of at least `bytes` (grown on demand, owned by the context) for copies on ctx().stream:
+// copies from and to pageable memory stage through a driver buffer and block the host.  The caller records
+// the end of its copies with host_staging_done(); the next host_staging() waits for them before it hands the
+// buffer out again.
+void *host_staging(size_t bytes);
+inline void host_staging_done() { KL_CUDA(cudaEventRecord(ctx().staging_ev, ctx().stream)); }
 
 // KMERLR_TRACE=1: host-side phase timestamps on stderr (where does a call spend its wall time)
 struct Trace {
@@ -218,6 +232,18 @@ enum ValType : int { VAL_ONE = 0, VAL_U32 = 1, VAL_F64 = 2 };
 //   * binarized matrices: the table levels (k <= 5, where nearly every class repeats) are a per-row bitmap
 //     over the classes of those levels (lowbits), the levels k >= 6 are matrix-free with one correction per
 //     REPEAT of a class inside a row (the events the extraction leaves at the tail of the row's slots).
+// The numbering set of an extraction: the classes that get a column (column = rank of the class among them) as a
+// bitmap over the dense class ids, the rank of every word's first bit (rank[nw] = count), and both interleaved for
+// the extraction kernel.  Never changed once built: the set of every class of an unfrozen configuration depends
+// on (M, N, strand op) only, so the context keeps one per configuration and the matrices share it.
+struct Numbering {
+  int M = 0, N = 0, op = 0;
+  int64_t nw = 0;
+  uint32_t count = 0;
+  DevBuf<uint32_t> bits, rank;     // nw, nw + 1
+  DevBuf<uint2> nbx;               // nw (empty for the observed-class sets of a renumbered matrix)
+};
+
 constexpr int IMP_MAX_N = 10;      // forward-code tables of 4^1 + ... + 4^N entries
 constexpr int IMP_SUPER_MAX = 11;  // longest "super k-mer" table (4^11 entries of 8 bytes = 32 MB)
 constexpr uint32_t NOCOL = 0xFFFFFFFFu;
@@ -227,7 +253,7 @@ struct Implicit {
   int Mlo = 0;                     // first matrix-free level (>= M)
   uint32_t level_off[16] = {0};    // dense class id of (k, code 0)
   uint32_t fo[16] = {0};           // offset of level j (Mlo..N) in the forward-code tables, fo[N+1] = total
-  DevBuf<uint32_t> bitmap, rank;   // class set over dense ids: column = rank[id>>5] + popc(bits below)
+  std::shared_ptr<const Numbering> num;   // class set over dense ids: column = rank[id>>5] + popc(bits below)
   // binarized matrices only
   bool binarized = false;
   int low_words = 0;               // 32-bit words of a row's bitmap over the table-level classes
@@ -296,6 +322,8 @@ struct Matrix : Object {
   DevBuf<uint8_t> labels;    // n
   int64_t n_pos = 0, n_neg = 0;   // label counts: this rank's until matrix_label_counts() has summed them over the ranks
   bool counts_global = true;
+  bool counts_pending = false;    // n_pos is still on the device (label_ones), read when somebody needs the counts
+  DevBuf<unsigned long long> label_ones;
   // class list: dense class ids on the device (extraction), decoded to (k, code) on the host the first
   // time somebody asks (matrix_class_list)
   int64_t n_classes = 0;
@@ -363,6 +391,7 @@ std::shared_ptr<Matrix> matrix_from_csr(int64_t n, int64_t m, const int64_t *row
                                         const double *val, int flags);
 void matrix_rows(Matrix &M, int64_t *rowptr, int32_t *col, double *val);
 void matrix_set_labels(Matrix &M, const uint8_t *labels, int64_t n);
+void matrix_label_counts_local(Matrix &M);   // n_pos / n_neg of this rank's rows on the host
 void matrix_label_counts(Matrix &M);   // n_pos / n_neg over all ranks (collective on a sharded matrix, first call only)
 void matrix_column_moments(Matrix &M, double *sum, double *sumsq, double *absmax, int64_t *count);
 void matrix_pair_moments(Matrix &M, double *sum, double *sumsq, double *absmax, int64_t *count);   // m (m - 1) / 2 pairs

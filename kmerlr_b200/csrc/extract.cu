@@ -146,10 +146,22 @@ __global__ void interleave_numbering(const uint32_t *__restrict__ bits, const ui
   int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (w < nw) out[w] = make_uint2(bits[w], rank[w]);
 }
-__global__ void bitmaps_differ(const uint32_t *__restrict__ a, const uint32_t *__restrict__ b, int64_t nw,
-                               uint32_t *__restrict__ flag) {
-  int64_t w = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (w < nw && a[w] != b[w]) atomicOr(flag, 1u);
+// after the extraction kernel: tot[0] += the stored entries (sum of the row counts), tot[3] = 1 if the observed
+// classes a differ from the numbering set b (b == nullptr: no check)
+__global__ void extract_totals(const uint32_t *__restrict__ rowcnt, int64_t n, const uint32_t *__restrict__ a,
+                               const uint32_t *__restrict__ b, int64_t nw, unsigned long long *__restrict__ tot) {
+  __shared__ unsigned long long sh;
+  if (threadIdx.x == 0) sh = 0ull;
+  __syncthreads();
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x, i0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  unsigned long long s = 0ull;
+  for (int64_t i = i0; i < n; i += stride) s += rowcnt[i];
+  if (b)
+    for (int64_t w = i0; w < nw; w += stride)
+      if (a[w] != b[w]) tot[3] = 1ull;
+  if (s) atomicAdd(&sh, s);
+  __syncthreads();
+  if (threadIdx.x == 0 && sh) atomicAdd(tot, sh);
 }
 // columns numbered in the numbering set -> ranks among the observed classes, in place (warp per row)
 __global__ void renumber_rows(uint32_t *__restrict__ col, const uint32_t *__restrict__ rowcnt, int64_t stride, int64_t n,
@@ -456,6 +468,31 @@ static std::shared_ptr<Matrix> apply_features(Matrix &cls, const int32_t *featur
   return out;
 }
 
+// rank, count and interleaved words of a numbering set whose bits are in place
+static void number_set(Numbering &S) {
+  const int64_t nw = S.nw;
+  DevBuf<uint32_t> pc((size_t)nw);
+  KL_LAUNCH(popc_words, (unsigned)((nw + 255) / 256), 256, 0, S.bits.p, nw, pc.p);
+  exclusive_scan_u32(pc.p, S.rank.p, nw);
+  S.nbx.alloc((size_t)nw);
+  KL_LAUNCH(interleave_numbering, (unsigned)((nw + 255) / 256), 256, 0, S.bits.p, S.rank.p, nw, S.nbx.p);
+}
+
+// every class the configuration can produce, built once per (M, N, strand op) and kept by the context
+static std::shared_ptr<const Numbering> numbering_all(const LevelInfo &LI, int64_t nw) {
+  for (auto &s : ctx().numbering)
+    if (s->M == LI.M && s->N == LI.N && s->op == LI.op) return s;
+  auto S = std::make_shared<Numbering>();
+  S->M = LI.M; S->N = LI.N; S->op = LI.op; S->nw = nw;
+  S->bits.alloc((size_t)nw); S->rank.alloc((size_t)nw + 1);
+  KL_LAUNCH(all_classes_bits, (unsigned)((nw + 255) / 256), 256, 0, LI, S->bits.p, nw);
+  number_set(*S);
+  KL_CUDA(cudaMemcpyAsync(&S->count, S->rank.p + nw, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx().stream));
+  sync_stream();
+  ctx().numbering.push_back(S);
+  return S;
+}
+
 static std::shared_ptr<Matrix> extract_impl(const kmerlr_config &cfg, std::shared_ptr<SeqSet> seqs,
                                             const int32_t *frozen_k, const uint64_t *frozen_code, int64_t n_frozen,
                                             const int32_t *features, int64_t n_features, int flags, HostFeed *feed) {
@@ -563,11 +600,12 @@ static std::shared_ptr<Matrix> extract_impl(const kmerlr_config &cfg, std::share
   DevBuf<uint32_t> dummy_cnt(1);
   // numbering set: the frozen list, or every class the configuration can produce (then the columns
   // are final unless some class never shows up, see below)
-  DevBuf<uint32_t> nb((size_t)nw), nbrank((size_t)nw + 1), pc((size_t)nw), bitmap((size_t)nw);
+  DevBuf<uint32_t> bitmap((size_t)nw);
   std::vector<uint32_t> frozen_bits;       // host image of the frozen class set (alive until the next sync)
   LevelInfo LI{};
   LI.M = cfg.M; LI.N = cfg.N; LI.op = P.op;
   for (int k = cfg.M; k <= cfg.N + 1; k++) LI.level_off[k] = P.level_off[k];
+  std::shared_ptr<const Numbering> num;
   if (n_frozen > 0) {
     frozen_bits.assign((size_t)nw, 0u);
     uint64_t prev = 0;
@@ -579,22 +617,25 @@ static std::shared_ptr<Matrix> extract_impl(const kmerlr_config &cfg, std::share
       prev = id;
       frozen_bits[id >> 5] |= 1u << (id & 31);
     }
-    nb.upload(frozen_bits.data(), (size_t)nw);
+    auto F = std::make_shared<Numbering>();
+    F->M = cfg.M; F->N = cfg.N; F->op = P.op; F->nw = nw; F->count = (uint32_t)n_frozen;
+    F->bits.alloc((size_t)nw); F->rank.alloc((size_t)nw + 1);
+    F->bits.upload(frozen_bits.data(), (size_t)nw);
+    number_set(*F);
+    num = F;
   } else {
-    KL_LAUNCH(all_classes_bits, (unsigned)((nw + 255) / 256), 256, 0, LI, nb.p, nw);
+    num = numbering_all(LI, nw);
   }
-  KL_LAUNCH(popc_words, (unsigned)((nw + 255) / 256), 256, 0, nb.p, nw, pc.p);
-  exclusive_scan_u32(pc.p, nbrank.p, nw);
+  // one zeroed block for everything the host reads after the kernel: [0] stored entries, [1, 2] row statistics,
+  // [3] "observed classes differ from the numbering set", [4] repeat events, [6, 9) the sharded exchange's totals
+  DevBuf<unsigned long long> tot(9);
+  tot.zero();
   bitmap.zero();
   DevBuf<uint32_t> full(1);                 // "every class has been observed" (set by the kernel, ends the marks)
   full.zero();
   P.full = full.p; P.nb_words = nw;
-  DevBuf<unsigned long long> stats(2);
-  stats.zero();
   P.st_id = out->col.p; P.st_cnt = P.binarize ? dummy_cnt.p : out->val_u32.p; P.rowcnt = out->rowcnt.p;
-  DevBuf<uint2> nbx((size_t)nw);
-  KL_LAUNCH(interleave_numbering, (unsigned)((nw + 255) / 256), 256, 0, nb.p, nbrank.p, nw, nbx.p);
-  P.bitmap = bitmap.p; P.nbx = nbx.p; P.filter = n_frozen > 0; P.stats = stats.p;
+  P.bitmap = bitmap.p; P.nbx = num->nbx.p; P.filter = n_frozen > 0; P.stats = tot.p + 1;
   P.mark = n_frozen == 0;
   DevBuf<uint32_t> lowbits, rowdup;
   if (hybrid) {
@@ -661,38 +702,40 @@ static std::shared_ptr<Matrix> extract_impl(const kmerlr_config &cfg, std::share
   tr.mark("extract_kernel");
   // observed classes, row count and row statistics of all ranks in ONE exchange; do the classes cover the
   // numbering set?
-  DevBuf<uint32_t> differ(1);
-  differ.zero();
-  DevBuf<unsigned long long> gres(3);
+  unsigned long long *const gres = tot.p + 6;
   if (sharded) {
     const int64_t xw = n_frozen == 0 ? nw : 0, per = xw + 6;
     DevBuf<uint32_t> mine((size_t)per), all((size_t)(per * ctx().world));
-    KL_LAUNCH(pack_exchange, (unsigned)((xw + 256) / 256), 256, 0, bitmap.p, xw, (unsigned long long)s.n, stats.p, mine.p);
+    KL_LAUNCH(pack_exchange, (unsigned)((xw + 256) / 256), 256, 0, bitmap.p, xw, (unsigned long long)s.n, tot.p + 1, mine.p);
     comm_allgather_bytes(mine.p, all.p, per * 4);
-    KL_LAUNCH(merge_exchange, (unsigned)((xw + 256) / 256), 256, 0, all.p, ctx().world, xw, bitmap.p, gres.p);
+    KL_LAUNCH(merge_exchange, (unsigned)((xw + 256) / 256), 256, 0, all.p, ctx().world, xw, bitmap.p, gres);
   }
-  if (n_frozen == 0)
-    KL_LAUNCH(bitmaps_differ, (unsigned)((nw + 255) / 256), 256, 0, bitmap.p, nb.p, nw, differ.p);
-  // one round trip: classes, stored entries, "columns are final", row statistics, global number of rows
-  DevBuf<int64_t> rp((size_t)s.n + 1);
-  if (s.n > 0) exclusive_scan_u32_to_i64(out->rowcnt.p, rp.p, s.n); else rp.zero();
-  int64_t nn = s.n;
-  unsigned long long hres[3] = {0, 0, 0};
-  if (sharded) gres.download(hres, 3);
-  uint32_t m32 = 0, hdiffer = 0;
-  unsigned long long hstats[2] = {0, 0};
+  {
+    int64_t blocks = ((s.n > nw ? s.n : nw) + 255) / 256;
+    if (blocks > 4 * ctx().sm_count) blocks = 4 * ctx().sm_count;
+    KL_LAUNCH(extract_totals, (unsigned)(blocks ? blocks : 1), 256, 0, out->rowcnt.p, s.n, bitmap.p,
+              n_frozen == 0 ? num->bits.p : (const uint32_t *)nullptr, nw, tot.p);
+  }
   DevBuf<int64_t> evptr;
-  int64_t n_events = 0;
   if (hybrid) {
     evptr.alloc((size_t)s.n + 1);
     exclusive_scan_u32_to_i64(rowdup.p, evptr.p, s.n);
-    KL_CUDA(cudaMemcpyAsync(&n_events, evptr.p + s.n, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx().stream));
+    KL_CUDA(cudaMemcpyAsync(tot.p + 4, evptr.p + s.n, sizeof(int64_t), cudaMemcpyDeviceToDevice, ctx().stream));
   }
-  KL_CUDA(cudaMemcpyAsync(&m32, nbrank.p + nw, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx().stream));
-  KL_CUDA(cudaMemcpyAsync(&out->nnz, rp.p + s.n, sizeof(int64_t), cudaMemcpyDeviceToHost, ctx().stream));
-  differ.download(&hdiffer, 1);
-  stats.download(hstats, 2);
+  // the class list of the numbering set goes out before the one round trip (a renumbering below redoes it)
+  uint32_t m32 = num->count;
+  out->class_ids.alloc((size_t)(m32 ? m32 : 1));
+  KL_LAUNCH(enumerate_bits, (unsigned)((nw + 255) / 256), 256, 0, num->bits.p, num->rank.p, nw, out->class_ids.p);
+  // one round trip: stored entries, "columns are final", row statistics, repeat events, global number of rows
+  unsigned long long *htot = (unsigned long long *)host_staging(9 * sizeof(unsigned long long));
+  tot.download(htot, 9);
+  host_staging_done();
   sync_stream();
+  out->nnz = (int64_t)htot[0];
+  const unsigned long long hstats[2] = {htot[1], htot[2]}, hres[3] = {htot[6], htot[7], htot[8]};
+  const bool hdiffer = htot[3] != 0;
+  const int64_t n_events = (int64_t)htot[4];
+  int64_t nn = s.n;
   if (sharded) {
     // the statistics are global already: no collective later (step size, fixed-point scale)
     nn = (int64_t)hres[0];
@@ -706,23 +749,29 @@ static std::shared_ptr<Matrix> extract_impl(const kmerlr_config &cfg, std::share
   if (hdiffer) {
     // some class of the configuration never occurs: the columns are the ranks among the OBSERVED
     // classes (kmerLr_data.go:316-324), renumber the stored columns in place
-    DevBuf<uint32_t> rank2((size_t)nw + 1), ids_nb((size_t)(m32 ? m32 : 1));
-    KL_LAUNCH(popc_words, (unsigned)((nw + 255) / 256), 256, 0, bitmap.p, nw, pc.p);
-    exclusive_scan_u32(pc.p, rank2.p, nw);
-    KL_LAUNCH(enumerate_bits, (unsigned)((nw + 255) / 256), 256, 0, nb.p, nbrank.p, nw, ids_nb.p);
+    auto obs = std::make_shared<Numbering>();
+    obs->M = cfg.M; obs->N = cfg.N; obs->op = P.op; obs->nw = nw;
+    obs->rank.alloc((size_t)nw + 1);
+    {
+      DevBuf<uint32_t> pc((size_t)nw);
+      KL_LAUNCH(popc_words, (unsigned)((nw + 255) / 256), 256, 0, bitmap.p, nw, pc.p);
+      exclusive_scan_u32(pc.p, obs->rank.p, nw);
+    }
     if (s.n > 0)
-      KL_LAUNCH(renumber_rows, (unsigned)((s.n * 32 + 127) / 128), 128, 0, out->col.p, out->rowcnt.p, stride, s.n, ids_nb.p,
-                bitmap.p, rank2.p, hybrid ? rowdup.p : (const uint32_t *)nullptr);
-    KL_CUDA(cudaMemcpyAsync(&m32, rank2.p + nw, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx().stream));
+      KL_LAUNCH(renumber_rows, (unsigned)((s.n * 32 + 127) / 128), 128, 0, out->col.p, out->rowcnt.p, stride, s.n,
+                out->class_ids.p, bitmap.p, obs->rank.p, hybrid ? rowdup.p : (const uint32_t *)nullptr);
+    KL_CUDA(cudaMemcpyAsync(&obs->count, obs->rank.p + nw, sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx().stream));
     sync_stream();
-    nb = std::move(bitmap); nbrank = std::move(rank2);
+    obs->bits = std::move(bitmap);
+    m32 = obs->count;
+    num = obs;
+    out->class_ids.alloc((size_t)(m32 ? m32 : 1));
+    KL_LAUNCH(enumerate_bits, (unsigned)((nw + 255) / 256), 256, 0, num->bits.p, num->rank.p, nw, out->class_ids.p);
     tr.mark("renumber");
   }
   out->m = (int64_t)m32;
   // class list: dense ids stay on the device, (k, code) pairs are decoded on demand
   out->n_classes = (int64_t)m32;
-  out->class_ids.alloc((size_t)(m32 ? m32 : 1));
-  KL_LAUNCH(enumerate_bits, (unsigned)((nw + 255) / 256), 256, 0, nb.p, nbrank.p, nw, out->class_ids.p);
   out->class_M = cfg.M; out->class_N = cfg.N; out->classes_on_host = false;
   for (int k = cfg.M; k <= cfg.N + 1; k++) out->class_level_off[k] = P.level_off[k];
   if (n_features > 0) { sync_stream(); return apply_features(*out, features, n_features); }
@@ -742,14 +791,14 @@ static std::shared_ptr<Matrix> extract_impl(const kmerlr_config &cfg, std::share
       imp->low_words = P.low_words;
       imp->lowcol.alloc((size_t)(P.low_words ? P.low_words * 32 : 1));
       if (P.low_words)
-        KL_LAUNCH(low_columns, (unsigned)((P.low_words * 32 + 127) / 128), 128, 0, P.tl, P.tl_cnt, P.low_words * 32, nb.p,
-                  nbrank.p, imp->lowcol.p);
+        KL_LAUNCH(low_columns, (unsigned)((P.low_words * 32 + 127) / 128), 128, 0, P.tl, P.tl_cnt, P.low_words * 32,
+                  num->bits.p, num->rank.p, imp->lowcol.p);
       imp->lowbits = std::move(lowbits);
       imp->events.alloc((size_t)(n_events ? n_events : 1));
       KL_LAUNCH(gather_events, (unsigned)((s.n * 32 + 127) / 128), 128, 0, out->col.p, stride, s.n, evptr.p, imp->events.p);
       imp->evptr = std::move(evptr);
     }
-    imp->bitmap = std::move(nb); imp->rank = std::move(nbrank);
+    imp->num = num;
     out->imp = imp;
   }
   sync_stream();

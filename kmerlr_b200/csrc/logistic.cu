@@ -263,15 +263,45 @@ __global__ void imp_build_TS(const ImpParams P, double *__restrict__ T, const Pg
   T[P.sup0 + U] = s;
 }
 
-// H[N][N-mer at offset t of U] += HS[U]
-__global__ void imp_fold_super(const ImpParams P, unsigned long long *__restrict__ H, const PgState *st) {
+// The fold of the forward-code tables after the pass, F_j[u] = H_j[u] + F_{j+1}[4u .. 4u+3] from level N-1 down to
+// Mlo, preceded by H[N][N-mer at offset t of U] += HS[U] when there is a super level.  The grid of one launch folds
+// `level` (P.N: the super level into level N) -- the large steps, one launch each; the block that finishes last then
+// folds the levels tail_top .. Mlo (at most 4^IMP_FOLD_TAIL entries each) in place of one launch per level.  The
+// integer sums are exact, so the order does not matter.  `ticket` is zero on entry and left zero.
+constexpr int IMP_FOLD_TAIL = 7;
+constexpr int IMP_FOLD_THREADS = 1024;
+__global__ void __launch_bounds__(IMP_FOLD_THREADS) imp_fold(const ImpParams P, int level, int tail_top,
+                                                             unsigned long long *__restrict__ H, unsigned int *ticket,
+                                                             const PgState *st) {
   if (st && st->done == 1) return;
-  const uint32_t U = blockIdx.x * blockDim.x + threadIdx.x;
-  if (U >= (1u << (2 * P.S))) return;
-  const unsigned long long h = H[P.sup0 + U];
-  if (!h) return;
-  const uint32_t maskN = (1u << (2 * P.N)) - 1u;
-  for (int t = 0; t < P.c; t++) atomicAdd(H + P.fo[P.N] + ((U >> (2 * (P.S - P.N - t))) & maskN), h);
+  const uint32_t u = blockIdx.x * blockDim.x + threadIdx.x;
+  if (level == P.N) {
+    if (u < (1u << (2 * P.S))) {
+      const unsigned long long h = H[P.sup0 + u];
+      const uint32_t maskN = (1u << (2 * P.N)) - 1u;
+      if (h)
+        for (int t = 0; t < P.c; t++) atomicAdd(H + P.fo[P.N] + ((u >> (2 * (P.S - P.N - t))) & maskN), h);
+    }
+  } else if (level >= P.Mlo && u < (1u << (2 * level))) {
+    const unsigned long long *c = H + P.fo[level + 1] + 4ull * u;
+    H[P.fo[level] + u] += c[0] + c[1] + c[2] + c[3];
+  }
+  if (tail_top < P.Mlo) return;
+  __shared__ int s_last;
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) s_last = atomicAdd(ticket, 1u) == gridDim.x - 1 ? 1 : 0;
+  __syncthreads();
+  if (!s_last) return;
+  __threadfence();
+  for (int j = tail_top; j >= P.Mlo; j--) {
+    for (uint32_t v = threadIdx.x; v < (1u << (2 * j)); v += blockDim.x) {   // (L2 reads: other blocks wrote there)
+      const unsigned long long *c = H + P.fo[j + 1] + 4ull * v;
+      H[P.fo[j] + v] = __ldcg(H + P.fo[j] + v) + __ldcg(c) + __ldcg(c + 1) + __ldcg(c + 2) + __ldcg(c + 3);
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) *ticket = 0u;
 }
 
 // binarized rows: lowtab[(i * 16 + v) * lwp + l] = sum of theta over the classes (l * 32 + 4 i + b) with bit b
@@ -580,23 +610,10 @@ __global__ void __launch_bounds__(256) low_accumulate(const uint32_t *__restrict
   }
 }
 
-// F_j[u] = H_j[u] + F_{j+1}[4u .. 4u+3], in place, one launch per level from N-1 down to Mlo
-__global__ void imp_fold_level(const ImpParams P, int j, unsigned long long *__restrict__ H, const PgState *st) {
-  if (st && st->done == 1) return;
-  const uint32_t u = blockIdx.x * blockDim.x + threadIdx.x;
-  if (u >= (1u << (2 * j))) return;
-  const unsigned long long *c = H + P.fo[j + 1] + 4ull * u;
-  H[P.fo[j] + u] += c[0] + c[1] + c[2] + c[3];
-}
-
-// G[col + 1] += F_k[code] + F_k[image(code)] for the columns of the matrix-free levels (G holds the repeat
+// G[col + 1] += F_k[code] + F_k[image(code)] for column j if it is one of the matrix-free levels (G holds the repeat
 // corrections of binarized rows by now, zero otherwise)
-__global__ void imp_columns(const ImpParams P, const uint32_t *__restrict__ col_id, int64_t m,
-                            const unsigned long long *__restrict__ F, unsigned long long *__restrict__ G,
-                            const PgState *st) {
-  if (st && st->done == 1) return;
-  const int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (j >= m) return;
+__device__ __forceinline__ void imp_column(const ImpParams &P, const uint32_t *__restrict__ col_id, int64_t j,
+                                           const unsigned long long *__restrict__ F, unsigned long long *__restrict__ G) {
   const uint32_t id = col_id[j];
   int k = P.M;
   while (k < P.N && id >= P.level_off[k + 1]) k++;
@@ -753,42 +770,17 @@ __global__ void pack_loss_slots(const PgState *st, const double *__restrict__ lo
   const int r = threadIdx.x;
   if (r < world) slots[r] = r == rank ? (unsigned long long)__double_as_longlong(local[0]) : 0ull;
 }
-__global__ void unpack_loss_slots(const PgState *st, const unsigned long long *__restrict__ slots, int world,
-                                  double *__restrict__ out) {
-  if (st && st->done == 1) return;
-  if (threadIdx.x == 0) {
-    double s = 0.0;
-    for (int r = 0; r < world; r++) s += __longlong_as_double((long long)slots[r]);
-    out[0] = s;
-  }
-}
 
-// hook (kmerLr_estimator_hook.go:46-99): loss = mean + lambda * sum_{j=1..m} |theta_j|
-// l1part[b] = sum over block b's stride of lambda |theta_j|, j >= 1 (fixed order: deterministic)
-__global__ void l1_partials(const PgState *st, const double *__restrict__ theta, int64_t ntheta, double lambda,
-                            double *__restrict__ l1part) {
-  if (st && st->done == 1) return;
-  __shared__ double sh[256];
-  double s = 0.0;
-  if (!isnan(lambda) && lambda != 0.0)
-    for (int64_t j = 1 + (int64_t)blockIdx.x * blockDim.x + threadIdx.x; j < ntheta; j += (int64_t)gridDim.x * blockDim.x)
-      s += lambda * fabs(theta[j]);
-  sh[threadIdx.x] = s;
-  __syncthreads();
-  for (int o = 128; o > 0; o >>= 1) {
-    if ((int)threadIdx.x < o) sh[threadIdx.x] += sh[threadIdx.x + o];
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) l1part[blockIdx.x] = sh[0];
-}
-__global__ void hook_kernel(PgState *st, const double *__restrict__ losssum, const double *__restrict__ l1part, int nparts,
-                            double inv_n, double eps_loss) {
-  if (st->done == 1) return;
+// hook (kmerLr_estimator_hook.go:46-99): loss = mean + lambda * sum_{j=1..m} |theta_j|, run by one warp.  losssum:
+// the sum of the loss terms (lane 0); l1part[b] = sum over block b's stride of lambda |theta_j|, j >= 1, added up
+// in a fixed order (deterministic)
+__device__ __forceinline__ void hook_warp(PgState *st, double losssum, const double *l1part, int nparts, double inv_n,
+                                          double eps_loss) {
   double l1 = 0.0;
-  for (int b = threadIdx.x; b < nparts; b += 32) l1 += l1part[b];
+  for (int b = (int)lane_id(); b < nparts; b += 32) l1 += __ldcg(l1part + b);
   l1 = warp_sum_down(l1);
-  if (threadIdx.x == 0) {
-    double l = losssum[0] * inv_n + l1;
+  if (lane_id() == 0) {
+    double l = losssum * inv_n + l1;
     st->lossval = l;
     if (st->first) { st->first = 0; return; }   // loss at the start point: no hook call yet
     double t = st->loss_old; st->loss_old = st->loss_new; st->loss_new = t;
@@ -800,13 +792,83 @@ __global__ void hook_kernel(PgState *st, const double *__restrict__ losssum, con
   }
 }
 
-// theta <- prox(theta - s g), eval_stopping (kmerLr_estimator_proximal.go:30-52,88-98).
-// prox_update: grid-wide update + per-block max |theta|, max |delta|; prox_finish: the decision.
-__global__ void prox_update(const PgState *st, double *__restrict__ theta, const unsigned long long *__restrict__ G,
+// the loss sums of the ranks in rank order, then the hook (one warp)
+__global__ void unpack_loss_hook(PgState *st, const unsigned long long *__restrict__ slots, int world,
+                                 double *__restrict__ out, const double *l1part, int nparts, double inv_n, double eps_loss) {
+  if (st->done == 1) return;
+  double s = 0.0;
+  if (threadIdx.x == 0) {
+    for (int r = 0; r < world; r++) s += __longlong_as_double((long long)slots[r]);
+    out[0] = s;
+  }
+  hook_warp(st, s, l1part, nparts, inv_n, eps_loss);
+}
+
+// sum of v over the 256 threads of the block in a fixed tree (deterministic); the result is valid in thread 0
+__device__ __forceinline__ double block_sum_256(double *sh, double v) {
+  sh[threadIdx.x] = v;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if ((int)threadIdx.x < o) sh[threadIdx.x] += sh[threadIdx.x + o];
+    __syncthreads();
+  }
+  const double r = sh[0];
+  __syncthreads();
+  return r;
+}
+
+// The tail of a pass, one launch of RED_BLOCKS x 256 threads: the columns of the matrix-free levels (F != nullptr:
+// a gradient pass over the forward-code tables), the block's partial sum of the loss terms (a fixed grid over
+// strided elements) and the block's partial sum of lambda |theta_j|.  The block that finishes last adds the loss
+// partials (one warp, lane l the partials l, l + 32, ..., then a fixed shuffle tree) into losssum[0] and, unless
+// the loss sums of the ranks have to be exchanged first (hook = 0), runs the hook.  `ticket` is zero on entry and
+// left zero.
+__global__ void __launch_bounds__(256) pass_tail(PgState *st, const ImpParams P, const uint32_t *__restrict__ col_id,
+                                                 int64_t m, const unsigned long long *__restrict__ F,
+                                                 unsigned long long *__restrict__ G, const double *__restrict__ lossterm,
+                                                 int64_t n, double *__restrict__ part, double *__restrict__ losssum,
+                                                 const double *__restrict__ theta, int64_t ntheta, double lambda,
+                                                 double *__restrict__ l1part, int hook, double inv_n, double eps_loss,
+                                                 unsigned int *ticket) {
+  if (st && st->done == 1) return;
+  __shared__ double sh[256];
+  __shared__ int s_last;
+  const int64_t stride = (int64_t)gridDim.x * blockDim.x, i0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (F)
+    for (int64_t j = i0; j < m; j += stride) imp_column(P, col_id, j, F, G);
+  double s = 0.0;
+  for (int64_t i = i0; i < n; i += stride) s += lossterm[i];
+  s = block_sum_256(sh, s);
+  if (threadIdx.x == 0) part[blockIdx.x] = s;
+  double l1 = 0.0;
+  if (!isnan(lambda) && lambda != 0.0)
+    for (int64_t j = 1 + i0; j < ntheta; j += stride) l1 += lambda * fabs(theta[j]);
+  l1 = block_sum_256(sh, l1);
+  if (threadIdx.x == 0) l1part[blockIdx.x] = l1;
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) s_last = atomicAdd(ticket, 1u) == gridDim.x - 1 ? 1 : 0;
+  __syncthreads();
+  if (!s_last) return;
+  __threadfence();
+  if (threadIdx.x < 32) {
+    double t = 0.0;
+    for (int i = threadIdx.x; i < (int)gridDim.x; i += 32) t += __ldcg(part + i);
+    t = warp_sum_down(t);
+    if (threadIdx.x == 0) { losssum[0] = t; *ticket = 0u; }
+    if (hook) hook_warp(st, t, l1part, (int)gridDim.x, inv_n, eps_loss);
+  }
+}
+
+// theta <- prox(theta - s g), eval_stopping (kmerLr_estimator_proximal.go:30-52,88-98): a grid-wide update with
+// per-block max |theta|, max |delta| and NaN flag; the block that finishes last takes the decision.  `ticket` is
+// zero on entry and left zero.
+__global__ void prox_update(PgState *st, double *__restrict__ theta, const unsigned long long *__restrict__ G,
                             double inv_scale, int64_t ntheta, double step, double lambda,
-                            double *__restrict__ blockmax) {
+                            double *__restrict__ blockmax, double eps, long long max_iter, unsigned int *ticket) {
   if (st->done) return;
   __shared__ double shx[256], shd[256], shn[256];
+  __shared__ int s_last;
   double mx = 0.0, md = 0.0, nn = 0.0;
   for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < ntheta; k += (int64_t)gridDim.x * blockDim.x) {
     double g = (double)(long long)G[k] * inv_scale;
@@ -831,12 +893,15 @@ __global__ void prox_update(const PgState *st, double *__restrict__ theta, const
     __syncthreads();
   }
   if (threadIdx.x == 0) { blockmax[3 * blockIdx.x] = shx[0]; blockmax[3 * blockIdx.x + 1] = shd[0]; blockmax[3 * blockIdx.x + 2] = shn[0]; }
-}
-__global__ void prox_finish(PgState *st, const double *__restrict__ blockmax, int nblocks, double eps, long long max_iter) {
-  if (st->done) return;
-  double mx = 0.0, md = 0.0, nn = 0.0;
-  for (int i = threadIdx.x; i < nblocks; i += 32) {
-    mx = fmax(mx, blockmax[3 * i]); md = fmax(md, blockmax[3 * i + 1]); nn = fmax(nn, blockmax[3 * i + 2]);
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) s_last = atomicAdd(ticket, 1u) == gridDim.x - 1 ? 1 : 0;
+  __syncthreads();
+  if (!s_last || threadIdx.x >= 32) return;
+  __threadfence();
+  mx = 0.0; md = 0.0; nn = 0.0;
+  for (int i = threadIdx.x; i < (int)gridDim.x; i += 32) {
+    mx = fmax(mx, __ldcg(blockmax + 3 * i)); md = fmax(md, __ldcg(blockmax + 3 * i + 1)); nn = fmax(nn, __ldcg(blockmax + 3 * i + 2));
   }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) {
@@ -845,6 +910,7 @@ __global__ void prox_finish(PgState *st, const double *__restrict__ blockmax, in
     nn = fmax(nn, __shfl_xor_sync(0xffffffffu, nn, o));
   }
   if (threadIdx.x == 0) {
+    *ticket = 0u;
     st->iter += 1;
     if (nn != 0.0) { st->delta = nan(""); st->done = 1; return; }
     st->delta = mx != 0.0 ? md / mx : md;
@@ -1474,7 +1540,11 @@ struct Work {
   DevBuf<unsigned long long> G, H;     // H: forward-code tables of the matrix-free pass
   DevBuf<double> T, lowtab;
   DevBuf<unsigned long long> q;        // binarized rows: round(w_i S) of every row, for low_accumulate
+  DevBuf<unsigned int> tickets;        // last-block counters of imp_fold, pass_tail, prox_update (zero between launches)
   double scale = 1.0, inv_scale = 1.0;
+  // after a matrix-free gradient pass: the folded tables whose columns pass_tail adds to G (nullptr: none pending)
+  const unsigned long long *F = nullptr;
+  ImpParams P{};
 };
 
 template <typename VT>
@@ -1589,6 +1659,7 @@ void launch_implicit(Matrix &M, Work &wk, const double cw[2], const PgState *st,
   P.M = I.M; P.N = I.N; P.op = I.op; P.Mlo = I.Mlo;
   for (int k = 0; k < 16; k++) { P.level_off[k] = I.level_off[k]; P.fo[k] = I.fo[k]; }
   const bool levels = I.Mlo <= I.N;            // (a binarized matrix with N <= 5 has table levels only)
+  wk.F = nullptr;
   P.S = levels ? super_length(I.N) : I.N;
   P.c = P.S - I.N + 1;
   const int64_t tlev = levels ? I.fo[I.N + 1] : 0, tsup = P.c > 1 ? (int64_t)1 << (2 * P.S) : 0, total = tlev + tsup;
@@ -1596,7 +1667,7 @@ void launch_implicit(Matrix &M, Work &wk, const double cw[2], const PgState *st,
   if (wk.T.n < (size_t)(total ? total : 1)) { wk.T.alloc((size_t)(total ? total : 1)); wk.H.alloc((size_t)(total ? total : 1)); }
   if (scatter && total) KL_CUDA(cudaMemsetAsync(wk.H.p, 0, (size_t)total * sizeof(unsigned long long), ctx().stream));
   if (levels) {
-    KL_LAUNCH(imp_build_T, (unsigned)((tlev + 255) / 256), 256, 0, P, I.bitmap.p, I.rank.p, wk.theta.p, wk.T.p, tlev, st);
+    KL_LAUNCH(imp_build_T, (unsigned)((tlev + 255) / 256), 256, 0, P, I.num->bits.p, I.num->rank.p, wk.theta.p, wk.T.p, tlev, st);
     if (P.c > 1) KL_LAUNCH(imp_build_TS, (unsigned)((tsup + 255) / 256), 256, 0, P, wk.T.p, st);
   }
   ImpArgs A{};
@@ -1636,10 +1707,22 @@ void launch_implicit(Matrix &M, Work &wk, const double cw[2], const PgState *st,
                 wk.G.p, st);
   if (!scatter) return;
   if (!levels) return;
-  if (P.c > 1) KL_LAUNCH(imp_fold_super, (unsigned)((tsup + 255) / 256), 256, 0, P, wk.H.p, st);
-  for (int j = I.N - 1; j >= I.Mlo; j--)
-    KL_LAUNCH(imp_fold_level, (unsigned)(((1u << (2 * j)) + 255) / 256), 256, 0, P, j, wk.H.p, st);
-  KL_LAUNCH(imp_columns, (unsigned)((M.m + 255) / 256), 256, 0, P, M.class_ids.p, M.m, wk.H.p, wk.G.p, st);
+  // the fold: the super level and the levels above IMP_FOLD_TAIL one launch each, the small levels in the last
+  // block of the last of those launches (or of a one-block launch when there is none)
+  const int small_top = I.N - 1 < IMP_FOLD_TAIL ? I.N - 1 : IMP_FOLD_TAIL;
+  int steps[IMP_MAX_N + 1], nsteps = 0;
+  if (P.c > 1) steps[nsteps++] = I.N;
+  for (int j = I.N - 1; j > small_top && j >= I.Mlo; j--) steps[nsteps++] = j;
+  if (nsteps == 0 && small_top >= I.Mlo) steps[nsteps++] = -1;
+  for (int s = 0; s < nsteps; s++) {
+    const int j = steps[s];
+    const int64_t items = j == I.N ? tsup : (j < 0 ? 1 : (int64_t)1 << (2 * j));
+    KL_LAUNCH(imp_fold, (unsigned)((items + IMP_FOLD_THREADS - 1) / IMP_FOLD_THREADS), IMP_FOLD_THREADS, 0, P, j,
+              s == nsteps - 1 ? small_top : -1, wk.H.p, wk.tickets.p, st);
+  }
+  // the columns are read off the folded tables by the pass tail (pass_tail)
+  wk.P = P;
+  wk.F = wk.H.p;
 }
 
 // the fused pass: loss terms + fixed-point gradient of the single-feature coefficients of THIS rank's rows
@@ -1690,6 +1773,18 @@ void alloc_work(const Matrix &M, int64_t ntheta, Work &wk) {
   wk.scalars.alloc(8);
   wk.blockmax.alloc(4 * PROX_BLOCKS);    // max |theta|, max |delta|, NaN flag per block + the L1 partials of the hook
   wk.gathered.alloc((size_t)(M.sharded ? ntheta * ctx().world : 1));
+  wk.tickets.alloc(3);
+  wk.tickets.zero();
+}
+
+// the tail of a pass (pass_tail): the pending matrix-free columns, the loss and L1 partials and, with a state and
+// hook = 1, the loss sum and the hook
+void launch_pass_tail(const Matrix &M, Work &wk, PgState *st, int64_t ntheta, double lambda, int hook, double eps_loss) {
+  static_assert(RED_BLOCKS == PROX_BLOCKS, "the L1 partials of pass_tail are the hook's PROX_BLOCKS partials");
+  KL_LAUNCH(pass_tail, RED_BLOCKS, 256, 0, st, wk.P, M.class_ids.p, M.m, wk.F, wk.G.p, wk.lossterm.p, st ? M.n : 0,
+            wk.red.p, wk.scalars.p, wk.theta.p, st ? ntheta : 0, lambda, wk.blockmax.p + 3 * PROX_BLOCKS, hook,
+            1.0 / (double)M.n_global, eps_loss, wk.tickets.p + 1);
+  wk.F = nullptr;
 }
 
 void check_theta(const Matrix &M, int64_t ntheta, int cooc) {
@@ -1735,6 +1830,7 @@ void gradient(Matrix &M, const double *theta, int64_t ntheta, const double cw[2]
     using VT = typename std::remove_pointer<decltype(tag)>::type;
     if (!cooc) {
       launch_fused<VT>(M, wk, cw, nullptr);
+      if (wk.F) launch_pass_tail(M, wk, nullptr, ntheta, NAN, 0, 0.0);
       if (M.sharded) comm_allreduce_sum_i64_fast((int64_t *)wk.G.p, M.m + 1);
     } else {
       // pair mode: z needs the pair terms, so the weights come from the general rows kernel; the
@@ -1810,12 +1906,17 @@ void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], doub
   double step = 1.0 / (2.0 * L + std::fmin(2.0 * l2, L)) * step_factor;
   Work wk; alloc_work(M, ntheta, wk);
   set_scale(M, wk, cw);
-  wk.theta.upload(theta, (size_t)ntheta);
+  // theta and the iteration state travel through the pinned staging buffer (theta first, the state behind it)
+  double *hth = (double *)host_staging((size_t)ntheta * sizeof(double) + sizeof(PgState));
+  PgState *hst = reinterpret_cast<PgState *>(hth + ntheta);
+  memcpy(hth, theta, (size_t)ntheta * sizeof(double));
+  wk.theta.upload(hth, (size_t)ntheta);
   DevBuf<PgState> st(1);
   PgState h{};
   h.iter = 0; h.done = max_iter > 0 ? 0 : 1; h.first = 1; h.delta = 0.0;
   h.loss_old = hook ? hook[0] : NAN; h.loss_new = hook ? hook[1] : NAN; h.lossval = NAN; h.error = 0;
-  st.upload(&h, 1);
+  *hst = h;
+  st.upload(hst, 1);
   const double inv_n = 1.0 / (double)M.n_global;
   // reduced matrices: long batches between host round trips.  The choice of the path uses quantities that are
   // the same on every rank (a rank with an empty shard must issue the same collectives as the others)
@@ -1974,30 +2075,34 @@ void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], doub
       dispatch_vt(M, [&](auto *tag) {
         using VT = typename std::remove_pointer<decltype(tag)>::type;
         launch_fused<VT>(M, wk, cw, st.p, scatter);
-        reduce_sum(M, wk.lossterm.p, M.n, wk, wk.scalars.p, st.p, false);
+        // columns, loss and L1 partials; one GPU: the loss sum and the hook in the same launch
+        launch_pass_tail(M, wk, st.p, M.m + 1, lambda, M.sharded ? 0 : 1, epsilon_loss);
         if (M.sharded) {
           // ONE collective per iteration: gradient words + the loss sums of the ranks
           unsigned long long *slots = wk.G.p + M.m + 1;
           KL_LAUNCH(pack_loss_slots, 1, 32, 0, st.p, wk.scalars.p, slots, ctx().rank, ctx().world);
           if (scatter) comm_allreduce_sum_i64_fast((int64_t *)wk.G.p, M.m + 1 + ctx().world);
           else comm_allreduce_sum_i64_fast((int64_t *)slots, ctx().world);
-          KL_LAUNCH(unpack_loss_slots, 1, 32, 0, st.p, slots, ctx().world, wk.scalars.p);
+          KL_LAUNCH(unpack_loss_hook, 1, 32, 0, st.p, slots, ctx().world, wk.scalars.p, wk.blockmax.p + 3 * PROX_BLOCKS,
+                    PROX_BLOCKS, inv_n, epsilon_loss);
         }
-        KL_LAUNCH(l1_partials, PROX_BLOCKS, 256, 0, st.p, wk.theta.p, M.m + 1, lambda, wk.blockmax.p + 3 * PROX_BLOCKS);
-        KL_LAUNCH(hook_kernel, 1, 32, 0, st.p, wk.scalars.p, wk.blockmax.p + 3 * PROX_BLOCKS, PROX_BLOCKS, inv_n, epsilon_loss);
-        KL_LAUNCH(prox_update, PROX_BLOCKS, 256, 0, st.p, wk.theta.p, wk.G.p, wk.inv_scale, ntheta, step, lambda,
-                  wk.blockmax.p);
-        KL_LAUNCH(prox_finish, 1, 32, 0, st.p, wk.blockmax.p, PROX_BLOCKS, epsilon, (long long)max_iter);
+        // the loss-only pass (number max_iter) follows the last prox step: the state is stopped (done != 0) by then
+        if (scatter)
+          KL_LAUNCH(prox_update, PROX_BLOCKS, 256, 0, st.p, wk.theta.p, wk.G.p, wk.inv_scale, ntheta, step, lambda,
+                    wk.blockmax.p, epsilon, (long long)max_iter, wk.tickets.p + 2);
       });
     }
-    st.download(&h, 1);
+    // theta comes down with the state: a batch is usually the last one, and then no second round trip is needed
+    st.download(hst, 1);
+    wk.theta.download(hth, (size_t)ntheta);
+    host_staging_done();
     sync_stream();
+    h = *hst;
     if (h.error) fail(KMERLR_ERR_CUDA, "proxgrad: a rank did not answer the gradient exchange over peer memory");
     if (M.sharded) comm_check_peer_errors();
     if (h.done == 1) break;
   }
-  wk.theta.download(theta, (size_t)ntheta);
-  sync_stream();
+  memcpy(theta, hth, (size_t)ntheta * sizeof(double));
   tr.mark("iterations");
   if (hook) { hook[0] = h.loss_old; hook[1] = h.loss_new; }
   if (iters) *iters = (int64_t)h.iter;

@@ -365,6 +365,7 @@ std::shared_ptr<Matrix> matrix_transform(Matrix &M, const double *offset, const 
   if (M.has_labels) {
     R->labels.alloc((size_t)(M.n ? M.n : 1));
     KL_CUDA(cudaMemcpyAsync(R->labels.p, M.labels.p, (size_t)M.n, cudaMemcpyDeviceToDevice, ctx().stream));
+    matrix_label_counts_local(M);
     R->n_pos = M.n_pos; R->n_neg = M.n_neg; R->counts_global = M.counts_global; R->has_labels = true;
     sync_stream();
   }
@@ -518,22 +519,56 @@ void matrix_rows(Matrix &M, int64_t *rowptr, int32_t *col, double *val) {
   }
 }
 
+// labels[i] = raw[i] != 0 in place, *ones += the number of ones
+__global__ void normalize_labels(uint8_t *__restrict__ labels, int64_t n, unsigned long long *__restrict__ ones) {
+  __shared__ unsigned int sh;
+  if (threadIdx.x == 0) sh = 0u;
+  __syncthreads();
+  unsigned int c = 0;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
+    const uint8_t v = labels[i] != 0;
+    labels[i] = v;
+    c += v;
+  }
+  if (c) atomicAdd(&sh, c);
+  __syncthreads();
+  if (threadIdx.x == 0 && sh) atomicAdd(ones, (unsigned long long)sh);
+}
+
+// the labels go up through the pinned staging buffer and are normalised and counted on the device: no host pass
+// over them and no wait for the device (the count is read when somebody asks for it)
 void matrix_set_labels(Matrix &M, const uint8_t *labels, int64_t n) {
   require_ready();
   KL_REQUIRE(n == M.n, "labels: length does not match the number of rows");
   M.labels.alloc((size_t)(n ? n : 1));
-  std::vector<uint8_t> l((size_t)n);
-  int64_t ones = 0;
-  for (int64_t i = 0; i < n; i++) { const uint8_t v = labels[i] != 0; l[i] = v; ones += v; }
-  M.labels.upload(l.data(), (size_t)n);
-  sync_stream();
+  M.label_ones.alloc(1);
+  M.label_ones.zero();
+  if (n > 0) {
+    uint8_t *h = (uint8_t *)host_staging((size_t)n);
+    memcpy(h, labels, (size_t)n);
+    M.labels.upload(h, (size_t)n);
+    host_staging_done();
+    int64_t blocks = (n + 255) / 256;
+    if (blocks > 4 * ctx().sm_count) blocks = 4 * ctx().sm_count;
+    KL_LAUNCH(normalize_labels, (unsigned)blocks, 256, 0, M.labels.p, n, M.label_ones.p);
+  }
   // the global counts (class weights) are summed over the ranks when somebody asks: no collective here
-  M.n_neg = n - ones; M.n_pos = ones;
+  M.counts_pending = true;
   M.counts_global = !M.sharded;
   M.has_labels = true;
 }
 
+void matrix_label_counts_local(Matrix &M) {
+  if (!M.counts_pending) return;
+  unsigned long long ones = 0;
+  M.label_ones.download(&ones, 1);
+  sync_stream();
+  M.n_pos = (int64_t)ones; M.n_neg = M.n - (int64_t)ones;
+  M.counts_pending = false;
+}
+
 void matrix_label_counts(Matrix &M) {
+  matrix_label_counts_local(M);
   if (M.counts_global) return;
   int64_t cnt[2] = {M.n_neg, M.n_pos};
   DevBuf<int64_t> tmp(2);
@@ -831,6 +866,7 @@ std::shared_ptr<Matrix> matrix_reduce(Matrix &M, const int64_t *sel, int64_t nse
   if (M.has_labels) {
     R->labels.alloc((size_t)(M.n ? M.n : 1));
     KL_CUDA(cudaMemcpyAsync(R->labels.p, M.labels.p, (size_t)M.n, cudaMemcpyDeviceToDevice, ctx().stream));
+    matrix_label_counts_local(M);
     R->n_pos = M.n_pos; R->n_neg = M.n_neg; R->counts_global = M.counts_global; R->has_labels = true;
     sync_stream();
   }
