@@ -142,7 +142,8 @@ __global__ void __launch_bounds__(256) fused_kernel(const Rows R, const uint32_t
                                                     const VT *__restrict__ val, int64_t n, int64_t m,
                                                     const double *__restrict__ theta,
                                                     const uint8_t *__restrict__ labels, double cw0, double cw1,
-                                                    double inv_n, double scale, unsigned long long *__restrict__ G,
+                                                    double inv_n, double scale, double scale0,
+                                                    unsigned long long *__restrict__ G,
                                                     double *__restrict__ lossterm, const PgState *st, int scatter,
                                                     int hot_limit, int rpb, unsigned long long *__restrict__ ticket) {
   if (st && st->done == 1) return;
@@ -168,7 +169,7 @@ __global__ void __launch_bounds__(256) fused_kernel(const Rows R, const uint32_t
       double z = theta[0] + s, r = -log_add0(-z);
       if (labels[row]) { w = inv_n * cw1 * (exp(r) - 1.0); lossterm[row] = -cw1 * r; }
       else             { w = inv_n * cw0 * exp(r);         lossterm[row] = cw0 * log_add0(z); }
-      bias_acc += __double2ll_rn(w * scale);
+      bias_acc += __double2ll_rn(w * scale0);
     }
     if (!scatter) return;                 // loss-only pass (the hook after the last iteration)
     w = __shfl_sync(0xffffffffu, w, 0);
@@ -628,23 +629,23 @@ __device__ __forceinline__ void imp_column(const ImpParams &P, const uint32_t *_
 template <typename VT>
 __global__ void scatter_w(const Rows R, const uint32_t *__restrict__ col,
                           const VT *__restrict__ val, int64_t n, const double *__restrict__ w, double scale,
-                          unsigned long long *__restrict__ G) {
+                          double scale0, unsigned long long *__restrict__ G) {
   int64_t row = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (row >= n) return;
   unsigned lane = lane_id();
   const double ws = w[row] * scale;
-  if (lane == 0) atomicAdd(&G[0], (unsigned long long)__double2ll_rn(ws));
+  if (lane == 0) atomicAdd(&G[0], (unsigned long long)__double2ll_rn(w[row] * scale0));
   int64_t a, b;
   R.range(row, a, b);
   for (int64_t p = a + lane; p < b; p += 32)
     atomicAdd(&G[col[p] + 1], (unsigned long long)__double2ll_rn(ws * valf(val, p)));
 }
 
-// g[j] = G[j] / S for the single-feature coefficients
-__global__ void finalize_g(const unsigned long long *__restrict__ G, int64_t count, double inv_scale,
+// g[j] = G[j] / S for the single-feature coefficients (the bias has a scale of its own, see set_scale)
+__global__ void finalize_g(const unsigned long long *__restrict__ G, int64_t count, double inv_scale, double inv_scale0,
                            double *__restrict__ g) {
   int64_t j = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (j < count) g[j] = (double)(long long)G[j] * inv_scale;
+  if (j < count) g[j] = (double)(long long)G[j] * (j == 0 ? inv_scale0 : inv_scale);
 }
 
 // pair coefficients (kmerLr_logistic_regression.go:183-195): g[Ind2Sub(a,b)] = sum_i (w_i v_ia) v_ib, a < b.
@@ -864,14 +865,14 @@ __global__ void __launch_bounds__(256) pass_tail(PgState *st, const ImpParams P,
 // per-block max |theta|, max |delta| and NaN flag; the block that finishes last takes the decision.  `ticket` is
 // zero on entry and left zero.
 __global__ void prox_update(PgState *st, double *__restrict__ theta, const unsigned long long *__restrict__ G,
-                            double inv_scale, int64_t ntheta, double step, double lambda,
+                            double inv_scale, double inv_scale0, int64_t ntheta, double step, double lambda,
                             double *__restrict__ blockmax, double eps, long long max_iter, unsigned int *ticket) {
   if (st->done) return;
   __shared__ double shx[256], shd[256], shn[256];
   __shared__ int s_last;
   double mx = 0.0, md = 0.0, nn = 0.0;
   for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < ntheta; k += (int64_t)gridDim.x * blockDim.x) {
-    double g = (double)(long long)G[k] * inv_scale;
+    double g = (double)(long long)G[k] * (k == 0 ? inv_scale0 : inv_scale);
     double t0 = theta[k], t1 = t0 - step * g;
     if (k > 0) {
       if (t1 >= 0.0) t1 = fmax(fabs(t1) - step * lambda, 0.0);
@@ -1541,7 +1542,8 @@ struct Work {
   DevBuf<double> T, lowtab;
   DevBuf<unsigned long long> q;        // binarized rows: round(w_i S) of every row, for low_accumulate
   DevBuf<unsigned int> tickets;        // last-block counters of imp_fold, pass_tail, prox_update (zero between launches)
-  double scale = 1.0, inv_scale = 1.0;
+  double scale = 1.0, inv_scale = 1.0;      // the columns of the matrix
+  double scale0 = 1.0, inv_scale0 = 1.0;    // the bias (its value is 1 in every row)
   // after a matrix-free gradient pass: the folded tables whose columns pass_tail adds to G (nullptr: none pending)
   const unsigned long long *F = nullptr;
   ImpParams P{};
@@ -1617,14 +1619,22 @@ void launch_rows(const Matrix &M, const double *theta, int cooc, const double cw
             sparse ? T->dev.p : (const PairTerm *)nullptr, sparse ? T->n : 0);
 }
 
-// fixed-point scale: sum_i |w_i v_ic| <= max(cw) * max|v|, kept below 2^60
-void set_scale(Matrix &M, Work &wk, const double cw[2]) {
-  double bound = std::fmax(std::fabs(cw[0]), std::fabs(cw[1])) * std::fmax(matrix_vmax(M), 1.0);
+// fixed-point scales: sum_i |w_i v_ic| <= max(cw) * max|v| for a column, <= max(cw) for the bias, each kept below
+// 2^60.  The columns of a matrix whose values are all below 1 get the finer scale their bound allows (a matrix of
+// frequencies would otherwise lose the bits between max|v| and 1); the bias keeps max(cw) * max(max|v|, 1).  Both
+// are the same whenever max|v| >= 1, as in every count and binarized matrix.
+static int scale_exponent(double bound) {
   if (!(bound > 0.0) || !std::isfinite(bound)) bound = 1.0;
-  int e = 60 - (int)std::ceil(std::log2(bound));
-  if (e > 1000) e = 1000;
+  const int e = 60 - (int)std::ceil(std::log2(bound));
+  return e > 1000 ? 1000 : e;
+}
+void set_scale(Matrix &M, Work &wk, const double cw[2]) {
+  const double cmax = std::fmax(std::fabs(cw[0]), std::fabs(cw[1])), vmax = matrix_vmax(M);
+  const int e = scale_exponent(cmax * (vmax > 0.0 ? vmax : 1.0)), e0 = scale_exponent(cmax * std::fmax(vmax, 1.0));
   wk.scale = std::ldexp(1.0, e);
   wk.inv_scale = std::ldexp(1.0, -e);
+  wk.scale0 = std::ldexp(1.0, e0);
+  wk.inv_scale0 = std::ldexp(1.0, -e0);
 }
 
 // kmerlr_option("implicit", 0) or KMERLR_IMPLICIT=0 forces the pass over the stored rows (tests compare the two)
@@ -1653,6 +1663,7 @@ void launch_imp_pass(const ImpParams &P, const ImpArgs &A, size_t smem) {
 }
 
 void launch_implicit(Matrix &M, Work &wk, const double cw[2], const PgState *st, int scatter) {
+  KL_INVARIANT(wk.scale == wk.scale0);       // (one round(w_i S) per row serves the bias and the columns)
   const Implicit &I = *M.imp;
   const SeqSet &S = *I.seqs;
   ImpParams P{};
@@ -1750,13 +1761,13 @@ void launch_fused(Matrix &M, Work &wk, const double cw[2], const PgState *st, in
         int64_t blocks = (int64_t)ctx().sm_count * per_sm, need = (M.n + 8 * tk - 1) / (8 * tk);
         if (blocks > need) blocks = need;
         KL_LAUNCH((fused_kernel<VT>), (unsigned)blocks, 256, smem, M.rows(), M.col.p, csr_val<VT>(M), M.n, M.m, wk.theta.p,
-                  M.labels.p, cw[0], cw[1], 1.0 / (double)M.n_global, wk.scale, wk.G.p, wk.lossterm.p, st, scatter, hot, tk,
+                  M.labels.p, cw[0], cw[1], 1.0 / (double)M.n_global, wk.scale, wk.scale0, wk.G.p, wk.lossterm.p, st, scatter, hot, tk,
                   ticket);
       } else {
         int rpb = FUSED_RPB;
         while ((M.n + rpb - 1) / rpb > 0x7fffffffLL) rpb *= 2;
         KL_LAUNCH((fused_kernel<VT>), (unsigned)((M.n + rpb - 1) / rpb), 256, smem, M.rows(), M.col.p, csr_val<VT>(M), M.n,
-                  M.m, wk.theta.p, M.labels.p, cw[0], cw[1], 1.0 / (double)M.n_global, wk.scale, wk.G.p, wk.lossterm.p, st,
+                  M.m, wk.theta.p, M.labels.p, cw[0], cw[1], 1.0 / (double)M.n_global, wk.scale, wk.scale0, wk.G.p, wk.lossterm.p, st,
                   scatter, hot, rpb, (unsigned long long *)nullptr);
       }
     }
@@ -1844,7 +1855,7 @@ void gradient(Matrix &M, const double *theta, int64_t ntheta, const double cw[2]
       KL_CUDA(cudaMemsetAsync(wk.G.p, 0, (size_t)(M.m + 1) * sizeof(unsigned long long), ctx().stream));
       if (M.n > 0)
         KL_LAUNCH((scatter_w<VT>), warp_grid(M.n, 256), 256, 0, M.rows(), M.col.p, csr_val<VT>(M), M.n, wk.w.p,
-                  wk.scale, wk.G.p);
+                  wk.scale, wk.scale0, wk.G.p);
       if (M.sharded) comm_allreduce_sum_i64((int64_t *)wk.G.p, M.m + 1);
       if (M.m > 1) {
         const int ntile = (int)((M.m + PAIR_T - 1) / PAIR_T);
@@ -1860,7 +1871,7 @@ void gradient(Matrix &M, const double *theta, int64_t ntheta, const double cw[2]
       }
     }
   });
-  KL_LAUNCH(finalize_g, (unsigned)((M.m + 1 + 255) / 256), 256, 0, wk.G.p, M.m + 1, wk.inv_scale, wk.g.p);
+  KL_LAUNCH(finalize_g, (unsigned)((M.m + 1 + 255) / 256), 256, 0, wk.G.p, M.m + 1, wk.inv_scale, wk.inv_scale0, wk.g.p);
   if (!std::isnan(lambda) && lambda != 0.0)
     KL_LAUNCH(add_l1_sign, (unsigned)((ntheta + 255) / 256), 256, 0, wk.theta.p, wk.g.p, ntheta, lambda);
   if (g_host) wk.g.download(g_host, (size_t)ntheta);
@@ -1921,6 +1932,8 @@ void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], doub
   // reduced matrices: long batches between host round trips.  The choice of the path uses quantities that are
   // the same on every rank (a rank with an empty shard must issue the same collectives as the others)
   const bool small = ntheta <= SMALL_MAX_THETA && !use_implicit(M);
+  // the kernels of reduced matrices accumulate the bias and the columns with one scale: the coarser one
+  if (small) { wk.scale = wk.scale0; wk.inv_scale = wk.inv_scale0; }
   // the passes of a batch are ONE cooperative launch (grid barriers instead of launches); sharded matrices
   // exchange the gradient inside that kernel over NVLink peer memory
   const bool p2p = M.sharded && ctx().peer && ctx().p2p_ok;
@@ -2088,7 +2101,7 @@ void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], doub
         }
         // the loss-only pass (number max_iter) follows the last prox step: the state is stopped (done != 0) by then
         if (scatter)
-          KL_LAUNCH(prox_update, PROX_BLOCKS, 256, 0, st.p, wk.theta.p, wk.G.p, wk.inv_scale, ntheta, step, lambda,
+          KL_LAUNCH(prox_update, PROX_BLOCKS, 256, 0, st.p, wk.theta.p, wk.G.p, wk.inv_scale, wk.inv_scale0, ntheta, step, lambda,
                     wk.blockmax.p, epsilon, (long long)max_iter, wk.tickets.p + 2);
       });
     }
