@@ -187,7 +187,12 @@ int kmerlr_coordinate(kmerlr_handle h, double *theta_inout, int64_t ntheta, cons
 
 /* ---- stage 3: genomicKmerLr.Predict / predict_window_genomic (kmerLr_predict_genomic.go:134-171)
  * One model = one KmerLrEnsemble; the per-window result is the sum over models of the ensemble
- * summary of log sigma(x . theta) (kmerLr_classifier_ensemble.go:64-139). */
+ * summary of log sigma(x . theta) (kmerLr_classifier_ensemble.go:64-139).
+ * Accepted: every model the extraction builds -- the nucleotide alphabet with 1 <= M <= N <= 14 and any subset of
+ * complement / reverse / revcomp, the gapped nucleotide alphabet with N <= 11 and any max_ambiguous, any number of
+ * model classes, any window size, 1..16 ensemble members.  Refused (KMERLR_ERR_ARG): the IUPAC alphabet, more than
+ * 16 members, an ensemble without a summary, classes outside [M, N] or with a code out of range, duplicate classes,
+ * feature indices out of range. */
 #define KMERLR_SUMMARY_NONE 0
 #define KMERLR_SUMMARY_MEAN 1
 #define KMERLR_SUMMARY_PRODUCT 2

@@ -10,6 +10,7 @@
 //     with k > 8 on rows too long for the register sort of the main kernel.
 // Codes are base-|alphabet| numbers (first letter most significant), class = min over the k-mer and its images.
 #include "common.cuh"
+#include "kmer_class.cuh"
 
 #include <cub/device/device_radix_sort.cuh>
 #include <cub/device/device_run_length_encode.cuh>
@@ -23,15 +24,12 @@ constexpr int SORT_MAX_N = 14;                      // nucleotide alphabet: 4^1 
 constexpr unsigned long long GAP_NONE = ~0ull;
 
 struct GapParams {
-  int M, N, max_amb;
-  int A;                        // alphabet size: 5 = gapped (wildcard variants), 4 = nucleotide
-  int revcomp, complement, reverse;
+  int M, N;
+  ClassRule R;                  // alphabet, max_ambiguous, strand flags (kmer_class.cuh)
   uint32_t level_off[16];       // dense id of (k, code 0), multiples of 32
   uint32_t slots_per_pos;       // sum over k of 2^max(k-2, 0)
   uint32_t slot_off[16];        // offset of level k inside the slots of one position
 };
-
-__device__ __forceinline__ uint32_t gap_comp(uint32_t d) { return d < 4u ? 3u - d : d; }
 
 // one thread per base position of the whole set: writes slots_per_pos keys
 __global__ void gapped_fill(const GapParams P, int64_t n, const int64_t *__restrict__ len,
@@ -47,34 +45,22 @@ __global__ void gapped_fill(const GapParams P, int64_t n, const int64_t *__restr
   const uint32_t *b2 = bits2 + blk[row] * 4;
   const uint16_t *iv = inv16 + blk[row] * 4;
   unsigned long long *out = keys + t * P.slots_per_pos;
-  uint32_t l[SORT_MAX_N + 1];
+  uint32_t e = 0;                                   // letter j in bits 2j, 2j+1
   int valid = 0;                                    // valid bases from p on
   for (int j = 0; j < P.N && p + j < L; j++) {
     const int64_t idx = p + j;
     if ((iv[idx >> 4] >> (idx & 15)) & 1u) break;
-    l[j] = (b2[idx >> 4] >> (2 * (idx & 15))) & 3u;
+    e |= ((b2[idx >> 4] >> (2 * (idx & 15))) & 3u) << (2 * j);
     valid = j + 1;
   }
-  const unsigned long long A = (unsigned long long)P.A;
   for (int k = P.M; k <= P.N; k++) {
-    const int nin = (P.A == 5 && k >= 2) ? k - 2 : 0;
     unsigned long long *o = out + P.slot_off[k];
-    for (uint32_t mask = 0; mask < (1u << nin); mask++) {
+    const uint32_t nm = kmer_masks(P.R, k);
+    for (uint32_t mask = 0; mask < nm; mask++) {
       unsigned long long key = GAP_NONE;
-      if (valid >= k && (P.max_amb < 0 || __popc(mask) <= P.max_amb)) {
-        // variant digits v[j]: wildcard where the mask says so (interior positions 1 .. k-2)
-        auto digit = [&](int j) -> uint32_t { return (j >= 1 && j <= nin && ((mask >> (j - 1)) & 1u)) ? 4u : l[j]; };
-        unsigned long long c0 = 0, cc = 0, cr = 0, crc = 0;
-        for (int j = 0; j < k; j++) {
-          c0 = c0 * A + digit(j);
-          cc = cc * A + gap_comp(digit(j));                 // complement keeps the order
-          cr = cr * A + digit(k - 1 - j);                   // reverse keeps the letters
-          crc = crc * A + gap_comp(digit(k - 1 - j));
-        }
-        if (P.complement && cc < c0) c0 = cc;
-        if (P.reverse && cr < c0) c0 = cr;
-        if (P.revcomp && crc < c0) c0 = crc;
-        key = ((unsigned long long)row << 40) | (unsigned long long)(P.level_off[k] + (uint32_t)c0);
+      if (valid >= k) {
+        const uint32_t c = kmer_variant_class(P.R, e, k, mask);
+        if (c != KMER_NONE) key = ((unsigned long long)row << 40) | (unsigned long long)(P.level_off[k] + c);
       }
       o[mask] = key;
     }
@@ -149,12 +135,11 @@ std::shared_ptr<Matrix> extract_gapped(const kmerlr_config &cfg, std::shared_ptr
   KL_REQUIRE(s.n < ((int64_t)1 << 24), "sort-based extraction path: at most 2^24 sequences per call");
   const bool sharded = (flags & KMERLR_FLAG_SHARDED) != 0 && ctx().world > 1;
   GapParams P{};
-  P.M = cfg.M; P.N = cfg.N; P.max_amb = gapped ? cfg.max_ambiguous : -1;
-  P.A = gapped ? 5 : 4;
-  P.revcomp = cfg.revcomp != 0; P.complement = cfg.complement != 0; P.reverse = cfg.reverse != 0;
+  P.M = cfg.M; P.N = cfg.N;
+  P.R = ClassRule{gapped ? 5 : 4, gapped ? cfg.max_ambiguous : -1, cfg.complement != 0, cfg.reverse != 0, cfg.revcomp != 0};
   uint64_t dense = 0, p5 = 1;
   for (int k = 1; k <= cfg.N; k++) {
-    p5 *= (uint64_t)P.A;
+    p5 *= (uint64_t)P.R.A;
     if (k < cfg.M) continue;
     P.level_off[k] = (uint32_t)dense;
     dense += (p5 + 31) / 32 * 32;
