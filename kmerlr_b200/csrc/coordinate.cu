@@ -28,6 +28,13 @@ namespace {
 constexpr int CD_MAX_THETA = 1024;
 constexpr int CD_THREADS = 1024;
 
+// the powers of two of the fixed-point sums, one per class of entry: xy of the bias and of a column; xx of
+// (bias, bias), (bias, column) and (column, column).  The bias is 1 in every row, a column at most max|v|: a matrix
+// whose values are all below 1 keeps the bits between max|v| and 1 in its column entries.
+struct CdScales {
+  double xy0, xy, xx00, xx0c, xxcc;
+};
+
 template <typename VT>
 __device__ __forceinline__ double cd_val(const VT *val, int64_t p) { return val ? (double)val[p] : 1.0; }
 
@@ -37,8 +44,8 @@ __global__ void __launch_bounds__(256) cd_rows_kernel(const Rows R, const uint32
                                                       const VT *__restrict__ val, int64_t n, int64_t ntheta,
                                                       const double *__restrict__ theta,
                                                       const uint8_t *__restrict__ labels, double cw0, double cw1,
-                                                      double scale_xy, double scale_xx, long long *__restrict__ XY,
-                                                      long long *__restrict__ XX, int *__restrict__ bad) {
+                                                      CdScales S, long long *__restrict__ XY, long long *__restrict__ XX,
+                                                      int *__restrict__ bad) {
   __shared__ double sth[CD_MAX_THETA];
   for (int i = threadIdx.x; i < ntheta; i += blockDim.x) sth[i] = theta[i];
   __syncthreads();
@@ -60,21 +67,26 @@ __global__ void __launch_bounds__(256) cd_rows_kernel(const Rows R, const uint32
   for (int64_t p1 = a - 1; p1 < b; p1++) {
     const int64_t j1 = p1 < a ? 0 : (int64_t)col[p1] + 1;
     const double v1 = p1 < a ? 1.0 : cd_val(val, p1);
-    atomicAdd((unsigned long long *)&XY[j1], (unsigned long long)__double2ll_rn(wz * v1 * scale_xy));
+    atomicAdd((unsigned long long *)&XY[j1], (unsigned long long)__double2ll_rn(wz * v1 * (j1 == 0 ? S.xy0 : S.xy)));
     const double wv1 = w * v1;
+    const double sb = j1 == 0 ? S.xx00 : S.xx0c, sc = j1 == 0 ? S.xx0c : S.xxcc;     // the scales of (j1, bias), (j1, column)
     for (int64_t p2 = a - 1; p2 < b; p2++) {
       const int64_t j2 = p2 < a ? 0 : (int64_t)col[p2] + 1;
       const double v2 = p2 < a ? 1.0 : cd_val(val, p2);
-      atomicAdd((unsigned long long *)&XX[j1 * ntheta + j2], (unsigned long long)__double2ll_rn(wv1 * v2 * scale_xx));
+      atomicAdd((unsigned long long *)&XX[j1 * ntheta + j2],
+                (unsigned long long)__double2ll_rn(wv1 * v2 * (j2 == 0 ? sb : sc)));
     }
   }
 }
 
 __global__ void cd_convert_kernel(const long long *__restrict__ XY, const long long *__restrict__ XX, int64_t ntheta,
-                                  double inv_xy, double inv_xx, double *__restrict__ xy, double *__restrict__ xx) {
+                                  CdScales inv, double *__restrict__ xy, double *__restrict__ xx) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < ntheta) xy[i] = (double)XY[i] * inv_xy;
-  if (i < ntheta * ntheta) xx[i] = (double)XX[i] * inv_xx;
+  if (i < ntheta) xy[i] = (double)XY[i] * (i == 0 ? inv.xy0 : inv.xy);
+  if (i < ntheta * ntheta) {
+    const bool b1 = i < ntheta, b2 = i % ntheta == 0;
+    xx[i] = (double)XX[i] * (b1 && b2 ? inv.xx00 : (b1 || b2 ? inv.xx0c : inv.xxcc));
+  }
 }
 
 struct CdState {
@@ -130,6 +142,14 @@ __global__ void __launch_bounds__(CD_THREADS) cd_sweep_kernel(const double *__re
   }
 }
 
+// 60 - ceil(log2(bound)): a sum bounded by `bound` stays below 2^60.  Clamped like scale_exponent (logistic.cu) so
+// that 2^e and 2^-e stay finite; a bound of 0 (an empty matrix) takes the exponent of 1
+int cd_exponent(double bound) {
+  if (!(bound > 0.0) || !std::isfinite(bound)) bound = 1.0;
+  const int e = 60 - (int)std::ceil(std::log2(bound));
+  return e > 1000 ? 1000 : e;
+}
+
 // eval_stopping on the host for the outer iteration (two short vectors)
 bool eval_stopping_host(const std::vector<double> &x0, const std::vector<double> &x1, double eps, double *delta) {
   double max_x = 0.0, max_d = 0.0;
@@ -160,7 +180,7 @@ void coordinate(Matrix &M, double *theta, int64_t ntheta, const double cw_hook[2
   const double ntot = (double)(M.n_pos + M.n_neg);
   const double cw[2] = {ntot / (2.0 * (double)M.n_neg), ntot / (2.0 * (double)M.n_pos)};
   const double cwmax = std::fmax(cw[0], cw[1]);
-  const double vmax = std::fmax(matrix_vmax(M), 1.0), maxsq = matrix_maxsq(M);
+  const double vmax = matrix_vmax(M), v1 = std::fmax(vmax, 1.0), maxsq = matrix_maxsq(M);
 
   DevBuf<double> dtheta((size_t)ntheta), xy((size_t)ntheta), xx((size_t)(ntheta * ntheta));
   DevBuf<long long> XY((size_t)ntheta), XX((size_t)(ntheta * ntheta));
@@ -184,25 +204,32 @@ void coordinate(Matrix &M, double *theta, int64_t ntheta, const double cw_hook[2
   const unsigned cv_grid = (unsigned)((ntheta * ntheta + 255) / 256);
   bool nan_abort = false;
   for (int64_t iter = 0; iter < max_iter; iter++) {
-    // scales of the fixed-point sums: |w x x| <= cw vmax^2 / 4, |w z x| <= cw vmax (|r| / 4 + 1)
+    // scales of the fixed-point sums: |w x_j x_k| <= cw |x_j| |x_k| / 4, |w z x_j| <= cw |x_j| (|r| / 4 + 1), with
+    // |x_0| = 1 for the bias and |x_j| <= vmax for a column; the bias bounds take max(vmax, 1) (v1), so every
+    // exponent is the same whenever vmax >= 1
     double th2 = 0.0;
     for (int64_t k = 1; k < ntheta; k++) th2 += th1[k] * th1[k];
     const double rmax = std::fabs(th1[0]) + std::sqrt(th2 * maxsq);
-    double bxx = (double)M.n * 0.25 * cwmax * vmax * vmax, bxy = (double)M.n * cwmax * vmax * (0.25 * rmax + 1.0);
-    if (!(bxx > 0.0) || !std::isfinite(bxx)) bxx = 1.0;
-    if (!(bxy > 0.0) || !std::isfinite(bxy)) { nan_abort = true; break; }
-    const int exx = 60 - (int)std::ceil(std::log2(bxx)), exy = 60 - (int)std::ceil(std::log2(bxy));
+    const double bxy0 = (double)M.n * cwmax * v1 * (0.25 * rmax + 1.0);
+    if (!(bxy0 > 0.0) || !std::isfinite(bxy0)) { nan_abort = true; break; }
+    const int exy0 = cd_exponent(bxy0), exy = cd_exponent((double)M.n * cwmax * vmax * (0.25 * rmax + 1.0));
+    const int exx00 = cd_exponent((double)M.n * 0.25 * cwmax * v1 * v1),
+              exx0c = cd_exponent((double)M.n * 0.25 * cwmax * v1 * vmax),
+              exxcc = cd_exponent((double)M.n * 0.25 * cwmax * vmax * vmax);
+    const CdScales S{std::ldexp(1.0, exy0), std::ldexp(1.0, exy), std::ldexp(1.0, exx00), std::ldexp(1.0, exx0c),
+                     std::ldexp(1.0, exxcc)};
+    const CdScales inv{std::ldexp(1.0, -exy0), std::ldexp(1.0, -exy), std::ldexp(1.0, -exx00), std::ldexp(1.0, -exx0c),
+                       std::ldexp(1.0, -exxcc)};
     dtheta.upload(th1.data(), (size_t)ntheta);
     XY.zero(); XX.zero(); bad.zero();
     if (M.vt == VAL_F64)
       KL_LAUNCH((cd_rows_kernel<double>), row_grid, 256, 0, M.rows(), M.col.p, M.val_f64.p, M.n, ntheta, dtheta.p, M.labels.p,
-                cw[0], cw[1], std::ldexp(1.0, exy), std::ldexp(1.0, exx), XY.p, XX.p, bad.p);
+                cw[0], cw[1], S, XY.p, XX.p, bad.p);
     else
       KL_LAUNCH((cd_rows_kernel<uint32_t>), row_grid, 256, 0, M.rows(), M.col.p,
                 M.vt == VAL_U32 ? M.val_u32.p : (const uint32_t *)nullptr, M.n, ntheta, dtheta.p, M.labels.p, cw[0], cw[1],
-                std::ldexp(1.0, exy), std::ldexp(1.0, exx), XY.p, XX.p, bad.p);
-    KL_LAUNCH(cd_convert_kernel, cv_grid, 256, 0, XY.p, XX.p, ntheta, std::ldexp(1.0, -exy), std::ldexp(1.0, -exx), xy.p,
-              xx.p);
+                S, XY.p, XX.p, bad.p);
+    KL_LAUNCH(cd_convert_kernel, cv_grid, 256, 0, XY.p, XX.p, ntheta, inv, xy.p, xx.p);
     int hbad = 0;
     bad.download(&hbad, 1);
     sync_stream();

@@ -933,7 +933,7 @@ constexpr int SMALL_MAX_THETA = 1024;
 template <int BT = 256>
 __device__ __forceinline__ void small_tail(PgState *st, const double *blockloss, int nblocks, double *theta,
                                            unsigned long long *G,
-                                           double inv_scale, int64_t ntheta, double inv_n, double lambda,
+                                           double inv_scale, double inv_scale0, int64_t ntheta, double inv_n, double lambda,
                                            double eps_loss, double step, double eps, long long max_iter,
                                            bool clear_g = true, int replicas = 1) {
   constexpr int NW = BT / 32;
@@ -979,7 +979,7 @@ __device__ __forceinline__ void small_tail(PgState *st, const double *blockloss,
     for (int64_t k = t; k < ntheta; k += BT) {
       unsigned long long gi = __ldcg(G + k);
       for (int r = 1; r < replicas; r++) gi += __ldcg(G + r * ntheta + k);     // exact integer sum: any order
-      double g = (double)(long long)gi * inv_scale;
+      double g = (double)(long long)gi * (k == 0 ? inv_scale0 : inv_scale);
       double t0 = theta[k], t1 = t0 - step * g;
       if (k > 0) {
         if (t1 >= 0.0) t1 = fmax(fabs(t1) - step * lambda, 0.0);
@@ -1030,8 +1030,8 @@ template <typename VT, bool LOAD_THETA = true>
 __device__ __forceinline__ void small_rows(const Rows &R, const uint32_t *__restrict__ col, const VT *__restrict__ val,
                                            int64_t n, int64_t ntheta, const double *theta,
                                            const uint8_t *__restrict__ labels, double cw0, double cw1, double inv_n,
-                                           double scale, unsigned long long *G, double *blockloss, int scatter,
-                                           uint32_t *acc_lo, uint32_t *acc_hi, double *sth, double *red) {
+                                           double scale, double scale0, unsigned long long *G, double *blockloss,
+                                           int scatter, uint32_t *acc_lo, uint32_t *acc_hi, double *sth, double *red) {
   for (int i = threadIdx.x; i < ntheta; i += blockDim.x) {
     acc_lo[i] = 0u; acc_hi[i] = 0u;
     if (LOAD_THETA) sth[i] = theta[i];
@@ -1057,7 +1057,7 @@ __device__ __forceinline__ void small_rows(const Rows &R, const uint32_t *__rest
     else             { w = inv_n * cw0 * exp(r);         lacc += cw0 * log_add0(z); }
     if (!scatter) continue;
     const double ws = w * scale;                    // scale is a power of two: exact
-    add(0u, (unsigned long long)__double2ll_rn(ws));
+    add(0u, (unsigned long long)__double2ll_rn(w * scale0));
     for (int64_t p = a; p < b; p++) add(col[p] + 1u, (unsigned long long)__double2ll_rn(ws * valf(val, p)));
   }
   // loss partial of the block: shuffle tree inside the warps, then the warp sums in warp order (fixed)
@@ -1114,7 +1114,7 @@ __device__ __forceinline__ void small_acc_add(uint32_t *acc_lo, uint32_t *acc_hi
 template <typename VT>
 __device__ __forceinline__ void long_forward(const Rows &R, const LongView<VT> &V, int64_t n, int64_t ntheta,
                                              const uint8_t *__restrict__ labels, double cw0, double cw1, double inv_n,
-                                             double scale, double *blockloss, int scatter, uint32_t *acc_lo,
+                                             double scale, double scale0, double *blockloss, int scatter, uint32_t *acc_lo,
                                              uint32_t *acc_hi, const double *sth, double *red, double *w_local = nullptr) {
   for (int i = threadIdx.x; i < ntheta; i += blockDim.x) { acc_lo[i] = 0u; acc_hi[i] = 0u; }
   __syncthreads();
@@ -1148,7 +1148,7 @@ __device__ __forceinline__ void long_forward(const Rows &R, const LongView<VT> &
     if (!scatter) continue;
     const double ws = w * scale;
     if (w_local) w_local[row - row_lo] = ws; else V.wbuf[row] = ws;
-    bias += __double2ll_rn(ws);
+    bias += __double2ll_rn(w * scale0);
   }
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) { lacc += __shfl_down_sync(0xffffffffu, lacc, o); bias += __shfl_down_sync(0xffffffffu, bias, o); }
@@ -1264,17 +1264,17 @@ __global__ void __launch_bounds__(256, SMALL_BLOCKS_PER_SM) fused_small_kernel(c
                                                           const VT *__restrict__ val, int64_t n, int64_t ntheta,
                                                           double *theta, const uint8_t *__restrict__ labels,
                                                           double cw0, double cw1, double inv_n, double scale,
-                                                          unsigned long long *G, double *blockloss, PgState *st,
-                                                          int scatter, unsigned int *counter, double inv_scale,
-                                                          double lambda, double eps_loss, double step, double eps,
+                                                          double scale0, unsigned long long *G, double *blockloss,
+                                                          PgState *st, int scatter, unsigned int *counter,
+                                                          double inv_scale, double inv_scale0, double lambda, double eps_loss, double step, double eps,
                                                           long long max_iter) {
   if (st->done == 1) return;
   __shared__ uint32_t acc_lo[SMALL_MAX_THETA], acc_hi[SMALL_MAX_THETA];
   __shared__ int s_last;
   __shared__ double sth[SMALL_MAX_THETA];
   __shared__ double red[256];
-  small_rows<VT>(R, col, val, n, ntheta, theta, labels, cw0, cw1, inv_n, scale, G, blockloss, scatter, acc_lo, acc_hi, sth,
-                 red);
+  small_rows<VT>(R, col, val, n, ntheta, theta, labels, cw0, cw1, inv_n, scale, scale0, G, blockloss, scatter, acc_lo, acc_hi,
+                 sth, red);
   // the block that finishes last runs the tail of the iteration (its reads see every block's results)
   if (!counter) return;                 // sharded: the collectives come first, the tail is its own launch
   __threadfence();
@@ -1283,7 +1283,8 @@ __global__ void __launch_bounds__(256, SMALL_BLOCKS_PER_SM) fused_small_kernel(c
   __syncthreads();
   if (!s_last) return;
   __threadfence();
-  small_tail(st, blockloss, (int)gridDim.x, theta, G, inv_scale, ntheta, inv_n, lambda, eps_loss, step, eps, max_iter);
+  small_tail(st, blockloss, (int)gridDim.x, theta, G, inv_scale, inv_scale0, ntheta, inv_n, lambda, eps_loss, step, eps,
+             max_iter);
   if (threadIdx.x == 0) *counter = 0u;
 }
 
@@ -1306,8 +1307,9 @@ constexpr int PERSIST_THREADS = 256;
 template <typename VT, bool SHARDED, int LONG>
 __global__ void __launch_bounds__(PERSIST_THREADS, SMALL_BLOCKS_PER_SM) fused_small_persistent(
     const Rows R, const uint32_t *__restrict__ col, const VT *__restrict__ val, int64_t n, int64_t ntheta, double *theta,
-    const uint8_t *__restrict__ labels, double cw0, double cw1, double inv_n, double scale, unsigned long long *G3,
-    double *blockloss2, PgState *st, long long pass0, int npass, double inv_scale, double lambda, double eps_loss,
+    const uint8_t *__restrict__ labels, double cw0, double cw1, double inv_n, double scale, double scale0,
+    unsigned long long *G3, double *blockloss2, PgState *st, long long pass0, int npass, double inv_scale,
+    double inv_scale0, double lambda, double eps_loss,
     double step, double eps, long long max_iter, const PeerBox *pb, unsigned long long *Gx, double *scratch,
     unsigned int *abort_flag, const LongView<VT> LV) {
   cooperative_groups::grid_group grid = cooperative_groups::this_grid();
@@ -1347,22 +1349,24 @@ __global__ void __launch_bounds__(PERSIST_THREADS, SMALL_BLOCKS_PER_SM) fused_sm
     if (blockIdx.x == 0)
       for (int i = threadIdx.x; i < SMALL_REPLICAS * ntheta; i += blockDim.x) Gnext[i] = 0ull;
     if constexpr (LONG == 1) {
-      long_forward<VT>(R, LV, n, ntheta, labels, cw0, cw1, inv_n, scale, blockloss, scatter, acc_lo, acc_hi, sth, red);
+      long_forward<VT>(R, LV, n, ntheta, labels, cw0, cw1, inv_n, scale, scale0, blockloss, scatter, acc_lo, acc_hi, sth,
+                       red);
       if (scatter) {
         grid.sync();
         long_columns<VT>(LV, ntheta, G + (blockIdx.x % SMALL_REPLICAS) * ntheta, acc_lo, acc_hi, scp, c_first);
       }
     } else if constexpr (LONG == 2) {
-      long_forward<VT>(R, LV, n, ntheta, labels, cw0, cw1, inv_n, scale, blockloss, scatter, acc_lo, acc_hi, sth, red, w_s);
+      long_forward<VT>(R, LV, n, ntheta, labels, cw0, cw1, inv_n, scale, scale0, blockloss, scatter, acc_lo, acc_hi, sth,
+                       red, w_s);
       if (scatter) block_columns<VT>(LV, ntheta, G + (blockIdx.x % SMALL_REPLICAS) * ntheta, acc_lo, acc_hi, w_s);
     } else {
-      small_rows<VT, false>(R, col, val, n, ntheta, sth, labels, cw0, cw1, inv_n, scale,
+      small_rows<VT, false>(R, col, val, n, ntheta, sth, labels, cw0, cw1, inv_n, scale, scale0,
                             G + (blockIdx.x % SMALL_REPLICAS) * ntheta, blockloss, scatter, acc_lo, acc_hi, sth, red);
     }
     grid.sync();
     if (!SHARDED) {
-      small_tail<PERSIST_THREADS>(&ls, blockloss, nblocks, sth, G, inv_scale, ntheta, inv_n, lambda, eps_loss, step, eps,
-                                  max_iter, false, SMALL_REPLICAS);
+      small_tail<PERSIST_THREADS>(&ls, blockloss, nblocks, sth, G, inv_scale, inv_scale0, ntheta, inv_n, lambda, eps_loss,
+                                  step, eps, max_iter, false, SMALL_REPLICAS);
     } else {
       if (blockIdx.x == 0) {
         const int t = threadIdx.x, me = pb->rank, world = pb->world;
@@ -1418,8 +1422,8 @@ __global__ void __launch_bounds__(PERSIST_THREADS, SMALL_BLOCKS_PER_SM) fused_sm
         __syncthreads();
         break;
       }
-      small_tail<PERSIST_THREADS>(&ls, scratch, pb->world, sth, Gx, inv_scale, ntheta, inv_n, lambda, eps_loss, step, eps,
-                                  max_iter, false, 1);
+      small_tail<PERSIST_THREADS>(&ls, scratch, pb->world, sth, Gx, inv_scale, inv_scale0, ntheta, inv_n, lambda, eps_loss,
+                                  step, eps, max_iter, false, 1);
     }
     __syncthreads();
   }
@@ -1449,11 +1453,11 @@ __global__ void __launch_bounds__(256) small_presum_kernel(const PgState *st, co
 }
 // ... and the tail over the gathered per-rank losses (rank order) and the all-reduced gradient
 __global__ void __launch_bounds__(256) small_tail_kernel(PgState *st, const double *partials, int nparts, double *theta,
-                                                         unsigned long long *G, double inv_scale, int64_t ntheta,
-                                                         double inv_n, double lambda, double eps_loss, double step,
-                                                         double eps, long long max_iter) {
+                                                         unsigned long long *G, double inv_scale, double inv_scale0,
+                                                         int64_t ntheta, double inv_n, double lambda, double eps_loss,
+                                                         double step, double eps, long long max_iter) {
   if (st->done == 1) return;
-  small_tail(st, partials, nparts, theta, G, inv_scale, ntheta, inv_n, lambda, eps_loss, step, eps, max_iter);
+  small_tail(st, partials, nparts, theta, G, inv_scale, inv_scale0, ntheta, inv_n, lambda, eps_loss, step, eps, max_iter);
 }
 
 // Sharded reduced matrices, ranks connected by NVLink: the gradient all-reduce, the loss all-gather and
@@ -1466,7 +1470,8 @@ __global__ void __launch_bounds__(256) small_tail_kernel(PgState *st, const doub
 // iteration at 8 ranks against 20 us on one GPU.)
 __global__ void __launch_bounds__(256) small_p2p_tail_kernel(PgState *st, const PeerBox *pb, const double *__restrict__ blockloss,
                                                              int nblocks, double *theta, unsigned long long *G,
-                                                             double *scratch, double inv_scale, int64_t ntheta, double inv_n,
+                                                             double *scratch, double inv_scale, double inv_scale0,
+                                                             int64_t ntheta, double inv_n,
                                                              double lambda, double eps_loss, double step, double eps,
                                                              long long max_iter) {
   if (st->done == 1) return;
@@ -1531,7 +1536,7 @@ __global__ void __launch_bounds__(256) small_p2p_tail_kernel(PgState *st, const 
   __threadfence();
   __syncthreads();
   if (t == 0) { mine->senders_done = 0u; mine->seq = seq; }
-  small_tail(st, scratch, world, theta, G, inv_scale, ntheta, inv_n, lambda, eps_loss, step, eps, max_iter);
+  small_tail(st, scratch, world, theta, G, inv_scale, inv_scale0, ntheta, inv_n, lambda, eps_loss, step, eps, max_iter);
 }
 
 constexpr int PROX_BLOCKS = 256;
@@ -1932,8 +1937,8 @@ void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], doub
   // reduced matrices: long batches between host round trips.  The choice of the path uses quantities that are
   // the same on every rank (a rank with an empty shard must issue the same collectives as the others)
   const bool small = ntheta <= SMALL_MAX_THETA && !use_implicit(M);
-  // the kernels of reduced matrices accumulate the bias and the columns with one scale: the coarser one
-  if (small) { wk.scale = wk.scale0; wk.inv_scale = wk.inv_scale0; }
+  // the kernels of reduced matrices accumulate the columns and the bias with their own scales (set_scale), as the
+  // full-space pass does: the same integers G as fused_kernel
   // the passes of a batch are ONE cooperative launch (grid barriers instead of launches); sharded matrices
   // exchange the gradient inside that kernel over NVLink peer memory
   const bool p2p = M.sharded && ctx().peer && ctx().p2p_ok;
@@ -2021,6 +2026,7 @@ void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], doub
         double *thp = wk.theta.p;
         const uint8_t *lab = M.labels.p;
         double cw0 = cw[0], cw1 = cw[1], invn = inv_n, scale = wk.scale, inv_scale = wk.inv_scale;
+        double scale0 = wk.scale0, inv_scale0 = wk.inv_scale0;
         unsigned long long *Gp = G3.p;
         double *bl = blockloss.p;
         PgState *stp = st.p;
@@ -2039,8 +2045,8 @@ void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], doub
           lv.wbuf = wbuf.p; lv.nnz = M.nnz;
           if (long_mode == 2) { lv.bv_off = M.bv_off.p; lv.bv_pack = M.bv_pack.p; lv.bv_row_bits = M.bv_row_bits; }
         }
-        void *args[] = {&rows, &colp, &valp, &n, &nt, &thp, &lab, &cw0, &cw1, &invn, &scale, &Gp, &bl, &stp, &pass0, &npass,
-                        &inv_scale, &lam, &el, &stp_size, &eps, &mi, &pbp, &gx, &scr, &abortp, &lv};
+        void *args[] = {&rows, &colp, &valp, &n, &nt, &thp, &lab, &cw0, &cw1, &invn, &scale, &scale0, &Gp, &bl, &stp, &pass0,
+                        &npass, &inv_scale, &inv_scale0, &lam, &el, &stp_size, &eps, &mi, &pbp, &gx, &scr, &abortp, &lv};
         if (ctx().profiling) profile_begin("fused_small_persistent");
         const cudaError_t e = cudaLaunchCooperativeKernel(
             persistent_kernel<VT>(M.sharded, long_mode),
@@ -2065,14 +2071,15 @@ void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], doub
         dispatch_vt(M, [&](auto *tag) {
           using VT = typename std::remove_pointer<decltype(tag)>::type;
           KL_LAUNCH((fused_small_kernel<VT>), (unsigned)small_blocks, 256, 0, M.rows(), M.col.p, csr_val<VT>(M), M.n, ntheta,
-                    wk.theta.p, M.labels.p, cw[0], cw[1], inv_n, wk.scale, wk.G.p, blockloss.p, st.p, scatter,
-                    M.sharded ? (unsigned int *)nullptr : counter.p, wk.inv_scale, lambda, epsilon_loss, step, epsilon,
-                    (long long)max_iter);
+                    wk.theta.p, M.labels.p, cw[0], cw[1], inv_n, wk.scale, wk.scale0, wk.G.p, blockloss.p, st.p, scatter,
+                    M.sharded ? (unsigned int *)nullptr : counter.p, wk.inv_scale, wk.inv_scale0, lambda, epsilon_loss, step,
+                    epsilon, (long long)max_iter);
         });
         if (M.sharded && ctx().peer && ctx().p2p_ok) {
           // exchange over peer memory fused with the tail of the iteration
           KL_LAUNCH(small_p2p_tail_kernel, (unsigned)(ctx().world + 1), 256, 0, st.p, ctx().peer, blockloss.p, small_blocks, wk.theta.p, wk.G.p,
-                    wk.gathered.p, wk.inv_scale, ntheta, inv_n, lambda, epsilon_loss, step, epsilon, (long long)max_iter);
+                    wk.gathered.p, wk.inv_scale, wk.inv_scale0, ntheta, inv_n, lambda, epsilon_loss, step, epsilon,
+                    (long long)max_iter);
         } else if (M.sharded) {
           // gradient: exact int64 all-reduce; loss: per-rank sums gathered and added in rank order
           unsigned long long *slots = wk.G.p + ntheta;
@@ -2081,7 +2088,7 @@ void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], doub
           if (scatter) comm_allreduce_sum_i64((int64_t *)wk.G.p, ntheta + ctx().world);
           else comm_allreduce_sum_i64((int64_t *)slots, ctx().world);
           KL_LAUNCH(small_tail_kernel, 1, 256, 0, st.p, reinterpret_cast<const double *>(slots), ctx().world, wk.theta.p,
-                    wk.G.p, wk.inv_scale, ntheta, inv_n, lambda, epsilon_loss, step, epsilon, (long long)max_iter);
+                    wk.G.p, wk.inv_scale, wk.inv_scale0, ntheta, inv_n, lambda, epsilon_loss, step, epsilon, (long long)max_iter);
         }
         continue;
       }

@@ -40,9 +40,9 @@ def scale_exponents(val, cw):
     return ex(cmax * (vmax if vmax > 0.0 else 1.0)), ex(cmax * max(vmax, 1.0))
 
 
-def reference(n, m, rowptr, col, val, y, theta, cw):
+def reference(n, m, rowptr, col, val, y, theta, cw, serial=False):
     """z = X theta, the weights w_i and g_j = sum_i w_i v_ij in long double, with the allowed error of every z_i,
-    g_j and of the loss"""
+    g_j and of the loss.  serial: z sums a row in entry order (the reduced-matrix kernels), not in 32-lane strides"""
     rowptr = np.asarray(rowptr, dtype=np.int64)
     col = np.asarray(col, dtype=np.int32)
     val = np.asarray(val, dtype=np.float64)
@@ -53,8 +53,9 @@ def reference(n, m, rowptr, col, val, y, theta, cw):
     A = sp.csr_matrix((np.abs(val), col, rowptr), shape=(n, m))
     Z = abs(th[0]) + A @ np.abs(th[1:])                   # |theta_0| + sum_k |v_ik theta_k|
     q = np.diff(rowptr)
-    # z on the device: per-lane partial sums of 32-strided entries, a shuffle tree, theta_0, the products
-    kz = np.maximum(8, np.ceil(q / 32.0) + 7)
+    # z on the device: per-lane partial sums of 32-strided entries, a shuffle tree, theta_0, the products; or one
+    # serial sum of q products plus theta_0
+    kz = q + 2.0 if serial else np.maximum(8, np.ceil(q / 32.0) + 7)
     cw0, cw1, cmax = LD(cw[0]), LD(cw[1]), max(abs(cw[0]), abs(cw[1]))
     w = np.where(lab, -cw1 / (1 + np.exp(z)), cw0 / (1 + np.exp(-z))) / LD(n)
     term = np.where(lab, cw1 * np.logaddexp(LD(0), -z), cw0 * np.logaddexp(LD(0), z))
