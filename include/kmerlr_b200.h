@@ -102,6 +102,32 @@ int kmerlr_comm_destroy(void);
  *                   NULL/0 = one column per class (generate_features = true)
  */
 int kmerlr_sequences_create(const uint8_t *seq, const int64_t *off, int64_t n, kmerlr_handle *out);
+
+/* import_fasta (kmerLr_data.go:101-121): the bytes of n_texts FASTA files -> one resident sequence set, parsed and
+ * packed on the device.  Records of text 0 come first, then those of text 1, ...; records_out[t] = the records of
+ * text t (compile_training_data's fg || bg, compile_data's sets: one call each).  The rule, on bytes: lines end at
+ * '\n' (a lone '\r' is a byte of its line, not a break); every line is stripped of leading and trailing
+ * ' ', '\t', '\r', '\v', '\f' and skipped when empty; a line starting with '>' begins a record whose name is the rest
+ * of the line, stripped; every other line is appended to the current record as it is (bytes other than a/c/g/t in
+ * either case are invalid positions).  KMERLR_ERR_ARG: sequence data before the first header of a text, a text
+ * starting with the gzip magic 1f 8b (decompress it first). */
+int kmerlr_sequences_from_fasta(const uint8_t *const *texts, const int64_t *nbytes, int64_t n_texts,
+                                int64_t *records_out, kmerlr_handle *out);
+/* number of sequences, total bases, and the length of every sequence (len_out may be NULL) */
+int kmerlr_sequences_info(kmerlr_handle sequences, int64_t *n, int64_t *total_bases, int64_t *len_out_or_null);
+/* record names of a set from kmerlr_sequences_from_fasta (empty for other sets): name i =
+ * buf[name_off[i], name_off[i+1]), not terminated.  name_off[n+1] is always written; buf NULL = size query
+ * (name_off[n] bytes), otherwise buflen must be at least name_off[n]. */
+int kmerlr_sequences_names(kmerlr_handle sequences, char *buf_or_null, int64_t buflen, int64_t *name_off);
+/* the slicing of extractFasta (kmerLr_predict_genomic.go:93-112): a new set whose sequence i = bases
+ * [from[i], to[i]) of sequence seq_index[i], cut out of the packed set on the device.  KMERLR_ERR_ARG (GetSlice's
+ * error, log.Fatal there): an index out of range, from < 0, to > length or from > to.  Empty regions are allowed. */
+int kmerlr_sequences_regions(kmerlr_handle sequences, const int64_t *seq_index, const int64_t *from,
+                             const int64_t *to, int64_t n, kmerlr_handle *out);
+/* read-back (tests, debugging): the bases of every sequence one after the other, total_bases bytes, as 'a', 'c',
+ * 'g', 't' and 'n' at invalid positions */
+int kmerlr_sequences_bases(kmerlr_handle sequences, char *out);
+
 int kmerlr_extract_resident(const kmerlr_config *cfg, kmerlr_handle sequences,
                             const int32_t *frozen_k, const uint64_t *frozen_code, int64_t n_frozen,
                             const int32_t *features, int64_t n_features, int flags, kmerlr_handle *out);

@@ -18,7 +18,8 @@ SUMMARY = {"": 0, "mean": 1, "product": 2, "min": 3, "max": 4}
 SYMBOLS = [
     "kmerlr_init", "kmerlr_shutdown", "kmerlr_last_error", "kmerlr_version", "kmerlr_last_device_ms",
     "kmerlr_launch_count", "kmerlr_option", "kmerlr_profile", "kmerlr_profile_read", "kmerlr_profile_dump", "kmerlr_comm_unique_id", "kmerlr_comm_init", "kmerlr_comm_destroy",
-    "kmerlr_sequences_create", "kmerlr_extract_resident", "kmerlr_extract", "kmerlr_matrix_info", "kmerlr_matrix_rows_global",
+    "kmerlr_sequences_create", "kmerlr_sequences_from_fasta", "kmerlr_sequences_info", "kmerlr_sequences_names",
+    "kmerlr_sequences_regions", "kmerlr_sequences_bases", "kmerlr_extract_resident", "kmerlr_extract", "kmerlr_matrix_info", "kmerlr_matrix_rows_global",
     "kmerlr_matrix_classes", "kmerlr_column_moments", "kmerlr_pair_moments", "kmerlr_matrix_transform", "kmerlr_matrix_rows", "kmerlr_matrix_set_labels", "kmerlr_matrix_from_csr",
     "kmerlr_free", "kmerlr_coeff_dim", "kmerlr_coeff_ind2sub", "kmerlr_coeff_sub2ind", "kmerlr_linear_pdf",
     "kmerlr_logpdf", "kmerlr_gradient", "kmerlr_loss", "kmerlr_class_weights", "kmerlr_select", "kmerlr_select_from_gradient", "kmerlr_reduce",
@@ -72,6 +73,11 @@ def lib():
     L.kmerlr_comm_unique_id.argtypes = [vp]
     L.kmerlr_comm_init.argtypes = [C.c_int, C.c_int, vp]
     L.kmerlr_sequences_create.argtypes = [vp, vp, i64, ph]
+    L.kmerlr_sequences_from_fasta.argtypes = [vp, vp, i64, vp, ph]
+    L.kmerlr_sequences_info.argtypes = [h, pi64, pi64, vp]
+    L.kmerlr_sequences_names.argtypes = [h, vp, i64, vp]
+    L.kmerlr_sequences_regions.argtypes = [h, vp, vp, vp, i64, ph]
+    L.kmerlr_sequences_bases.argtypes = [h, vp]
     L.kmerlr_extract_resident.argtypes = [C.POINTER(Config), h, vp, vp, i64, vp, i64, C.c_int, ph]
     L.kmerlr_extract.argtypes = [C.POINTER(Config), vp, vp, i64, vp, vp, i64, vp, i64, C.c_int, ph]
     L.kmerlr_matrix_info.argtypes = [h, pi64, pi64, pi64, pi64]

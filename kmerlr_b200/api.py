@@ -126,7 +126,11 @@ class CoeffIndex(int):
 # data (kmerLr_data.go)
 # ---------------------------------------------------------------------------------------------------
 class Sequences:
-    """2-bit packed sequences resident in HBM."""
+    """2-bit packed sequences resident in HBM.  A set parsed from FASTA text (import_fasta) also carries the
+    record names (.names) and the number of records of every text (.records); for other sets both are None."""
+
+    names = None
+    records = None
 
     def __init__(self, seqs):
         buf, off = flatten(seqs)
@@ -136,12 +140,83 @@ class Sequences:
         check(lib().kmerlr_sequences_create(_p(buf), _p(off), self.n, h))
         self.h = h.value
 
+    @classmethod
+    def _resident(cls, handle):
+        s = cls.__new__(cls)
+        s.h = handle
+        n, total = C.c_int64(), C.c_int64()
+        check(lib().kmerlr_sequences_info(handle, n, total, None))
+        s.n, s.total_bases = n.value, total.value
+        return s
+
+    def lengths(self):
+        out = np.zeros(max(self.n, 1), dtype=np.int64)
+        check(lib().kmerlr_sequences_info(self.h, None, None, _p(out)))
+        return out[:self.n]
+
+    def bases(self):
+        """the bases of every sequence one after the other as b"acgt", b"n" at invalid positions (read-back)"""
+        out = np.zeros(max(self.total_bases, 1), dtype=np.uint8)
+        check(lib().kmerlr_sequences_bases(self.h, _p(out)))
+        return out[:self.total_bases].tobytes()
+
+    def regions(self, seq_index, from_, to):
+        """the slicing of extractFasta (kmerLr_predict_genomic.go:93-112): sequence i of the new set is bases
+        [from_[i], to[i]) of sequence seq_index[i], cut out on the device"""
+        idx = np.ascontiguousarray(seq_index, dtype=np.int64)
+        frm = np.ascontiguousarray(from_, dtype=np.int64)
+        to = np.ascontiguousarray(to, dtype=np.int64)
+        if not len(idx) == len(frm) == len(to):
+            raise KmerLrError(_lib.ERR_ARG, "regions: seq_index, from and to differ in length")
+        h = C.c_uint64()
+        check(lib().kmerlr_sequences_regions(self.h, _p(idx), _p(frm), _p(to), len(idx), h))
+        return Sequences._resident(h.value)
+
     def free(self):
         if getattr(self, "h", 0):
             lib().kmerlr_free(self.h)
             self.h = 0
 
     __del__ = free
+
+
+def _host_bytes(t):
+    """a text as a contiguous uint8 array without a copy where the buffer allows it"""
+    if isinstance(t, np.ndarray):
+        return np.ascontiguousarray(t).view(np.uint8).reshape(-1)
+    return np.frombuffer(t, dtype=np.uint8) if len(t) else np.zeros(0, dtype=np.uint8)
+
+
+def import_fasta(*texts):
+    """import_fasta (kmerLr_data.go:101-121) for the bytes of one or more FASTA files (bytes, bytearray, memoryview
+    or uint8 arrays): one resident Sequences with the records of text 0 first, then text 1, ...; .names are the
+    record names (the whole header line after '>', stripped), .records the number of records of every text.  The
+    caller decompresses gzip files."""
+    arrs = [_host_bytes(t) for t in texts]
+    ptrs = (C.c_void_p * max(len(arrs), 1))(*[a.ctypes.data if len(a) else None for a in arrs])
+    nbytes = np.array([len(a) for a in arrs] or [0], dtype=np.int64)
+    records = np.zeros(max(len(arrs), 1), dtype=np.int64)
+    h = C.c_uint64()
+    check(lib().kmerlr_sequences_from_fasta(ptrs, _p(nbytes), len(arrs), _p(records), h))
+    s = Sequences._resident(h.value)
+    s.records = records[:len(arrs)].tolist()
+    off = np.zeros(s.n + 1, dtype=np.int64)
+    check(lib().kmerlr_sequences_names(s.h, None, 0, _p(off)))
+    buf = C.create_string_buffer(max(int(off[-1]), 1))
+    check(lib().kmerlr_sequences_names(s.h, buf, len(buf), _p(off)))
+    raw = buf.raw
+    s.names = [raw[off[i]:off[i + 1]].decode("utf-8", "surrogateescape") for i in range(s.n)]
+    return s
+
+
+def _text_sets(seqs):
+    """the sets of a FASTA-parsed Sequences, one per text it was read from, as resident copies (whole records)"""
+    lens, sets, r = seqs.lengths(), [], 0
+    for k in seqs.records:
+        idx = np.arange(r, r + k, dtype=np.int64)
+        sets.append(seqs.regions(idx, np.zeros(k, dtype=np.int64), lens[r:r + k]))
+        r += k
+    return sets
 
 
 class KmerDataSet:
@@ -252,13 +327,20 @@ def _convert(cfg, seqs, kmers, features, generate_features, sharded):
     return data
 
 
-def compile_training_data(config, kmersCounter, kmers, features, generate_features, binarize, fg, bg,
+def compile_training_data(config, kmersCounter, kmers, features, generate_features, binarize, fg, bg=None,
                           sharded=False):
     """compile_training_data (kmerLr_data.go:306-325).  fg / bg are the sequences import_fasta returned
-    (lists of str/bytes, or (buffer, offsets)); labels = true for fg."""
+    (lists of str/bytes, or (buffer, offsets)); labels = true for fg.  Or fg = the resident set of
+    import_fasta(fg_text, bg_text) and bg = None: its records per text give the labels."""
     del config
     cfg = Config.from_buffer_copy(kmersCounter)
     cfg.binarize = int(binarize)
+    if isinstance(fg, Sequences):
+        if bg is not None or fg.records is None or len(fg.records) != 2:
+            raise KmerLrError(_lib.ERR_ARG, "compile_training_data: a resident set must come from import_fasta(fg, bg)")
+        data = _convert(cfg, fg, kmers, features, generate_features, sharded)
+        data.SetLabels(np.concatenate([np.ones(fg.records[0], dtype=np.uint8), np.zeros(fg.records[1], dtype=np.uint8)]))
+        return data
     fb, fo = flatten(fg)
     bb, bo = flatten(bg)
     nfg, nbg = len(fo) - 1, len(bo) - 1
@@ -270,7 +352,8 @@ def compile_training_data(config, kmersCounter, kmers, features, generate_featur
 
 
 def compile_test_data(config, kmersCounter, kmers, features, generate_features, binarize, sequences):
-    """compile_test_data (kmerLr_data.go:327-335): counter frozen to the classifier's k-mers."""
+    """compile_test_data (kmerLr_data.go:327-335): counter frozen to the classifier's k-mers.  sequences may be a
+    resident set (Sequences, import_fasta)."""
     del config
     cfg = Config.from_buffer_copy(kmersCounter)
     cfg.binarize = int(binarize)
@@ -281,10 +364,23 @@ def compile_data(config, kmersCounter, kmers, features, generate_features, binar
     """compile_data (kmerLr_data.go:339-358): several sequence sets, ONE class numbering (the union of the
     classes observed in all of them, or the supplied list), one KmerDataSet per set.  The union comes from one
     extraction over the concatenation; every set is then extracted against that frozen list, which gives the
-    rows `counts_list.Slice(k[i], k[i+1])` would."""
+    rows `counts_list.Slice(k[i], k[i+1])` would.  sequence_sets may also be the resident set of
+    import_fasta(text_0, text_1, ...): one data set per text."""
     del config
     cfg = Config.from_buffer_copy(kmersCounter)
     cfg.binarize = int(binarize)
+    if isinstance(sequence_sets, Sequences):
+        if sequence_sets.records is None:
+            raise KmerLrError(_lib.ERR_ARG, "compile_data: a resident set must come from import_fasta")
+        if kmers is None or len(kmers[0]) == 0:
+            joint = _extract(cfg, sequence_sets, None, None, False)
+            kmers = joint.Kmers()
+            joint.free()
+        sets = _text_sets(sequence_sets)
+        out = [_convert(cfg, s, kmers, features, generate_features, False) for s in sets]
+        for s in sets:
+            s.free()
+        return out
     sets = [flatten(s) for s in sequence_sets]
     if kmers is None or len(kmers[0]) == 0:
         buf = np.concatenate([b[:o[-1]] for b, o in sets] + [np.zeros(1, dtype=np.uint8)])
@@ -670,6 +766,7 @@ class genomicKmerLr:
         return res
 
     def predict_resident(self, sequences, window_size, window_step, fetch=False, total_slots=0):
+        """scores of a resident set (Sequences, import_fasta, Sequences.regions); fetch: the total_slots scores"""
         out = np.zeros(max(total_slots, 1)) if fetch else None
         check(lib().kmerlr_score_windows_resident(self._arr, len(self.classifiers), sequences.h, window_size,
                                                   window_step, _p(out), None))

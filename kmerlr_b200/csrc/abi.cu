@@ -273,6 +273,56 @@ int kmerlr_sequences_create(const uint8_t *seq, const int64_t *off, int64_t n, k
   });
 }
 
+// import_fasta (kmerLr_data.go:101-121)
+int kmerlr_sequences_from_fasta(const uint8_t *const *texts, const int64_t *nbytes, int64_t n_texts,
+                                int64_t *records_out, kmerlr_handle *out) {
+  return guarded([&] {
+    KL_REQUIRE(out, "null output handle");
+    *out = register_object(sequences_from_fasta(texts, nbytes, n_texts, records_out));
+  });
+}
+
+int kmerlr_sequences_info(kmerlr_handle sequences, int64_t *n, int64_t *total_bases, int64_t *len_out_or_null) {
+  return guarded([&] {
+    auto s = lookup<SeqSet>(sequences, "sequences");
+    if (n) *n = s->n;
+    if (total_bases) *total_bases = s->total_bases;
+    if (len_out_or_null && s->n) {
+      s->len.download(len_out_or_null, (size_t)s->n);
+      sync_stream();
+    }
+  }, false);
+}
+
+int kmerlr_sequences_names(kmerlr_handle sequences, char *buf_or_null, int64_t buflen, int64_t *name_off) {
+  return guarded([&] {
+    KL_REQUIRE(name_off, "null argument");
+    auto s = lookup<SeqSet>(sequences, "sequences");
+    const bool named = (int64_t)s->name_off.size() == s->n + 1;
+    for (int64_t i = 0; i <= s->n; i++) name_off[i] = named ? s->name_off[(size_t)i] : 0;
+    if (!buf_or_null) return;
+    KL_REQUIRE(buflen >= name_off[s->n], "sequences_names: buffer too small");
+    if (name_off[s->n]) memcpy(buf_or_null, s->names.data(), (size_t)name_off[s->n]);
+  }, false);
+}
+
+// the slicing of extractFasta (kmerLr_predict_genomic.go:93-112)
+int kmerlr_sequences_regions(kmerlr_handle sequences, const int64_t *seq_index, const int64_t *from,
+                             const int64_t *to, int64_t n, kmerlr_handle *out) {
+  return guarded([&] {
+    KL_REQUIRE(out, "null output handle");
+    *out = register_object(sequences_regions(*lookup<SeqSet>(sequences, "sequences"), seq_index, from, to, n));
+  });
+}
+
+int kmerlr_sequences_bases(kmerlr_handle sequences, char *out) {
+  return guarded([&] {
+    auto s = lookup<SeqSet>(sequences, "sequences");
+    KL_REQUIRE(out || s->total_bases == 0, "null argument");
+    sequences_letters(*s, out);
+  });
+}
+
 int kmerlr_extract_resident(const kmerlr_config *cfg, kmerlr_handle sequences, const int32_t *frozen_k,
                             const uint64_t *frozen_code, int64_t n_frozen, const int32_t *features,
                             int64_t n_features, int flags, kmerlr_handle *out) {

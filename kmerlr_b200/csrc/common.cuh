@@ -221,6 +221,10 @@ struct SeqSet : Object {
   DevBuf<int64_t> blk;      // n+1, in 64-base blocks
   DevBuf<uint32_t> bits2;   // total_blocks*4
   DevBuf<uint16_t> inv16;   // total_blocks*4
+  // record names of a set parsed from FASTA text (fasta.cu): name i = names[name_off[i], name_off[i+1]); empty
+  // for every other set
+  std::string names;
+  std::vector<int64_t> name_off;
 };
 
 enum ValType : int { VAL_ONE = 0, VAL_U32 = 1, VAL_F64 = 2 };
@@ -382,6 +386,12 @@ std::shared_ptr<Matrix> extract(const kmerlr_config &cfg, std::shared_ptr<SeqSet
 std::shared_ptr<Matrix> extract_host(const kmerlr_config &cfg, const uint8_t *seq, const int64_t *off, int64_t n,
                                      const int32_t *frozen_k, const uint64_t *frozen_code, int64_t n_frozen,
                                      const int32_t *features, int64_t n_features, int flags);
+// fasta.cu
+std::shared_ptr<SeqSet> sequences_from_fasta(const uint8_t *const *texts, const int64_t *nbytes, int64_t n_texts,
+                                             int64_t *records_out);
+std::shared_ptr<SeqSet> sequences_regions(const SeqSet &src, const int64_t *seq_index, const int64_t *from,
+                                          const int64_t *to, int64_t n);
+void sequences_letters(const SeqSet &s, char *out);   // total_bases bytes: a/c/g/t, 'n' at invalid positions
 // gapped.cu
 std::shared_ptr<Matrix> extract_gapped(const kmerlr_config &cfg, std::shared_ptr<SeqSet> seqs, const int32_t *frozen_k,
                                        const uint64_t *frozen_code, int64_t n_frozen, int flags);
