@@ -6,6 +6,7 @@
 #include <stdint.h>
 
 #include <chrono>
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -460,6 +461,14 @@ void comm_allreduce_max_u8(uint8_t *dev, int64_t count);
 void comm_allgather_f64(const double *dev_in, double *dev_out, int64_t count_per_rank);
 void comm_allgather_bytes(const void *dev_in, void *dev_out, int64_t bytes_per_rank);
 
+// exponent e of the fixed-point sums (scale 2^e): 60 - ceil(log2(bound)), so a sum bounded by `bound` stays below
+// 2^60.  Clamped so that 2^e and 2^-e stay finite; a bound of 0 (an empty matrix) takes the exponent of 1
+inline int fixed_point_exponent(double bound) {
+  if (!(bound > 0.0) || !std::isfinite(bound)) bound = 1.0;
+  const int e = 60 - (int)std::ceil(std::log2(bound));
+  return e > 1000 ? 1000 : e;
+}
+
 // ---------------------------------------------------------------------------------------------
 // device helpers
 // ---------------------------------------------------------------------------------------------
@@ -522,6 +531,23 @@ __device__ __forceinline__ void mbar_wait(unsigned long long *bar, uint32_t pari
 // max(0,x) + log1p(exp(-|x|))  (kmerLr_logistic_regression.go:138-145)
 __device__ __forceinline__ double log_add0(double x) {
   return x > 0.0 ? x + log1p(exp(-x)) : log1p(exp(x));
+}
+
+// value of CSR entry p; val == nullptr: a binarized matrix, every stored entry is 1
+template <typename VT>
+__device__ __forceinline__ double valf(const VT *val, int64_t p) { return val ? (double)val[p] : 1.0; }
+
+// proximal step of the L1 penalty on one coefficient: sign(x) max(|x| - t, 0) (kmerLr_estimator_proximal.go:88-98)
+__device__ __forceinline__ double soft_threshold(double x, double t) {
+  return x >= 0.0 ? fmax(fabs(x) - t, 0.0) : -fmax(fabs(x) - t, 0.0);
+}
+
+// eval_stopping (kmerLr_estimator_proximal.go:30-52) from max |x1|, max |x1 - x0| and whether x1 holds a NaN:
+// delta = max|dx| / max|x| (max|dx| when x = 0, NaN on a NaN); stop when delta <= eps, on x = dx = 0 or on a NaN
+__host__ __device__ __forceinline__ bool eval_stopping(double mx, double md, bool nan_seen, double eps, double *delta) {
+  if (nan_seen) { *delta = nan(""); return true; }
+  *delta = mx != 0.0 ? md / mx : md;
+  return (mx != 0.0 && md / mx <= eps) || (mx == 0.0 && md == 0.0);
 }
 #endif
 

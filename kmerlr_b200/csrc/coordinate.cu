@@ -35,9 +35,6 @@ struct CdScales {
   double xy0, xy, xx00, xx0c, xxcc;
 };
 
-template <typename VT>
-__device__ __forceinline__ double cd_val(const VT *val, int64_t p) { return val ? (double)val[p] : 1.0; }
-
 // row pass: Gram and xy of the weighted least-squares problem of this outer iteration
 template <typename VT>
 __global__ void __launch_bounds__(256) cd_rows_kernel(const Rows R, const uint32_t *__restrict__ col,
@@ -54,7 +51,7 @@ __global__ void __launch_bounds__(256) cd_rows_kernel(const Rows R, const uint32
   int64_t a, b;
   R.range(row, a, b);
   double s = 0.0;
-  for (int64_t p = a; p < b; p++) s += cd_val(val, p) * sth[col[p] + 1];
+  for (int64_t p = a; p < b; p++) s += valf(val, p) * sth[col[p] + 1];
   const double r = sth[0] + s;                                   // LinearPdf (:98)
   const double pr = exp(-log_add0(-r));                          // (:99)
   double w = pr * (1.0 - pr);                                    // (:100)
@@ -66,13 +63,13 @@ __global__ void __launch_bounds__(256) cd_rows_kernel(const Rows R, const uint32
   // entry -1 = the bias column (index 0, value 1)
   for (int64_t p1 = a - 1; p1 < b; p1++) {
     const int64_t j1 = p1 < a ? 0 : (int64_t)col[p1] + 1;
-    const double v1 = p1 < a ? 1.0 : cd_val(val, p1);
+    const double v1 = p1 < a ? 1.0 : valf(val, p1);
     atomicAdd((unsigned long long *)&XY[j1], (unsigned long long)__double2ll_rn(wz * v1 * (j1 == 0 ? S.xy0 : S.xy)));
     const double wv1 = w * v1;
     const double sb = j1 == 0 ? S.xx00 : S.xx0c, sc = j1 == 0 ? S.xx0c : S.xxcc;     // the scales of (j1, bias), (j1, column)
     for (int64_t p2 = a - 1; p2 < b; p2++) {
       const int64_t j2 = p2 < a ? 0 : (int64_t)col[p2] + 1;
-      const double v2 = p2 < a ? 1.0 : cd_val(val, p2);
+      const double v2 = p2 < a ? 1.0 : valf(val, p2);
       atomicAdd((unsigned long long *)&XX[j1 * ntheta + j2],
                 (unsigned long long)__double2ll_rn(wv1 * v2 * (j2 == 0 ? sb : sc)));
     }
@@ -118,10 +115,7 @@ __global__ void __launch_bounds__(CD_THREADS) cd_sweep_kernel(const double *__re
       const double norm = xx[j * ntheta + j];
       double tj = xy[j] + norm * sth[j];
       tj -= dot;
-      if (j > 0) {
-        if (tj >= 0.0) tj =  fmax(fabs(tj) - l1, 0.0);
-        else           tj = -fmax(fabs(tj) - l1, 0.0);
-      }
+      if (j > 0) tj = soft_threshold(tj, l1);
       tj /= (norm + l2);
       const double old = sth[j];
       sth[j] = tj;
@@ -132,34 +126,7 @@ __global__ void __launch_bounds__(CD_THREADS) cd_sweep_kernel(const double *__re
     __syncthreads();
   }
   for (int i = t; i < ntheta; i += CD_THREADS) theta[i] = sth[i];
-  if (t == 0) {
-    // eval_stopping (kmerLr_estimator_proximal.go:30-52)
-    if (isnan_seen) { st->delta = nan(""); st->stop = 1; }
-    else {
-      st->delta = max_x != 0.0 ? max_d / max_x : max_d;
-      st->stop = ((max_x != 0.0 && max_d / max_x <= eps) || (max_x == 0.0 && max_d == 0.0)) ? 1 : 0;
-    }
-  }
-}
-
-// 60 - ceil(log2(bound)): a sum bounded by `bound` stays below 2^60.  Clamped like scale_exponent (logistic.cu) so
-// that 2^e and 2^-e stay finite; a bound of 0 (an empty matrix) takes the exponent of 1
-int cd_exponent(double bound) {
-  if (!(bound > 0.0) || !std::isfinite(bound)) bound = 1.0;
-  const int e = 60 - (int)std::ceil(std::log2(bound));
-  return e > 1000 ? 1000 : e;
-}
-
-// eval_stopping on the host for the outer iteration (two short vectors)
-bool eval_stopping_host(const std::vector<double> &x0, const std::vector<double> &x1, double eps, double *delta) {
-  double max_x = 0.0, max_d = 0.0;
-  for (size_t i = 0; i < x1.size(); i++) {
-    if (std::isnan(x1[i])) { *delta = NAN; return true; }
-    max_x = std::fmax(max_x, std::fabs(x1[i]));
-    max_d = std::fmax(max_d, std::fabs(x1[i] - x0[i]));
-  }
-  *delta = max_x != 0.0 ? max_d / max_x : max_d;
-  return (max_x != 0.0 && max_d / max_x <= eps) || (max_x == 0.0 && max_d == 0.0);
+  if (t == 0) st->stop = eval_stopping(max_x, max_d, isnan_seen, eps, &st->delta) ? 1 : 0;
 }
 
 }  // namespace
@@ -212,10 +179,11 @@ void coordinate(Matrix &M, double *theta, int64_t ntheta, const double cw_hook[2
     const double rmax = std::fabs(th1[0]) + std::sqrt(th2 * maxsq);
     const double bxy0 = (double)M.n * cwmax * v1 * (0.25 * rmax + 1.0);
     if (!(bxy0 > 0.0) || !std::isfinite(bxy0)) { nan_abort = true; break; }
-    const int exy0 = cd_exponent(bxy0), exy = cd_exponent((double)M.n * cwmax * vmax * (0.25 * rmax + 1.0));
-    const int exx00 = cd_exponent((double)M.n * 0.25 * cwmax * v1 * v1),
-              exx0c = cd_exponent((double)M.n * 0.25 * cwmax * v1 * vmax),
-              exxcc = cd_exponent((double)M.n * 0.25 * cwmax * vmax * vmax);
+    const int exy0 = fixed_point_exponent(bxy0),
+              exy = fixed_point_exponent((double)M.n * cwmax * vmax * (0.25 * rmax + 1.0));
+    const int exx00 = fixed_point_exponent((double)M.n * 0.25 * cwmax * v1 * v1),
+              exx0c = fixed_point_exponent((double)M.n * 0.25 * cwmax * v1 * vmax),
+              exxcc = fixed_point_exponent((double)M.n * 0.25 * cwmax * vmax * vmax);
     const CdScales S{std::ldexp(1.0, exy0), std::ldexp(1.0, exy), std::ldexp(1.0, exx00), std::ldexp(1.0, exx0c),
                      std::ldexp(1.0, exxcc)};
     const CdScales inv{std::ldexp(1.0, -exy0), std::ldexp(1.0, -exy), std::ldexp(1.0, -exx00), std::ldexp(1.0, -exx0c),
@@ -247,8 +215,15 @@ void coordinate(Matrix &M, double *theta, int64_t ntheta, const double cw_hook[2
       if (hs.stop) break;
       if (run_hook(th1)) break;
     }
-    // (:117-125)
-    if (eval_stopping_host(th0, th1, epsilon, &delta)) break;
+    // (:117-125) eval_stopping over the outer iteration
+    double max_x = 0.0, max_d = 0.0;
+    bool isnan_seen = false;
+    for (int64_t k = 0; k < ntheta && !isnan_seen; k++) {
+      isnan_seen = std::isnan(th1[k]);
+      max_x = std::fmax(max_x, std::fabs(th1[k]));
+      max_d = std::fmax(max_d, std::fabs(th1[k] - th0[k]));
+    }
+    if (eval_stopping(max_x, max_d, isnan_seen, epsilon, &delta)) break;
     if (run_hook(th1)) break;
   }
   if (nan_abort) {

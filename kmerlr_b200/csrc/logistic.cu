@@ -32,12 +32,29 @@ struct PgState {
   int error;         // 1: a peer never answered the gradient exchange
 };
 
+// the hook's state transition (kmerLr_estimator_hook.go:46-99) for the loss l at the current theta
+__device__ __forceinline__ void hook_update(PgState *st, double l, double eps_loss) {
+  st->lossval = l;
+  if (st->first) { st->first = 0; return; }   // loss at the start point: no hook call yet
+  const double t = st->loss_old; st->loss_old = st->loss_new; st->loss_new = t;
+  if (eps_loss != 0.0) {
+    st->loss_new = l;
+    if (st->done == 0 && fabs(st->loss_old - st->loss_new) < eps_loss) st->done = 1;
+  }
+  if (st->done == 2) st->done = 1;
+}
+
+// end of a prox step: eval_stopping on max |theta|, max |delta| and the NaN flag of the new theta; after max_iter
+// steps one more pass evaluates the hook's loss (done = 2)
+__device__ __forceinline__ void pg_stop(PgState *st, double mx, double md, double nn, double eps, long long max_iter) {
+  st->iter += 1;
+  if (eval_stopping(mx, md, nn != 0.0, eps, &st->delta)) st->done = 1;
+  else if (st->iter >= max_iter) st->done = 2;
+}
+
 __device__ __forceinline__ int64_t ind2sub(int64_t n, int64_t k1, int64_t k2) {
   return n + (n * (n - 1) / 2) - (n - k1) * ((n - k1) - 1) / 2 + k2 - k1;
 }
-
-template <typename VT>
-__device__ __forceinline__ double valf(const VT *val, int64_t p) { return val ? (double)val[p] : 1.0; }
 
 // a non-zero pair coefficient theta[Ind2Sub(a, b)], a < b (pair mode with a sparse theta)
 struct PairTerm {
@@ -51,6 +68,19 @@ __device__ __forceinline__ double row_value(const uint32_t *__restrict__ col, co
   int64_t lo = a, hi = b;
   while (lo < hi) { const int64_t mid = (lo + hi) >> 1; if (col[mid] < c) lo = mid + 1; else hi = mid; }
   return (lo < b && col[lo] == c) ? valf(val, lo) : 0.0;
+}
+
+// Gradient weight (kmerLr_logistic_regression.go:166-178) and Loss term (:257-263) of a row with label y and
+// z = x theta: returns w, the loss term goes to `lossterm`.  The label and the weights are references so that they
+// are read where the formula uses them: read ahead of the logarithm, they stay live across it and ptxas spills in
+// imp_pass<8, true>.
+__device__ __forceinline__ double row_weight(double z, const uint8_t &y, const double &cw0, const double &cw1, const double &inv_n,
+                                             double &lossterm) {
+  const double r = -log_add0(-z);
+  double w;
+  if (y) { w = inv_n * cw1 * (exp(r) - 1.0); lossterm = -cw1 * r; }
+  else   { w = inv_n * cw0 * exp(r);         lossterm = cw0 * log_add0(z); }
+  return w;
 }
 
 // rows pass: MODE 0 = z only, 1 = log sigma(z), 2 = w_i and loss term.
@@ -91,37 +121,26 @@ __global__ void rows_kernel(const Rows R, const uint32_t *__restrict__ col,
     double z = theta[0] + s;
     if (MODE == 0) out[row] = z;
     else if (MODE == 1) out[row] = -log_add0(-z);
-    else {
-      // Gradient weight (:166-178) and Loss term (:257-263)
-      double r = -log_add0(-z);
-      if (labels[row]) { out[row] = inv_n * cw1 * (exp(r) - 1.0); lossterm[row] = -cw1 * r; }
-      else             { out[row] = inv_n * cw0 * exp(r);         lossterm[row] = cw0 * log_add0(z); }
-    }
+    else out[row] = row_weight(z, labels[row], cw0, cw1, inv_n, lossterm[row]);
   }
 }
 
-// deterministic sum of x[0..n): fixed grid, strided sequential sums, fixed tree
-__global__ void reduce_stage1(const double *__restrict__ x, int64_t n, double *__restrict__ part, const PgState *st) {
-  if (st && st->done == 1) return;
-  __shared__ double sh[256];
-  double s = 0.0;
-  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) s += x[i];
-  sh[threadIdx.x] = s;
-  __syncthreads();
-  for (int o = 128; o > 0; o >>= 1) {
-    if ((int)threadIdx.x < o) sh[threadIdx.x] += sh[threadIdx.x + o];
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) part[blockIdx.x] = sh[0];
+// 64-bit accumulators as two 32-bit words (acc_lo[c], acc_hi[c]): shared memory has native 32-bit atomic adds only (a
+// 64-bit add would be a compare-and-swap loop); the carry out of the low word is added to the high word by the thread
+// whose add wrapped, so the pair is an exact 64-bit sum
+__device__ __forceinline__ void acc64_add(uint32_t *acc_lo, uint32_t *acc_hi, uint32_t c, unsigned long long q) {
+  const uint32_t lo = (uint32_t)q, hi = (uint32_t)(q >> 32);
+  const uint32_t old = atomicAdd(&acc_lo[c], lo);
+  const uint32_t add_hi = hi + ((old + lo) < old ? 1u : 0u);
+  if (add_hi) atomicAdd(&acc_hi[c], add_hi);
 }
-// out[0] = sum(part): one warp, lane l adds part[l], part[l + 32], ... in index order, then a fixed shuffle tree
-// (deterministic; a single thread walking the 256 partials took 25 us of dependent loads)
-__global__ void reduce_stage2(const double *__restrict__ part, int np, double *__restrict__ out, const PgState *st) {
-  if (st && st->done == 1) return;
-  double s = 0.0;
-  for (int i = threadIdx.x; i < np; i += 32) s += part[i];
-  s = warp_sum_down(s);
-  if (threadIdx.x == 0) out[0] = s;
+// G[i] += the pair i for i < count, by the threads of the block once its adds are done (after a barrier).  `count` is
+// an int: a 64-bit bound widens the loop index and ptxas spills in fused_kernel<uint32_t>.
+__device__ __forceinline__ void acc64_flush(const uint32_t *acc_lo, const uint32_t *acc_hi, int count, unsigned long long *G) {
+  for (int i = threadIdx.x; i < count; i += blockDim.x) {
+    const unsigned long long v = ((unsigned long long)acc_hi[i] << 32) | acc_lo[i];
+    if (v) atomicAdd(&G[i], v);
+  }
 }
 
 // the fused pass over the stored rows: one warp per row
@@ -147,9 +166,6 @@ __global__ void __launch_bounds__(256) fused_kernel(const Rows R, const uint32_t
                                                     double *__restrict__ lossterm, const PgState *st, int scatter,
                                                     int hot_limit, int rpb, unsigned long long *__restrict__ ticket) {
   if (st && st->done == 1) return;
-  // 64-bit accumulators as two 32-bit words: shared memory has native 32-bit atomic adds only
-  // (a 64-bit add would be a compare-and-swap loop); the carry out of the low word is added to
-  // the high word by the thread whose add wrapped, so the pair is an exact 64-bit sum
   extern __shared__ uint32_t hot_smem[];
   uint32_t *hot_lo = hot_smem, *hot_hi = hot_smem + hot_limit;
   const int64_t hot_cols = m < hot_limit ? m : hot_limit;
@@ -165,10 +181,7 @@ __global__ void __launch_bounds__(256) fused_kernel(const Rows R, const uint32_t
     s = warp_sum_down(s);
     double w = 0.0;
     if (lane == 0) {
-      // Gradient weight (:166-178) and Loss term (:257-263)
-      double z = theta[0] + s, r = -log_add0(-z);
-      if (labels[row]) { w = inv_n * cw1 * (exp(r) - 1.0); lossterm[row] = -cw1 * r; }
-      else             { w = inv_n * cw0 * exp(r);         lossterm[row] = cw0 * log_add0(z); }
+      w = row_weight(theta[0] + s, labels[row], cw0, cw1, inv_n, lossterm[row]);
       bias_acc += __double2ll_rn(w * scale0);
     }
     if (!scatter) return;                 // loss-only pass (the hook after the last iteration)
@@ -177,12 +190,8 @@ __global__ void __launch_bounds__(256) fused_kernel(const Rows R, const uint32_t
     for (int64_t p = a + lane; p < b; p += 32) {
       const uint32_t c = col[p];
       const unsigned long long q = (unsigned long long)__double2ll_rn(ws * valf(val, p));
-      if (c < (uint32_t)hot_cols) {
-        const uint32_t lo = (uint32_t)q, hi = (uint32_t)(q >> 32);
-        const uint32_t old = atomicAdd(&hot_lo[c], lo);
-        const uint32_t add_hi = hi + ((old + lo) < old ? 1u : 0u);
-        if (add_hi) atomicAdd(&hot_hi[c], add_hi);
-      } else atomicAdd(&G[c + 1], q);
+      if (c < (uint32_t)hot_cols) acc64_add(hot_lo, hot_hi, c, q);
+      else atomicAdd(&G[c + 1], q);
     }
   };
   if (ticket) {
@@ -200,10 +209,7 @@ __global__ void __launch_bounds__(256) fused_kernel(const Rows R, const uint32_t
   }
   if (lane == 0 && bias_acc != 0) atomicAdd(&G[0], (unsigned long long)bias_acc);
   __syncthreads();
-  for (int i = threadIdx.x; i < hot_cols; i += blockDim.x) {
-    unsigned long long v = ((unsigned long long)hot_hi[i] << 32) | hot_lo[i];
-    if (v) atomicAdd(&G[i + 1], v);
-  }
+  acc64_flush(hot_lo, hot_hi, hot_cols, G + 1);
 }
 
 // ---- matrix-free pass (matrices straight from the extraction, Matrix::imp) ----------------------------
@@ -264,6 +270,19 @@ __global__ void imp_build_TS(const ImpParams P, double *__restrict__ T, const Pg
   T[P.sup0 + U] = s;
 }
 
+// true in every thread of the block that arrives last at `ticket` (one arrival per block of the grid): its reads
+// then see what the other blocks wrote before they arrived.  The caller resets the ticket.
+__device__ __forceinline__ bool last_block(unsigned int *ticket) {
+  __shared__ int s_last;
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) s_last = atomicAdd(ticket, 1u) == gridDim.x - 1 ? 1 : 0;
+  __syncthreads();
+  if (!s_last) return false;
+  __threadfence();
+  return true;
+}
+
 // The fold of the forward-code tables after the pass, F_j[u] = H_j[u] + F_{j+1}[4u .. 4u+3] from level N-1 down to
 // Mlo, preceded by H[N][N-mer at offset t of U] += HS[U] when there is a super level.  The grid of one launch folds
 // `level` (P.N: the super level into level N) -- the large steps, one launch each; the block that finishes last then
@@ -287,14 +306,7 @@ __global__ void __launch_bounds__(IMP_FOLD_THREADS) imp_fold(const ImpParams P, 
     const unsigned long long *c = H + P.fo[level + 1] + 4ull * u;
     H[P.fo[level] + u] += c[0] + c[1] + c[2] + c[3];
   }
-  if (tail_top < P.Mlo) return;
-  __shared__ int s_last;
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) s_last = atomicAdd(ticket, 1u) == gridDim.x - 1 ? 1 : 0;
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
+  if (tail_top < P.Mlo || !last_block(ticket)) return;
   for (int j = tail_top; j >= P.Mlo; j--) {
     for (uint32_t v = threadIdx.x; v < (1u << (2 * j)); v += blockDim.x) {   // (L2 reads: other blocks wrote there)
       const unsigned long long *c = H + P.fo[j + 1] + 4ull * v;
@@ -505,10 +517,7 @@ imp_pass(const ImpParams P, const ImpArgs A) {
     // ---- (B) Gradient weight (:166-178) and Loss term (:257-263) of the round's rows, one lane per row ----
     if (threadIdx.x < RR && base + threadIdx.x < last) {
       const int64_t row = base + threadIdx.x;
-      const double z = A.theta[0] + s_z[threadIdx.x], r = -log_add0(-z);
-      double w;
-      if (A.labels[row]) { w = A.inv_n * A.cw1 * (exp(r) - 1.0); A.lossterm[row] = -A.cw1 * r; }
-      else               { w = A.inv_n * A.cw0 * exp(r);         A.lossterm[row] = A.cw0 * log_add0(z); }
+      const double w = row_weight(A.theta[0] + s_z[threadIdx.x], A.labels[row], A.cw0, A.cw1, A.inv_n, A.lossterm[row]);
       const unsigned long long q = (unsigned long long)__double2ll_rn(w * A.scale);
       s_q[threadIdx.x] = q;
       if (A.scatter) { bias_acc += (long long)q; if (BIN) A.q_out[row] = q; }
@@ -780,17 +789,7 @@ __device__ __forceinline__ void hook_warp(PgState *st, double losssum, const dou
   double l1 = 0.0;
   for (int b = (int)lane_id(); b < nparts; b += 32) l1 += __ldcg(l1part + b);
   l1 = warp_sum_down(l1);
-  if (lane_id() == 0) {
-    double l = losssum * inv_n + l1;
-    st->lossval = l;
-    if (st->first) { st->first = 0; return; }   // loss at the start point: no hook call yet
-    double t = st->loss_old; st->loss_old = st->loss_new; st->loss_new = t;
-    if (eps_loss != 0.0) {
-      st->loss_new = l;
-      if (st->done == 0 && fabs(st->loss_old - st->loss_new) < eps_loss) st->done = 1;
-    }
-    if (st->done == 2) st->done = 1;
-  }
+  if (lane_id() == 0) hook_update(st, losssum * inv_n + l1, eps_loss);
 }
 
 // the loss sums of the ranks in rank order, then the hook (one warp)
@@ -805,7 +804,7 @@ __global__ void unpack_loss_hook(PgState *st, const unsigned long long *__restri
   hook_warp(st, s, l1part, nparts, inv_n, eps_loss);
 }
 
-// sum of v over the 256 threads of the block in a fixed tree (deterministic); the result is valid in thread 0
+// sum of v over the 256 threads of the block in a fixed tree (deterministic), returned to every thread
 __device__ __forceinline__ double block_sum_256(double *sh, double v) {
   sh[threadIdx.x] = v;
   __syncthreads();
@@ -833,7 +832,6 @@ __global__ void __launch_bounds__(256) pass_tail(PgState *st, const ImpParams P,
                                                  unsigned int *ticket) {
   if (st && st->done == 1) return;
   __shared__ double sh[256];
-  __shared__ int s_last;
   const int64_t stride = (int64_t)gridDim.x * blockDim.x, i0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (F)
     for (int64_t j = i0; j < m; j += stride) imp_column(P, col_id, j, F, G);
@@ -846,12 +844,7 @@ __global__ void __launch_bounds__(256) pass_tail(PgState *st, const ImpParams P,
     for (int64_t j = 1 + i0; j < ntheta; j += stride) l1 += lambda * fabs(theta[j]);
   l1 = block_sum_256(sh, l1);
   if (threadIdx.x == 0) l1part[blockIdx.x] = l1;
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) s_last = atomicAdd(ticket, 1u) == gridDim.x - 1 ? 1 : 0;
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
+  if (!last_block(ticket)) return;
   if (threadIdx.x < 32) {
     double t = 0.0;
     for (int i = threadIdx.x; i < (int)gridDim.x; i += 32) t += __ldcg(part + i);
@@ -869,15 +862,11 @@ __global__ void prox_update(PgState *st, double *__restrict__ theta, const unsig
                             double *__restrict__ blockmax, double eps, long long max_iter, unsigned int *ticket) {
   if (st->done) return;
   __shared__ double shx[256], shd[256], shn[256];
-  __shared__ int s_last;
   double mx = 0.0, md = 0.0, nn = 0.0;
   for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < ntheta; k += (int64_t)gridDim.x * blockDim.x) {
     double g = (double)(long long)G[k] * (k == 0 ? inv_scale0 : inv_scale);
     double t0 = theta[k], t1 = t0 - step * g;
-    if (k > 0) {
-      if (t1 >= 0.0) t1 = fmax(fabs(t1) - step * lambda, 0.0);
-      else           t1 = -fmax(fabs(t1) - step * lambda, 0.0);
-    }
+    if (k > 0) t1 = soft_threshold(t1, step * lambda);
     theta[k] = t1;
     if (isnan(t1)) nn = 1.0;
     mx = fmax(mx, fabs(t1));
@@ -894,12 +883,7 @@ __global__ void prox_update(PgState *st, double *__restrict__ theta, const unsig
     __syncthreads();
   }
   if (threadIdx.x == 0) { blockmax[3 * blockIdx.x] = shx[0]; blockmax[3 * blockIdx.x + 1] = shd[0]; blockmax[3 * blockIdx.x + 2] = shn[0]; }
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) s_last = atomicAdd(ticket, 1u) == gridDim.x - 1 ? 1 : 0;
-  __syncthreads();
-  if (!s_last || threadIdx.x >= 32) return;
-  __threadfence();
+  if (!last_block(ticket) || threadIdx.x >= 32) return;
   mx = 0.0; md = 0.0; nn = 0.0;
   for (int i = threadIdx.x; i < (int)gridDim.x; i += 32) {
     mx = fmax(mx, __ldcg(blockmax + 3 * i)); md = fmax(md, __ldcg(blockmax + 3 * i + 1)); nn = fmax(nn, __ldcg(blockmax + 3 * i + 2));
@@ -912,11 +896,7 @@ __global__ void prox_update(PgState *st, double *__restrict__ theta, const unsig
   }
   if (threadIdx.x == 0) {
     *ticket = 0u;
-    st->iter += 1;
-    if (nn != 0.0) { st->delta = nan(""); st->done = 1; return; }
-    st->delta = mx != 0.0 ? md / mx : md;
-    if ((mx != 0.0 && md / mx <= eps) || (mx == 0.0 && md == 0.0)) st->done = 1;
-    else if (st->iter >= max_iter) st->done = 2;
+    pg_stop(st, mx, md, nn, eps, max_iter);
   }
 }
 
@@ -960,17 +940,7 @@ __device__ __forceinline__ void small_tail(PgState *st, const double *blockloss,
   if (t == 0) {
     double ssum = sh[0][0], lsum = sh[1][0];
     for (int w = 1; w < NW; w++) { ssum += sh[0][w]; lsum += sh[1][w]; }
-    const double l = ssum * inv_n + lsum;
-    st->lossval = l;
-    if (st->first) st->first = 0;                 // loss at the start point: no hook call yet
-    else {
-      double tmp = st->loss_old; st->loss_old = st->loss_new; st->loss_new = tmp;
-      if (eps_loss != 0.0) {
-        st->loss_new = l;
-        if (st->done == 0 && fabs(st->loss_old - st->loss_new) < eps_loss) st->done = 1;
-      }
-      if (st->done == 2) st->done = 1;
-    }
+    hook_update(st, ssum * inv_n + lsum, eps_loss);
     s_done = st->done;
   }
   __syncthreads();
@@ -981,10 +951,7 @@ __device__ __forceinline__ void small_tail(PgState *st, const double *blockloss,
       for (int r = 1; r < replicas; r++) gi += __ldcg(G + r * ntheta + k);     // exact integer sum: any order
       double g = (double)(long long)gi * (k == 0 ? inv_scale0 : inv_scale);
       double t0 = theta[k], t1 = t0 - step * g;
-      if (k > 0) {
-        if (t1 >= 0.0) t1 = fmax(fabs(t1) - step * lambda, 0.0);
-        else           t1 = -fmax(fabs(t1) - step * lambda, 0.0);
-      }
+      if (k > 0) t1 = soft_threshold(t1, step * lambda);
       theta[k] = t1;
       if (isnan(t1)) nn = 1.0;
       mx = fmax(mx, fabs(t1));
@@ -1000,13 +967,7 @@ __device__ __forceinline__ void small_tail(PgState *st, const double *blockloss,
     __syncthreads();
     if (t == 0) {
       for (int w = 1; w < NW; w++) { mx = fmax(mx, sh[0][w]); md = fmax(md, sh[1][w]); nn = fmax(nn, sh[2][w]); }
-      st->iter += 1;
-      if (nn != 0.0) { st->delta = nan(""); st->done = 1; }
-      else {
-        st->delta = mx != 0.0 ? md / mx : md;
-        if ((mx != 0.0 && md / mx <= eps) || (mx == 0.0 && md == 0.0)) st->done = 1;
-        else if (st->iter >= max_iter) st->done = 2;
-      }
+      pg_stop(st, mx, md, nn, eps, max_iter);
     }
   }
   if (clear_g)
@@ -1037,12 +998,6 @@ __device__ __forceinline__ void small_rows(const Rows &R, const uint32_t *__rest
     if (LOAD_THETA) sth[i] = theta[i];
   }
   __syncthreads();
-  auto add = [&](uint32_t c, unsigned long long q) {
-    const uint32_t lo = (uint32_t)q, hi = (uint32_t)(q >> 32);
-    const uint32_t old = atomicAdd(&acc_lo[c], lo);
-    const uint32_t add_hi = hi + ((old + lo) < old ? 1u : 0u);
-    if (add_hi) atomicAdd(&acc_hi[c], add_hi);
-  };
   double lacc = 0.0;
   // every block takes an equal, contiguous share of the rows
   const int64_t row_lo = n * blockIdx.x / gridDim.x, row_hi = n * (blockIdx.x + 1) / gridDim.x;
@@ -1051,14 +1006,13 @@ __device__ __forceinline__ void small_rows(const Rows &R, const uint32_t *__rest
     R.range(row, a, b);
     double s = 0.0;
     for (int64_t p = a; p < b; p++) s += valf(val, p) * sth[col[p] + 1];
-    // Gradient weight (:166-178) and Loss term (:257-263)
-    double z = sth[0] + s, r = -log_add0(-z), w;
-    if (labels[row]) { w = inv_n * cw1 * (exp(r) - 1.0); lacc += -cw1 * r; }
-    else             { w = inv_n * cw0 * exp(r);         lacc += cw0 * log_add0(z); }
+    double lt;
+    const double w = row_weight(sth[0] + s, labels[row], cw0, cw1, inv_n, lt);
+    lacc += lt;
     if (!scatter) continue;
     const double ws = w * scale;                    // scale is a power of two: exact
-    add(0u, (unsigned long long)__double2ll_rn(w * scale0));
-    for (int64_t p = a; p < b; p++) add(col[p] + 1u, (unsigned long long)__double2ll_rn(ws * valf(val, p)));
+    acc64_add(acc_lo, acc_hi, 0u, (unsigned long long)__double2ll_rn(w * scale0));
+    for (int64_t p = a; p < b; p++) acc64_add(acc_lo, acc_hi, col[p] + 1u, (unsigned long long)__double2ll_rn(ws * valf(val, p)));
   }
   // loss partial of the block: shuffle tree inside the warps, then the warp sums in warp order (fixed)
 #pragma unroll
@@ -1070,11 +1024,7 @@ __device__ __forceinline__ void small_rows(const Rows &R, const uint32_t *__rest
     for (int w = 1; w < (int)(blockDim.x >> 5); w++) l += red[w];
     blockloss[blockIdx.x] = l;
   }
-  if (scatter)
-    for (int i = threadIdx.x; i < ntheta; i += blockDim.x) {
-      unsigned long long v = ((unsigned long long)acc_hi[i] << 32) | acc_lo[i];
-      if (v) atomicAdd(&G[i], v);
-    }
+  if (scatter) acc64_flush(acc_lo, acc_hi, ntheta, G);
 }
 
 #ifndef KL_LONG_U
@@ -1103,13 +1053,6 @@ struct LongView {
   // the gradient of the block's rows is summed by the block itself -- one grid barrier per iteration instead of two
   const int64_t *bv_off; const uint32_t *bv_pack; int bv_row_bits;
 };
-
-__device__ __forceinline__ void small_acc_add(uint32_t *acc_lo, uint32_t *acc_hi, uint32_t c, unsigned long long q) {
-  const uint32_t lo = (uint32_t)q, hi = (uint32_t)(q >> 32);
-  const uint32_t old = atomicAdd(&acc_lo[c], lo);
-  const uint32_t add_hi = hi + ((old + lo) < old ? 1u : 0u);
-  if (add_hi) atomicAdd(&acc_hi[c], add_hi);
-}
 
 template <typename VT>
 __device__ __forceinline__ void long_forward(const Rows &R, const LongView<VT> &V, int64_t n, int64_t ntheta,
@@ -1142,9 +1085,9 @@ __device__ __forceinline__ void long_forward(const Rows &R, const LongView<VT> &
     } else {
       for (int k = 0; k < len; k++) s += valf(V.sval, base + 32 * k) * sth[V.scol[base + 32 * k] + 1];
     }
-    double z = sth[0] + s, r = -log_add0(-z), w;
-    if (labels[row]) { w = inv_n * cw1 * (exp(r) - 1.0); lacc += -cw1 * r; }
-    else             { w = inv_n * cw0 * exp(r);         lacc += cw0 * log_add0(z); }
+    double lt;
+    const double w = row_weight(sth[0] + s, labels[row], cw0, cw1, inv_n, lt);
+    lacc += lt;
     if (!scatter) continue;
     const double ws = w * scale;
     if (w_local) w_local[row - row_lo] = ws; else V.wbuf[row] = ws;
@@ -1154,7 +1097,7 @@ __device__ __forceinline__ void long_forward(const Rows &R, const LongView<VT> &
   for (int o = 16; o > 0; o >>= 1) { lacc += __shfl_down_sync(0xffffffffu, lacc, o); bias += __shfl_down_sync(0xffffffffu, bias, o); }
   if ((threadIdx.x & 31) == 0) {
     red[threadIdx.x >> 5] = lacc;
-    if (bias) small_acc_add(acc_lo, acc_hi, 0u, (unsigned long long)bias);
+    if (bias) acc64_add(acc_lo, acc_hi, 0u, (unsigned long long)bias);
   }
   __syncthreads();
   if (threadIdx.x == 0) {
@@ -1177,7 +1120,7 @@ __device__ __forceinline__ void long_columns(const LongView<VT> &V, int64_t nthe
     long long cend = scp[c + 1];
     auto boundary = [&](int64_t q) {
       if (q >= cend) {
-        if (acc) small_acc_add(acc_lo, acc_hi, (uint32_t)c + 1u, (unsigned long long)acc);
+        if (acc) acc64_add(acc_lo, acc_hi, (uint32_t)c + 1u, (unsigned long long)acc);
         acc = 0;
         do { c++; cend = scp[c + 1]; } while (q >= cend);
       }
@@ -1213,15 +1156,12 @@ __device__ __forceinline__ void long_columns(const LongView<VT> &V, int64_t nthe
   if (__all_sync(0xffffffffu, c == c0)) {
 #pragma unroll
     for (int o = 16; o > 0; o >>= 1) acc += __shfl_down_sync(0xffffffffu, acc, o);
-    if ((threadIdx.x & 31) == 0 && c >= 0 && acc) small_acc_add(acc_lo, acc_hi, (uint32_t)c + 1u, (unsigned long long)acc);
+    if ((threadIdx.x & 31) == 0 && c >= 0 && acc) acc64_add(acc_lo, acc_hi, (uint32_t)c + 1u, (unsigned long long)acc);
   } else if (c >= 0 && acc) {
-    small_acc_add(acc_lo, acc_hi, (uint32_t)c + 1u, (unsigned long long)acc);
+    acc64_add(acc_lo, acc_hi, (uint32_t)c + 1u, (unsigned long long)acc);
   }
   __syncthreads();
-  for (int i = threadIdx.x; i < ntheta; i += blockDim.x) {
-    unsigned long long v = ((unsigned long long)acc_hi[i] << 32) | acc_lo[i];
-    if (v) atomicAdd(&G[i], v);
-  }
+  acc64_flush(acc_lo, acc_hi, ntheta, G);
 }
 
 // LONG == 2: gradient of the block's OWN rows from the block-local view (thread t sums its contiguous share of the
@@ -1245,18 +1185,15 @@ __device__ __forceinline__ void block_columns(const LongView<VT> &V, int64_t nth
       if (e[i] == 0xFFFFFFFFu) continue;
       const int c = (int)((e[i] >> cs) & 1023u);
       if (c != cur) {
-        if (acc) small_acc_add(acc_lo, acc_hi, (uint32_t)cur + 1u, (unsigned long long)acc);
+        if (acc) acc64_add(acc_lo, acc_hi, (uint32_t)cur + 1u, (unsigned long long)acc);
         acc = 0; cur = c;
       }
       acc += __double2ll_rn(w_s[e[i] & rmask] * (double)(e[i] >> vs));
     }
   }
-  if (acc) small_acc_add(acc_lo, acc_hi, (uint32_t)cur + 1u, (unsigned long long)acc);
+  if (acc) acc64_add(acc_lo, acc_hi, (uint32_t)cur + 1u, (unsigned long long)acc);
   __syncthreads();
-  for (int i = threadIdx.x; i < ntheta; i += blockDim.x) {
-    unsigned long long v = ((unsigned long long)acc_hi[i] << 32) | acc_lo[i];
-    if (v) atomicAdd(&G[i], v);
-  }
+  acc64_flush(acc_lo, acc_hi, ntheta, G);
 }
 
 template <typename VT>
@@ -1270,19 +1207,13 @@ __global__ void __launch_bounds__(256, SMALL_BLOCKS_PER_SM) fused_small_kernel(c
                                                           long long max_iter) {
   if (st->done == 1) return;
   __shared__ uint32_t acc_lo[SMALL_MAX_THETA], acc_hi[SMALL_MAX_THETA];
-  __shared__ int s_last;
   __shared__ double sth[SMALL_MAX_THETA];
   __shared__ double red[256];
   small_rows<VT>(R, col, val, n, ntheta, theta, labels, cw0, cw1, inv_n, scale, scale0, G, blockloss, scatter, acc_lo, acc_hi,
                  sth, red);
   // the block that finishes last runs the tail of the iteration (its reads see every block's results)
   if (!counter) return;                 // sharded: the collectives come first, the tail is its own launch
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) s_last = atomicAdd(counter, 1u) == gridDim.x - 1 ? 1 : 0;
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
+  if (!last_block(counter)) return;
   small_tail(st, blockloss, (int)gridDim.x, theta, G, inv_scale, inv_scale0, ntheta, inv_n, lambda, eps_loss, step, eps,
              max_iter);
   if (threadIdx.x == 0) *counter = 0u;
@@ -1373,23 +1304,18 @@ __global__ void __launch_bounds__(PERSIST_THREADS, SMALL_BLOCKS_PER_SM) fused_sm
         PeerMail *mine = pb->box[me];
         const unsigned long long seq = s_seq + 1ull;
         const int par = (int)(seq & 1ull);
+        if (t == 0) s_timeout = 0;
         // loss partial of this rank: block partials in a fixed order
         double s = 0.0;
         for (int i = t; i < nblocks; i += PERSIST_THREADS) s += __ldcg(blockloss + i);
-        red[t] = s;
-        if (t == 0) s_timeout = 0;
-        __syncthreads();
-        for (int o = PERSIST_THREADS / 2; o > 0; o >>= 1) {
-          if (t < o) red[t] += red[t + o];
-          __syncthreads();
-        }
+        s = block_sum_256(red, s);
         // payload into every mailbox (NVLink stores), one system fence, then the flags
         for (int64_t k = t; k < ntheta; k += PERSIST_THREADS) {
           unsigned long long g = 0ull;
           for (int r = 0; r < SMALL_REPLICAS; r++) g += __ldcg(G + r * ntheta + k);
           for (int r = 0; r < world; r++) pb->box[r]->slot[par][me][k] = g;
         }
-        if (t < world) pb->box[t]->slot[par][me][ntheta] = (unsigned long long)__double_as_longlong(red[0]);
+        if (t < world) pb->box[t]->slot[par][me][ntheta] = (unsigned long long)__double_as_longlong(s);
         __syncthreads();
         if (t == 0) __threadfence_system();
         __syncthreads();
@@ -1443,13 +1369,8 @@ __global__ void __launch_bounds__(256) small_presum_kernel(const PgState *st, co
   __shared__ double sh[256];
   double s = 0.0;
   for (int i = threadIdx.x; i < nblocks; i += 256) s += blockloss[i];
-  sh[threadIdx.x] = s;
-  __syncthreads();
-  for (int o = 128; o > 0; o >>= 1) {
-    if ((int)threadIdx.x < o) sh[threadIdx.x] += sh[threadIdx.x + o];
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) out[0] = sh[0];
+  s = block_sum_256(sh, s);
+  if (threadIdx.x == 0) out[0] = s;
 }
 // ... and the tail over the gathered per-rank losses (rank order) and the all-reduced gradient
 __global__ void __launch_bounds__(256) small_tail_kernel(PgState *st, const double *partials, int nparts, double *theta,
@@ -1487,15 +1408,10 @@ __global__ void __launch_bounds__(256) small_p2p_tail_kernel(PgState *st, const 
     const int dst_rank = (int)blockIdx.x;
     double s = 0.0;
     for (int i = t; i < nblocks; i += 256) s += blockloss[i];      // loss partial of this rank, fixed order
-    shs[t] = s;
-    __syncthreads();
-    for (int o = 128; o > 0; o >>= 1) {
-      if (t < o) shs[t] += shs[t + o];
-      __syncthreads();
-    }
+    s = block_sum_256(shs, s);
     unsigned long long *dst = pb->box[dst_rank]->slot[par][me];
     for (int64_t k = t; k < ntheta; k += 256) dst[k] = G[k];
-    if (t == 0) dst[ntheta] = (unsigned long long)__double_as_longlong(shs[0]);
+    if (t == 0) dst[ntheta] = (unsigned long long)__double_as_longlong(s);
     __threadfence_system();
     __syncthreads();
     if (t == 0) {
@@ -1576,17 +1492,6 @@ template <> const double *csc_val<double>(const Matrix &M) { return M.cval_f64.p
 
 inline unsigned warp_grid(int64_t items, int threads) { return (unsigned)((items * 32 + threads - 1) / threads); }
 
-// deterministic sum of a device vector into out[0] (all ranks when sharded)
-void reduce_sum(const Matrix &M, const double *x, int64_t n, Work &wk, double *out, const PgState *st,
-                bool all_ranks = true) {
-  KL_LAUNCH(reduce_stage1, RED_BLOCKS, 256, 0, x, n, wk.red.p, st);
-  KL_LAUNCH(reduce_stage2, 1, 32, 0, wk.red.p, RED_BLOCKS, out, st);
-  if (M.sharded && all_ranks) {
-    comm_allgather_f64(out, wk.gathered.p, 1);
-    KL_LAUNCH(sum_ranks, 1, 32, 0, wk.gathered.p, ctx().world, (int64_t)1, out);
-  }
-}
-
 // the non-zero pair coefficients of a host theta, in coefficient order; empty optional = too many (dense theta)
 constexpr int64_t PAIR_TERMS_MAX = 8192;
 struct PairTerms {
@@ -1628,14 +1533,9 @@ void launch_rows(const Matrix &M, const double *theta, int cooc, const double cw
 // 2^60.  The columns of a matrix whose values are all below 1 get the finer scale their bound allows (a matrix of
 // frequencies would otherwise lose the bits between max|v| and 1); the bias keeps max(cw) * max(max|v|, 1).  Both
 // are the same whenever max|v| >= 1, as in every count and binarized matrix.
-static int scale_exponent(double bound) {
-  if (!(bound > 0.0) || !std::isfinite(bound)) bound = 1.0;
-  const int e = 60 - (int)std::ceil(std::log2(bound));
-  return e > 1000 ? 1000 : e;
-}
 void set_scale(Matrix &M, Work &wk, const double cw[2]) {
   const double cmax = std::fmax(std::fabs(cw[0]), std::fabs(cw[1])), vmax = matrix_vmax(M);
-  const int e = scale_exponent(cmax * (vmax > 0.0 ? vmax : 1.0)), e0 = scale_exponent(cmax * std::fmax(vmax, 1.0));
+  const int e = fixed_point_exponent(cmax * (vmax > 0.0 ? vmax : 1.0)), e0 = fixed_point_exponent(cmax * std::fmax(vmax, 1.0));
   wk.scale = std::ldexp(1.0, e);
   wk.inv_scale = std::ldexp(1.0, -e);
   wk.scale0 = std::ldexp(1.0, e0);
@@ -1793,12 +1693,13 @@ void alloc_work(const Matrix &M, int64_t ntheta, Work &wk) {
   wk.tickets.zero();
 }
 
-// the tail of a pass (pass_tail): the pending matrix-free columns, the loss and L1 partials and, with a state and
-// hook = 1, the loss sum and the hook
-void launch_pass_tail(const Matrix &M, Work &wk, PgState *st, int64_t ntheta, double lambda, int hook, double eps_loss) {
+// the tail of a pass (pass_tail): the pending matrix-free columns, the sum of the first n loss terms into
+// wk.scalars[0], the L1 partials of theta[1, ntheta) and, with a state and hook = 1, the hook
+void launch_pass_tail(const Matrix &M, Work &wk, PgState *st, int64_t n, int64_t ntheta, double lambda, int hook,
+                      double eps_loss) {
   static_assert(RED_BLOCKS == PROX_BLOCKS, "the L1 partials of pass_tail are the hook's PROX_BLOCKS partials");
-  KL_LAUNCH(pass_tail, RED_BLOCKS, 256, 0, st, wk.P, M.class_ids.p, M.m, wk.F, wk.G.p, wk.lossterm.p, st ? M.n : 0,
-            wk.red.p, wk.scalars.p, wk.theta.p, st ? ntheta : 0, lambda, wk.blockmax.p + 3 * PROX_BLOCKS, hook,
+  KL_LAUNCH(pass_tail, RED_BLOCKS, 256, 0, st, wk.P, M.class_ids.p, M.m, wk.F, wk.G.p, wk.lossterm.p, n,
+            wk.red.p, wk.scalars.p, wk.theta.p, ntheta, lambda, wk.blockmax.p + 3 * PROX_BLOCKS, hook,
             1.0 / (double)M.n_global, eps_loss, wk.tickets.p + 1);
   wk.F = nullptr;
 }
@@ -1846,7 +1747,7 @@ void gradient(Matrix &M, const double *theta, int64_t ntheta, const double cw[2]
     using VT = typename std::remove_pointer<decltype(tag)>::type;
     if (!cooc) {
       launch_fused<VT>(M, wk, cw, nullptr);
-      if (wk.F) launch_pass_tail(M, wk, nullptr, ntheta, NAN, 0, 0.0);
+      if (wk.F) launch_pass_tail(M, wk, nullptr, 0, 0, NAN, 0, 0.0);
       if (M.sharded) comm_allreduce_sum_i64_fast((int64_t *)wk.G.p, M.m + 1);
     } else {
       // pair mode: z needs the pair terms, so the weights come from the general rows kernel; the
@@ -1898,7 +1799,12 @@ double loss(Matrix &M, const double *theta, int64_t ntheta, const double cw[2], 
     using VT = typename std::remove_pointer<decltype(tag)>::type;
     launch_rows<VT, 2>(M, wk.theta.p, cooc, cw, wk.w.p, wk.lossterm.p, nullptr, &terms);
   });
-  reduce_sum(M, wk.lossterm.p, M.n, wk, wk.scalars.p, nullptr);
+  launch_pass_tail(M, wk, nullptr, M.n, 0, NAN, 0, 0.0);
+  if (M.sharded) {
+    // the sums of the ranks in rank order (the same bits on every rank)
+    comm_allgather_f64(wk.scalars.p, wk.gathered.p, 1);
+    KL_LAUNCH(sum_ranks, 1, 32, 0, wk.gathered.p, ctx().world, (int64_t)1, wk.scalars.p);
+  }
   double s = 0.0;
   wk.scalars.download(&s, 1);
   sync_stream();
@@ -2096,7 +2002,7 @@ void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], doub
         using VT = typename std::remove_pointer<decltype(tag)>::type;
         launch_fused<VT>(M, wk, cw, st.p, scatter);
         // columns, loss and L1 partials; one GPU: the loss sum and the hook in the same launch
-        launch_pass_tail(M, wk, st.p, M.m + 1, lambda, M.sharded ? 0 : 1, epsilon_loss);
+        launch_pass_tail(M, wk, st.p, M.n, M.m + 1, lambda, M.sharded ? 0 : 1, epsilon_loss);
         if (M.sharded) {
           // ONE collective per iteration: gradient words + the loss sums of the ranks
           unsigned long long *slots = wk.G.p + M.m + 1;
