@@ -200,6 +200,24 @@ int kmerlr_proxgrad(kmerlr_handle h, double *theta_inout, int64_t ntheta, const 
                     double lambda, double l2, double step_factor, double epsilon, double epsilon_loss,
                     int64_t max_iter, double hook_state[2], int64_t *iters_out, double *delta_out);
 
+/* Accelerated proximal gradient (FISTA with gradient restart, O'Donoghue & Candes), opt-in; reduced matrices on one GPU
+ * only.  Same inputs as kmerlr_proxgrad, plus the extrapolated point y (ntheta doubles) and the momentum t, carried in
+ * and out so that a later call resumes exactly; a fresh start is y = theta, t = 1.  The step s is kmerlr_step_size's.
+ * One iteration:
+ *   g = gradient at y;  theta' = y - s g, soft-thresholded at s lambda for j >= 1 (the bias is not penalised);
+ *   eval_stopping(theta, theta', epsilon) stops with theta = theta' (y and t stay);
+ *   restart when (y - theta').(theta' - theta) > 0: t' = 1, y' = theta';
+ *   else t' = (1 + sqrt(1 + 4 t^2)) / 2, y' = theta' + ((t - 1) / t') (theta' - theta);
+ *   the hook's delta-loss test runs on F(y') = f(y') + lambda |y'_{1:}|_1, the objective the next pass evaluates anyway.
+ * So hook_state holds F(y) values, and after max_iter steps the loss-only pass evaluates F(y).  theta_inout returns the
+ * prox output (sparse), y_inout and t_inout the momentum state; delta_out as kmerlr_proxgrad; restarts_out = the
+ * restarts of this call.  KMERLR_ERR_ARG: a sharded matrix; a matrix the reduced-matrix path does not take (more than
+ * 1023 columns, or a matrix-free view straight from kmerlr_extract); t < 1 or not finite; a null theta, y, t or class_w. */
+int kmerlr_proxgrad_accel(kmerlr_handle h, double *theta_inout, double *y_inout, double *t_inout, int64_t ntheta,
+                          const double class_w[2], double lambda, double l2, double step_factor, double epsilon,
+                          double epsilon_loss, int64_t max_iter, double hook_state[2], int64_t *iters_out,
+                          double *delta_out, int64_t *restarts_out);
+
 /* ---- IRLS + coordinate-descent estimator (kmerLr_estimator_coordinate.go:31-139), reduced matrices only
  * (ntheta <= 1024: it keeps the dense Gram matrix, as the reference does), one GPU.  The reference never
  * calls it and its theta slices alias (:89-91); built with the slices de-aliased, like kmerlr_proxgrad.

@@ -639,7 +639,7 @@ class KmerLrEstimator:
     L1Reg, the hook's loss_old / loss_new."""
 
     def __init__(self, Cooccurrence=False, Epsilon=0.0, EpsilonLoss=1e-8, EpsilonLambda=0.0, L2Reg=0.0,
-                 StepSizeFactor=1.0, MaxIterations=100000, MaxEpochs=0, tie=TIE_GO118):
+                 StepSizeFactor=1.0, MaxIterations=100000, MaxEpochs=0, tie=TIE_GO118, Accelerated=False):
         self.Cooccurrence, self.Epsilon, self.EpsilonLoss = Cooccurrence, Epsilon, EpsilonLoss
         self.EpsilonLambda, self.L2Reg, self.StepSizeFactor = EpsilonLambda, L2Reg, StepSizeFactor
         self.MaxIterations, self.MaxEpochs, self.tie = MaxIterations, MaxEpochs, tie
@@ -650,15 +650,34 @@ class KmerLrEstimator:
         self.hook_state = np.array([np.nan, np.nan])
         self.path = []
         self.Transform = None            # the selected transform of the last estimate (r.Transform of the reference's KmerLr)
+        # Accelerated: estimate_proximal runs FISTA with gradient restart (kmerlr_proxgrad_accel; reduced matrices, one
+        # GPU).  accel_state = (handle of the data, y, t, restarts of the last call): the momentum carried between calls
+        # on the same reduced data, so that a run cut into slices of MaxIterations resumes exactly.
+        self.Accelerated = Accelerated
+        self.accel_state = None
 
     def estimate_proximal(self, data_train, lam):
         """estimate_proximal (kmerLr_estimator_proximal.go:78-120) on the (reduced) data set."""
         theta = np.ascontiguousarray(self.Theta, dtype=np.float64).copy()
         iters, delta = C.c_int64(), C.c_double()
+        if self.Accelerated:
+            return self._estimate_accelerated(data_train, lam, theta, iters, delta)
         check(lib().kmerlr_proxgrad(data_train.h, _p(theta), len(theta), _p(self.ClassWeights), float(lam),
                                     self.L2Reg, self.StepSizeFactor, self.Epsilon, self.EpsilonLoss,
                                     self.MaxIterations, _p(self.hook_state), iters, delta))
         self.Theta = theta
+        return iters.value, delta.value
+
+    def _estimate_accelerated(self, data_train, lam, theta, iters, delta):
+        st = self.accel_state
+        if st is None or st[0] != data_train.h or len(st[1]) != len(theta):
+            st = (data_train.h, theta.copy(), 1.0, 0)         # fresh start: y = theta, t = 1
+        y, t, restarts = st[1].copy(), C.c_double(st[2]), C.c_int64()
+        check(lib().kmerlr_proxgrad_accel(data_train.h, _p(theta), _p(y), t, len(theta), _p(self.ClassWeights),
+                                          float(lam), self.L2Reg, self.StepSizeFactor, self.Epsilon, self.EpsilonLoss,
+                                          self.MaxIterations, _p(self.hook_state), iters, delta, restarts))
+        self.Theta = theta
+        self.accel_state = (data_train.h, y, t.value, restarts.value)
         return iters.value, delta.value
 
     def estimate_coordinate(self, data_train):
@@ -698,6 +717,7 @@ class KmerLrEstimator:
                 tdata = self.Transform.Apply(reduced)
                 reduced.free()
                 reduced = tdata
+            self.accel_state = None          # the momentum restarts at every epoch: y = theta of the new reduced matrix, t = 1
             iters, _ = self.estimate_proximal(reduced, lam)
             reduced_nnz = reduced.nnz
             reduced.free()

@@ -31,6 +31,12 @@ struct PgState {
   double delta, loss_old, loss_new, lossval;
   int error;         // 1: a peer never answered the gradient exchange
 };
+// the accelerated solver's state: PgState + the momentum scalar t and the restarts of this call.  A separate type,
+// so that the ISTA kernels keep their shared-memory copy of PgState at its size.
+struct PgStateAccel : PgState {
+  double t;
+  long long restarts;
+};
 
 // the hook's state transition (kmerLr_estimator_hook.go:46-99) for the loss l at the current theta
 __device__ __forceinline__ void hook_update(PgState *st, double l, double eps_loss) {
@@ -908,16 +914,86 @@ __global__ void prox_update(PgState *st, double *__restrict__ theta, const unsig
 // cooperative launch.
 constexpr int SMALL_MAX_THETA = 1024;
 
+// the accelerated step of small_tail: thread t owns coefficients t, t + BT, ... (at most SMALL_MAX_THETA / BT), keeps
+// theta'_k and theta'_k - theta_k in registers across the block-wide decision and then writes theta and y
+template <int BT>
+__device__ __forceinline__ void accel_step(PgStateAccel *st, double *y, double *xth, const unsigned long long *G,
+                                           double inv_scale, double inv_scale0, int64_t ntheta, double lambda, double step,
+                                           double eps, long long max_iter, int replicas, double (*sh)[BT / 32]) {
+  constexpr int NW = BT / 32, PER = SMALL_MAX_THETA / BT;
+  __shared__ double s_beta;
+  __shared__ int s_mode;       // 0: stopped (theta = theta', y and t stay), 1: restart, 2: momentum
+  const int t = threadIdx.x, lane = t & 31, wid = t >> 5;
+  double tn[PER], dl[PER];
+  double mx = 0.0, md = 0.0, nn = 0.0, dot = 0.0;
+#pragma unroll
+  for (int j = 0; j < PER; j++) {
+    const int64_t k = t + (int64_t)j * BT;
+    tn[j] = 0.0; dl[j] = 0.0;
+    if (k < ntheta) {
+      unsigned long long gi = __ldcg(G + k);
+      for (int r = 1; r < replicas; r++) gi += __ldcg(G + r * ntheta + k);
+      const double g = (double)(long long)gi * (k == 0 ? inv_scale0 : inv_scale);
+      const double yk = y[k], x0 = xth[k];
+      double t1 = yk - step * g;
+      if (k > 0) t1 = soft_threshold(t1, step * lambda);
+      tn[j] = t1; dl[j] = t1 - x0;
+      if (isnan(t1)) nn = 1.0;
+      mx = fmax(mx, fabs(t1));
+      md = fmax(md, fabs(dl[j]));
+      dot += (yk - t1) * dl[j];
+    }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    mx = fmax(mx, __shfl_down_sync(0xffffffffu, mx, o));
+    md = fmax(md, __shfl_down_sync(0xffffffffu, md, o));
+    nn = fmax(nn, __shfl_down_sync(0xffffffffu, nn, o));
+    dot += __shfl_down_sync(0xffffffffu, dot, o);
+  }
+  if (lane == 0) { sh[0][wid] = mx; sh[1][wid] = md; sh[2][wid] = nn; sh[3][wid] = dot; }
+  __syncthreads();
+  if (t == 0) {
+    for (int w = 1; w < NW; w++) { mx = fmax(mx, sh[0][w]); md = fmax(md, sh[1][w]); nn = fmax(nn, sh[2][w]); dot += sh[3][w]; }
+    pg_stop(st, mx, md, nn, eps, max_iter);
+    if (st->done == 1) {
+      s_mode = 0;
+    } else if (dot > 0.0) {
+      s_mode = 1; st->t = 1.0; st->restarts += 1;
+    } else {
+      const double t0 = st->t, t1 = (1.0 + sqrt(1.0 + 4.0 * (t0 * t0))) / 2.0;
+      s_mode = 2; s_beta = (t0 - 1.0) / t1; st->t = t1;
+    }
+  }
+  __syncthreads();
+  const int mode = s_mode;
+  const double beta = s_beta;
+#pragma unroll
+  for (int j = 0; j < PER; j++) {
+    const int64_t k = t + (int64_t)j * BT;
+    if (k < ntheta) {
+      xth[k] = tn[j];
+      if (mode == 1) y[k] = tn[j];
+      else if (mode == 2) y[k] = tn[j] + beta * dl[j];
+    }
+  }
+}
+
 // hook (kmerLr_estimator_hook.go:46-99) + prox step + eval_stopping (kmerLr_estimator_proximal.go:30-52,88-98),
-// run by ONE block of 256 threads once every block's partials are in
-template <int BT = 256>
+// run by ONE block of 256 threads once every block's partials are in.  `theta` is the point the row pass evaluated.
+// ACCEL (FISTA with gradient restart): `theta` is the extrapolated point y, `xth` the iterate theta, st a PgStateAccel.
+// theta' = prox(y - s g); eval_stopping on (theta, theta'); unless it stops, restart (t' = 1, y' = theta') when
+// (y - theta').(theta' - theta) > 0, else t' = (1 + sqrt(1 + 4 t^2)) / 2, y' = theta' + ((t - 1) / t') (theta' - theta).
+// The dot product is summed in a fixed order (per thread by index, a shuffle tree, the warps in order), so every block
+// of the persistent kernel takes the same decision.
+template <int BT = 256, bool ACCEL = false>
 __device__ __forceinline__ void small_tail(PgState *st, const double *blockloss, int nblocks, double *theta,
                                            unsigned long long *G,
                                            double inv_scale, double inv_scale0, int64_t ntheta, double inv_n, double lambda,
                                            double eps_loss, double step, double eps, long long max_iter,
-                                           bool clear_g = true, int replicas = 1) {
+                                           bool clear_g = true, int replicas = 1, double *xth = nullptr) {
   constexpr int NW = BT / 32;
-  __shared__ double sh[3][NW];
+  __shared__ double sh[ACCEL ? 4 : 3][NW];
   __shared__ int s_done;
   const int t = threadIdx.x, lane = t & 31, wid = t >> 5;
   // loss = sum of the block partials (index order inside a thread, fixed tree across threads) + L1 term;
@@ -944,7 +1020,10 @@ __device__ __forceinline__ void small_tail(PgState *st, const double *blockloss,
     s_done = st->done;
   }
   __syncthreads();
-  if (!s_done) {
+  if constexpr (ACCEL) {
+    if (!s_done) accel_step<BT>(static_cast<PgStateAccel *>(st), theta, xth, G, inv_scale, inv_scale0, ntheta, lambda,
+                                step, eps, max_iter, replicas, sh);
+  } else if (!s_done) {
     double mx = 0.0, md = 0.0, nn = 0.0;
     for (int64_t k = t; k < ntheta; k += BT) {
       unsigned long long gi = __ldcg(G + k);
@@ -1196,7 +1275,8 @@ __device__ __forceinline__ void block_columns(const LongView<VT> &V, int64_t nth
   acc64_flush(acc_lo, acc_hi, ntheta, G);
 }
 
-template <typename VT>
+// ACCEL: theta holds y (what the row pass reads), theta + ntheta the iterate theta, st is a PgStateAccel
+template <typename VT, bool ACCEL = false>
 __global__ void __launch_bounds__(256, SMALL_BLOCKS_PER_SM) fused_small_kernel(const Rows R, const uint32_t *__restrict__ col,
                                                           const VT *__restrict__ val, int64_t n, int64_t ntheta,
                                                           double *theta, const uint8_t *__restrict__ labels,
@@ -1214,8 +1294,8 @@ __global__ void __launch_bounds__(256, SMALL_BLOCKS_PER_SM) fused_small_kernel(c
   // the block that finishes last runs the tail of the iteration (its reads see every block's results)
   if (!counter) return;                 // sharded: the collectives come first, the tail is its own launch
   if (!last_block(counter)) return;
-  small_tail(st, blockloss, (int)gridDim.x, theta, G, inv_scale, inv_scale0, ntheta, inv_n, lambda, eps_loss, step, eps,
-             max_iter);
+  small_tail<256, ACCEL>(st, blockloss, (int)gridDim.x, theta, G, inv_scale, inv_scale0, ntheta, inv_n, lambda, eps_loss,
+                         step, eps, max_iter, true, 1, theta + ntheta);
   if (threadIdx.x == 0) *counter = 0u;
 }
 
@@ -1229,13 +1309,16 @@ __global__ void __launch_bounds__(256, SMALL_BLOCKS_PER_SM) fused_small_kernel(c
 // pass - 1.  The loss partials of pass + 2 overwrite those of `pass` for the same reason.  The passes of
 // one launch are pass0, pass0 + 1, ...; pass number max_iter only evaluates the hook's loss.
 // (1024-thread blocks, one per SM -- fewer loss partials, a cheaper barrier -- measured no faster: 23 vs 21 us)
+// ACCEL (one GPU only): sth holds the extrapolated point y, which the row pass reads; the iterate theta lives in a
+// second shared array sx; theta[0, ntheta) is y and theta[ntheta, 2 ntheta) the iterate in global memory, and st is a
+// PgStateAccel (the momentum t and the restarts travel with the state).
 constexpr int PERSIST_THREADS = 256;
 // SHARDED: the rows are this rank's shard and the ranks are connected by NVLink peer memory.  After the grid
 // barrier block 0 exchanges the rank's payload (fixed-point gradient + loss partial) with all ranks through
 // the mailboxes -- stores into every rank's slot, a flag, a wait for the flags of the others, the sum in rank
 // order (integers: the same bits on every rank) -- and a second grid barrier releases the tail.  The
 // collective lives INSIDE the persistent kernel: no launch and no NCCL call per iteration.
-template <typename VT, bool SHARDED, int LONG>
+template <typename VT, bool SHARDED, int LONG, bool ACCEL = false>
 __global__ void __launch_bounds__(PERSIST_THREADS, SMALL_BLOCKS_PER_SM) fused_small_persistent(
     const Rows R, const uint32_t *__restrict__ col, const VT *__restrict__ val, int64_t n, int64_t ntheta, double *theta,
     const uint8_t *__restrict__ labels, double cw0, double cw1, double inv_n, double scale, double scale0,
@@ -1247,14 +1330,19 @@ __global__ void __launch_bounds__(PERSIST_THREADS, SMALL_BLOCKS_PER_SM) fused_sm
   __shared__ uint32_t acc_lo[SMALL_MAX_THETA], acc_hi[SMALL_MAX_THETA];
   __shared__ double sth[SMALL_MAX_THETA];
   __shared__ double red[256];
-  __shared__ PgState ls;
+  using State = typename std::conditional<ACCEL, PgStateAccel, PgState>::type;
+  __shared__ State ls;
+  __shared__ double sx[ACCEL ? SMALL_MAX_THETA : 1];
   __shared__ unsigned long long s_seq;
   __shared__ int s_timeout;
   if (threadIdx.x == 0) {
-    ls = *st;
+    ls = *static_cast<State *>(st);
     if (SHARDED) s_seq = pb->box[pb->rank]->seq;
   }
-  for (int i = threadIdx.x; i < ntheta; i += blockDim.x) sth[i] = theta[i];
+  for (int i = threadIdx.x; i < ntheta; i += blockDim.x) {
+    sth[i] = theta[i];
+    if constexpr (ACCEL) sx[i] = theta[ntheta + i];
+  }
   // LONG: the column offsets stay in shared memory; c_first = the column of this thread's first column-major entry
   __shared__ long long scp[LONG == 1 ? SMALL_MAX_THETA + 1 : 1];
   extern __shared__ __align__(16) double w_s[];          // LONG == 2: the scaled weights of the block's rows
@@ -1296,8 +1384,8 @@ __global__ void __launch_bounds__(PERSIST_THREADS, SMALL_BLOCKS_PER_SM) fused_sm
     }
     grid.sync();
     if (!SHARDED) {
-      small_tail<PERSIST_THREADS>(&ls, blockloss, nblocks, sth, G, inv_scale, inv_scale0, ntheta, inv_n, lambda, eps_loss,
-                                  step, eps, max_iter, false, SMALL_REPLICAS);
+      small_tail<PERSIST_THREADS, ACCEL>(&ls, blockloss, nblocks, sth, G, inv_scale, inv_scale0, ntheta, inv_n, lambda,
+                                         eps_loss, step, eps, max_iter, false, SMALL_REPLICAS, sx);
     } else {
       if (blockIdx.x == 0) {
         const int t = threadIdx.x, me = pb->rank, world = pb->world;
@@ -1354,9 +1442,12 @@ __global__ void __launch_bounds__(PERSIST_THREADS, SMALL_BLOCKS_PER_SM) fused_sm
     __syncthreads();
   }
   if (blockIdx.x == 0) {
-    for (int i = threadIdx.x; i < ntheta; i += blockDim.x) theta[i] = sth[i];
+    for (int i = threadIdx.x; i < ntheta; i += blockDim.x) {
+      theta[i] = sth[i];
+      if constexpr (ACCEL) theta[ntheta + i] = sx[i];
+    }
     if (threadIdx.x == 0) {
-      *st = ls;
+      *static_cast<State *>(st) = ls;
       if (SHARDED) pb->box[pb->rank]->seq = s_seq;
     }
   }
@@ -1479,7 +1570,10 @@ const VT *sliced_val(const Matrix &M);
 template <> const uint32_t *sliced_val<uint32_t>(const Matrix &M) { return M.vt == VAL_U32 ? M.sval_u32.p : nullptr; }
 template <> const double *sliced_val<double>(const Matrix &M) { return M.sval_f64.p; }
 template <typename VT>
-const void *persistent_kernel(bool sharded, int long_mode) {
+const void *persistent_kernel(bool sharded, int long_mode, bool accel) {
+  if (accel) return long_mode == 2 ? (const void *)fused_small_persistent<VT, false, 2, true>
+                  : long_mode == 1 ? (const void *)fused_small_persistent<VT, false, 1, true>
+                                   : (const void *)fused_small_persistent<VT, false, 0, true>;
   if (sharded) return long_mode == 2 ? (const void *)fused_small_persistent<VT, true, 2>
                     : long_mode == 1 ? (const void *)fused_small_persistent<VT, true, 1> : (const void *)fused_small_persistent<VT, true, 0>;
   return long_mode == 2 ? (const void *)fused_small_persistent<VT, false, 2>
@@ -1815,34 +1909,43 @@ double loss(Matrix &M, const double *theta, int64_t ntheta, const double cw[2], 
   return r;
 }
 
-void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], double lambda, double l2,
-              double step_factor, double epsilon, double epsilon_loss, int64_t max_iter, double hook[2],
-              int64_t *iters, double *delta) {
-  require_ready();
-  check_theta(M, ntheta, 0);
-  KL_REQUIRE(M.has_labels, "proxgrad: the matrix has no labels (kmerlr_matrix_set_labels)");
-  KL_REQUIRE(M.n_global > 0, "proxgrad: empty data set");
-  Trace tr("proxgrad");
+// the body of proxgrad and proxgrad_accel: they differ in the kernels' ACCEL instantiation and in y and the
+// accelerated state, which travel with theta and the iteration state (y == nullptr: ISTA)
+static void proxgrad_run(Matrix &M, double *theta, double *y, double *t_acc, int64_t ntheta, const double cw[2],
+                         double lambda, double l2, double step_factor, double epsilon, double epsilon_loss,
+                         int64_t max_iter, double hook[2], int64_t *iters, double *delta, int64_t *restarts) {
+  const bool accel = y != nullptr;
+  Trace tr(accel ? "proxgrad_accel" : "proxgrad");
   // estimate_step_size (kmerLr_estimator_proximal.go:54-76)
   double L = 0.25 * (matrix_maxsq(M) + 1.0) + l2 / (double)M.n_global;
   double step = 1.0 / (2.0 * L + std::fmin(2.0 * l2, L)) * step_factor;
   Work wk; alloc_work(M, ntheta, wk);
   set_scale(M, wk, cw);
-  // theta and the iteration state travel through the pinned staging buffer (theta first, the state behind it)
-  double *hth = (double *)host_staging((size_t)ntheta * sizeof(double) + sizeof(PgState));
-  PgState *hst = reinterpret_cast<PgState *>(hth + ntheta);
-  memcpy(hth, theta, (size_t)ntheta * sizeof(double));
-  wk.theta.upload(hth, (size_t)ntheta);
-  DevBuf<PgState> st(1);
-  PgState h{};
+  // theta and the iteration state travel through the pinned staging buffer (theta first, the state behind it).
+  // Accelerated: the point the row pass reads (y) first, then theta, then the state.
+  const int64_t nv = accel ? 2 * ntheta : ntheta;
+  if (accel) wk.theta.alloc((size_t)nv);
+  double *hth = (double *)host_staging((size_t)nv * sizeof(double) + sizeof(PgStateAccel));
+  PgStateAccel *hst = reinterpret_cast<PgStateAccel *>(hth + nv);
+  if (accel) {
+    memcpy(hth, y, (size_t)ntheta * sizeof(double));
+    memcpy(hth + ntheta, theta, (size_t)ntheta * sizeof(double));
+  } else {
+    memcpy(hth, theta, (size_t)ntheta * sizeof(double));
+  }
+  wk.theta.upload(hth, (size_t)nv);
+  DevBuf<PgStateAccel> st(1);
+  PgStateAccel h{};
   h.iter = 0; h.done = max_iter > 0 ? 0 : 1; h.first = 1; h.delta = 0.0;
   h.loss_old = hook ? hook[0] : NAN; h.loss_new = hook ? hook[1] : NAN; h.lossval = NAN; h.error = 0;
+  h.t = accel ? *t_acc : 1.0; h.restarts = 0;
   *hst = h;
   st.upload(hst, 1);
   const double inv_n = 1.0 / (double)M.n_global;
   // reduced matrices: long batches between host round trips.  The choice of the path uses quantities that are
   // the same on every rank (a rank with an empty shard must issue the same collectives as the others)
   const bool small = ntheta <= SMALL_MAX_THETA && !use_implicit(M);
+  KL_INVARIANT(!accel || (small && !M.sharded));
   // the kernels of reduced matrices accumulate the columns and the bias with their own scales (set_scale), as the
   // full-space pass does: the same integers G as fused_kernel
   // the passes of a batch are ONE cooperative launch (grid barriers instead of launches); sharded matrices
@@ -1876,8 +1979,8 @@ void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], doub
         dispatch_vt(M, [&](auto *tag) {
           using VT = typename std::remove_pointer<decltype(tag)>::type;
           if (smem > 16 * 1024)
-            KL_CUDA(cudaFuncSetAttribute(persistent_kernel<VT>(M.sharded, mode), cudaFuncAttributeMaxDynamicSharedMemorySize, 32 * 1024));
-          KL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, persistent_kernel<VT>(M.sharded, mode), PERSIST_THREADS, smem));
+            KL_CUDA(cudaFuncSetAttribute(persistent_kernel<VT>(M.sharded, mode, accel), cudaFuncAttributeMaxDynamicSharedMemorySize, 32 * 1024));
+          KL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, persistent_kernel<VT>(M.sharded, mode, accel), PERSIST_THREADS, smem));
         });
         if (ctx().persist_bps > 0 && ctx().persist_bps < per_sm) per_sm = ctx().persist_bps;
         return per_sm;
@@ -1955,7 +2058,7 @@ void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], doub
                         &npass, &inv_scale, &inv_scale0, &lam, &el, &stp_size, &eps, &mi, &pbp, &gx, &scr, &abortp, &lv};
         if (ctx().profiling) profile_begin("fused_small_persistent");
         const cudaError_t e = cudaLaunchCooperativeKernel(
-            persistent_kernel<VT>(M.sharded, long_mode),
+            persistent_kernel<VT>(M.sharded, long_mode, accel),
             dim3((unsigned)small_blocks), dim3(PERSIST_THREADS), args, dyn_smem, ctx().stream);
         if (ctx().profiling) profile_end();
         if (e == cudaErrorCooperativeLaunchTooLarge && !M.sharded) {
@@ -1976,6 +2079,11 @@ void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], doub
       if (small) {
         dispatch_vt(M, [&](auto *tag) {
           using VT = typename std::remove_pointer<decltype(tag)>::type;
+          if (accel)
+            KL_LAUNCH((fused_small_kernel<VT, true>), (unsigned)small_blocks, 256, 0, M.rows(), M.col.p, csr_val<VT>(M), M.n,
+                      ntheta, wk.theta.p, M.labels.p, cw[0], cw[1], inv_n, wk.scale, wk.scale0, wk.G.p, blockloss.p, st.p,
+                      scatter, counter.p, wk.inv_scale, wk.inv_scale0, lambda, epsilon_loss, step, epsilon, (long long)max_iter);
+          else
           KL_LAUNCH((fused_small_kernel<VT>), (unsigned)small_blocks, 256, 0, M.rows(), M.col.p, csr_val<VT>(M), M.n, ntheta,
                     wk.theta.p, M.labels.p, cw[0], cw[1], inv_n, wk.scale, wk.scale0, wk.G.p, blockloss.p, st.p, scatter,
                     M.sharded ? (unsigned int *)nullptr : counter.p, wk.inv_scale, wk.inv_scale0, lambda, epsilon_loss, step,
@@ -2020,7 +2128,7 @@ void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], doub
     }
     // theta comes down with the state: a batch is usually the last one, and then no second round trip is needed
     st.download(hst, 1);
-    wk.theta.download(hth, (size_t)ntheta);
+    wk.theta.download(hth, (size_t)nv);
     host_staging_done();
     sync_stream();
     h = *hst;
@@ -2028,11 +2136,46 @@ void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], doub
     if (M.sharded) comm_check_peer_errors();
     if (h.done == 1) break;
   }
-  memcpy(theta, hth, (size_t)ntheta * sizeof(double));
+  if (accel) {
+    memcpy(y, hth, (size_t)ntheta * sizeof(double));
+    memcpy(theta, hth + ntheta, (size_t)ntheta * sizeof(double));
+    *t_acc = h.t;
+    if (restarts) *restarts = (int64_t)h.restarts;
+  } else {
+    memcpy(theta, hth, (size_t)ntheta * sizeof(double));
+  }
   tr.mark("iterations");
   if (hook) { hook[0] = h.loss_old; hook[1] = h.loss_new; }
   if (iters) *iters = (int64_t)h.iter;
   if (delta) *delta = h.delta;
+}
+
+void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], double lambda, double l2,
+              double step_factor, double epsilon, double epsilon_loss, int64_t max_iter, double hook[2],
+              int64_t *iters, double *delta) {
+  require_ready();
+  check_theta(M, ntheta, 0);
+  KL_REQUIRE(M.has_labels, "proxgrad: the matrix has no labels (kmerlr_matrix_set_labels)");
+  KL_REQUIRE(M.n_global > 0, "proxgrad: empty data set");
+  proxgrad_run(M, theta, nullptr, nullptr, ntheta, cw, lambda, l2, step_factor, epsilon, epsilon_loss, max_iter, hook,
+               iters, delta, nullptr);
+}
+
+void proxgrad_accel(Matrix &M, double *theta, double *y, double *t, int64_t ntheta, const double cw[2], double lambda,
+                    double l2, double step_factor, double epsilon, double epsilon_loss, int64_t max_iter, double hook[2],
+                    int64_t *iters, double *delta, int64_t *restarts) {
+  require_ready();
+  KL_REQUIRE(theta && y && t && cw, "proxgrad_accel: null argument (theta, y, t and class_w are required)");
+  KL_REQUIRE(std::isfinite(*t) && *t >= 1.0, "proxgrad_accel: the momentum t must be finite and >= 1 (1 = fresh start)");
+  check_theta(M, ntheta, 0);
+  KL_REQUIRE(M.has_labels, "proxgrad_accel: the matrix has no labels (kmerlr_matrix_set_labels)");
+  KL_REQUIRE(M.n_global > 0, "proxgrad_accel: empty data set");
+  KL_REQUIRE(!M.sharded, "proxgrad_accel: sharded matrices are not supported (one GPU, reduced matrices only)");
+  KL_REQUIRE(ntheta <= SMALL_MAX_THETA && !use_implicit(M),
+             "proxgrad_accel: reduced matrices only (at most 1023 columns, stored rows; not a matrix straight from "
+             "kmerlr_extract)");
+  proxgrad_run(M, theta, y, t, ntheta, cw, lambda, l2, step_factor, epsilon, epsilon_loss, max_iter, hook, iters, delta,
+               restarts);
 }
 
 }  // namespace kl
