@@ -16,7 +16,8 @@
 //              bitmap level too when the rows are too long for the register sort;
 //   * k >= 8   "sorted levels": per level ONE bitonic sort of the canonical codes in registers --
 //              in-register compare-exchanges below distance E, warp shuffles above; a run of equal
-//              keys is a class, its length the count.
+//              keys is a class, its length the count.  Under revcomp with N <= 8 the keys are 16-bit,
+//              two to a register (warp_sort16).
 // Rows leave the kernel sorted by (k, code) = by final column index; columns are ranks in the
 // bitmap of observed (or frozen) classes; observed classes are gathered per block in shared memory.
 // Host sequences (kmerlr_extract) arrive in chunks on a copy stream while earlier chunks are

@@ -142,6 +142,122 @@ __device__ __forceinline__ void warp_sort(uint32_t (&K)[E], unsigned lane) {
   }
 }
 
+// ---- the same network on 16-bit keys, two to a register (levels k <= PACK_MAX) -------------------
+// P[q] holds the keys at sorted indices lane*E + q (low half) and lane*E + q + E/2 (high half).  Every
+// stage at an in-lane distance below E/2, and every cross-lane half-cleaner, pairs low halves with low
+// halves and high halves with high halves, so one __vminu2 / __vmaxu2 / shuffle serves two keys.  Only
+// the stages that pair the two halves of a lane (distance E/2, and the flips of the in-lane merge of E
+// keys and of the cross-lane merges) swap halves with a PRMT.  0xFFFF is the sentinel: under revcomp
+// no canonical code of a level k <= 8 is 0xFFFF (TTTTTTTT canonicalises to AAAAAAAA).
+constexpr int PACK_MAX = 8;
+__device__ __forceinline__ uint32_t swap_halves(uint32_t x) { return __byte_perm(x, 0u, 0x1032); }
+__device__ __forceinline__ void ce2(uint32_t &a, uint32_t &b) {
+  uint32_t lo = __vminu2(a, b), hi = __vmaxu2(a, b);
+  a = lo; b = hi;
+}
+
+template <int E>
+__device__ __forceinline__ void warp_sort16(uint32_t (&P)[E / 2], unsigned lane) {
+  constexpr int H = E / 2;
+#pragma unroll
+  for (int k = 2; k <= 32 * E; k <<= 1) {
+    // first stage of the merge: partner = i ^ (k-1)
+    if (k <= H) {
+#pragma unroll
+      for (int q = 0; q < H; q++) {
+        int pq = q ^ (k - 1);
+        if (pq > q) ce2(P[q], P[pq]);
+      }
+    } else if (k == E) {
+      // index q pairs with E-1-q (the high half of P[H-1-q]), index q+H with H-1-q (its low half)
+#pragma unroll
+      for (int q = 0; 2 * q < H; q++) {
+        const uint32_t b = swap_halves(P[H - 1 - q]);
+        const uint32_t mn = __vminu2(P[q], b), mx = __vmaxu2(P[q], b);
+        P[q] = __byte_perm(mn, mx, 0x7610);           // index q: min, index q+H: max
+        P[H - 1 - q] = __byte_perm(mn, mx, 0x5432);   // index H-1-q: min, index E-1-q: max
+      }
+    } else {
+      const int lm = k / E - 1;                       // lane xor mask
+      const bool keepmin = (lane & ((k / E) >> 1)) == 0;
+#pragma unroll
+      for (int q = 0; 2 * q < H; q++) {
+        uint32_t a = P[q], b = P[H - 1 - q];
+        uint32_t va = swap_halves(__shfl_xor_sync(0xffffffffu, b, lm));   // partner's (K[E-1-q], K[H-1-q])
+        uint32_t vb = swap_halves(__shfl_xor_sync(0xffffffffu, a, lm));   // partner's (K[H+q], K[q])
+        P[q] = keepmin ? __vminu2(a, va) : __vmaxu2(a, va);
+        P[H - 1 - q] = keepmin ? __vminu2(b, vb) : __vmaxu2(b, vb);
+      }
+    }
+    // remaining half-cleaners
+#pragma unroll
+    for (int j = k / 4; j >= 1; j >>= 1) {
+      if (j < H) {
+#pragma unroll
+        for (int q = 0; q < H; q++)
+          if ((q & j) == 0) ce2(P[q], P[q | j]);
+      } else if (j == H) {
+#pragma unroll
+        for (int q = 0; q < H; q++) {
+          const uint32_t s = swap_halves(P[q]);
+          P[q] = __byte_perm(__vminu2(P[q], s), __vmaxu2(P[q], s), 0x7610);
+        }
+      } else {
+        const int lm = j / E;
+        const bool keepmin = (lane & lm) == 0;
+#pragma unroll
+        for (int q = 0; q < H; q++) {
+          uint32_t v = __shfl_xor_sync(0xffffffffu, P[q], lm);
+          P[q] = keepmin ? __vminu2(P[q], v) : __vmaxu2(P[q], v);
+        }
+      }
+    }
+  }
+}
+
+// A lane's sorted keys as emit_sorted reads them: key(r) at sorted index lane*E + r, the last one, and the
+// mask of run starts (bit r: key(r) differs from the key before it; prevlast: the previous lane's last key).
+template <int E>
+struct Keys32 {
+  const uint32_t (&K)[E];
+  __device__ __forceinline__ uint32_t key(int r) const { return K[r]; }
+  __device__ __forceinline__ uint32_t last() const { return K[E - 1]; }
+  template <class MaskT>
+  __device__ __forceinline__ MaskT bounds(uint32_t prevlast, unsigned) const {
+    MaskT bnd = (MaskT)(K[0] != prevlast);
+#pragma unroll
+    for (int r = 1; r < E; r++) bnd |= (MaskT)(K[r] != K[r - 1]) << r;
+    return bnd;
+  }
+};
+template <int E>
+struct Keys16 {
+  static constexpr int H = E / 2;
+  const uint32_t (&P)[H];
+  __device__ __forceinline__ uint32_t key(int r) const { return r < H ? P[r] & 0xFFFFu : P[r - H] >> 16; }
+  __device__ __forceinline__ uint32_t last() const { return P[H - 1] >> 16; }
+  template <class MaskT>
+  __device__ __forceinline__ MaskT bounds(uint32_t prevlast, unsigned lane) const {
+    // __vsetne2 compares both halves at once: bit 0 of the result is index q, bit 16 index q + H
+    // (lane 0 starts a run at index 0 whatever the low half of NOKEY compares to)
+    const uint32_t s0 = __vsetne2(P[0], __byte_perm(prevlast, P[H - 1], 0x5410)) | (lane == 0 ? 1u : 0u);
+    if constexpr (H <= 16) {
+      uint32_t acc = s0;
+#pragma unroll
+      for (int q = 1; q < H; q++) acc |= __vsetne2(P[q], P[q - 1]) << q;
+      return (MaskT)((acc & ((1u << H) - 1u)) | ((acc >> 16) << H));
+    } else {
+      uint32_t lo = s0 & 1u, hi = s0 >> 16;
+#pragma unroll
+      for (int q = 1; q < H; q++) {
+        const uint32_t s = __vsetne2(P[q], P[q - 1]);
+        lo |= (s & 1u) << q; hi |= (s >> 16) << q;
+      }
+      return (MaskT)lo | ((MaskT)hi << H);
+    }
+  }
+};
+
 struct Emitter {
   uint32_t *sid, *scnt;            // this row's slices of the column / count arrays
   uint32_t *obs, *bitmap;          // observed classes: per-block (shared) and global bitmap
@@ -198,16 +314,14 @@ __host__ __device__ constexpr int ext_threads(int E) { return E <= 16 ? 512 : (E
 // K[r] sits at sorted index lane*E + r.  A run (equal keys) is one class, its length the count; a run
 // is emitted by the lane holding the position right after it.  Ids and counts go through the warp's
 // shared-memory buffer so that the global stores are coalesced.
-template <int E>
-__device__ __forceinline__ void emit_sorted(const uint32_t (&K)[E], unsigned lane, uint32_t *sbuf, Emitter &em,
+template <int E, class Keys>
+__device__ __forceinline__ void emit_sorted(const Keys &K, unsigned lane, uint32_t *sbuf, Emitter &em,
                                             uint32_t idbase, int events, int64_t stride) {
   using MaskT = typename std::conditional<(E <= 32), uint32_t, unsigned long long>::type;
-  uint32_t prevlast = __shfl_up_sync(0xffffffffu, K[E - 1], 1);
+  uint32_t prevlast = __shfl_up_sync(0xffffffffu, K.last(), 1);
   if (lane == 0) prevlast = NOKEY;
   // bit r of bnd: a run starts at this lane's key r (sorted index lane*E + r)
-  MaskT bnd = (MaskT)(K[0] != prevlast);
-#pragma unroll
-  for (int r = 1; r < E; r++) bnd |= (MaskT)(K[r] != K[r - 1]) << r;
+  const MaskT bnd = K.template bounds<MaskT>(prevlast, lane);
   // a run is emitted by the position right after it: every boundary but sorted index 0
   const MaskT cls = lane == 0 ? (bnd & ~(MaskT)1) : bnd;
   const int c = sizeof(MaskT) == 4 ? __popc((uint32_t)cls) : __popcll(cls);
@@ -224,35 +338,30 @@ __device__ __forceinline__ void emit_sorted(const uint32_t (&K)[E], unsigned lan
   const int nvalid = __shfl_sync(0xffffffffu, mx, 31);
   int start0 = __shfl_up_sync(0xffffffffu, mx, 1);   // last boundary before this lane's keys
   if (lane == 0) start0 = 0;
-  // round 1: ids
+  // the runs this lane emits, in sorted order: f(j = entry of the level, r, count).  The run emitted at key r
+  // started at the last boundary below r (start0 when this lane has none below r); j counts up from base.
+  auto each_run = [&](auto &&f) {
+    int j = base;
 #pragma unroll
-  for (int r = 0; r < E; r++) {
-    if ((cls >> r) & 1) {
-      const MaskT below = cls & (((MaskT)1 << r) - 1);
-      const int j = base + (sizeof(MaskT) == 4 ? __popc((uint32_t)below) : __popcll(below));
-      sbuf[sw(j)] = idbase + (r == 0 ? prevlast : K[r > 0 ? r - 1 : 0]);
-    }
-  }
+    for (int r = 0; r < E; r++)
+      if ((cls >> r) & 1) {
+        const MaskT bbelow = bnd & (((MaskT)1 << r) - 1);
+        const int st = bbelow ? (int)lane * E + (sizeof(MaskT) == 4 ? 31 - __clz((uint32_t)bbelow) : 63 - __clzll(bbelow))
+                              : start0;
+        f(j, r, (uint32_t)((int)lane * E + r - st)); j++;
+      }
+  };
+  // round 1: ids
+  each_run([&](int j, int r, uint32_t) { sbuf[sw(j)] = idbase + (r == 0 ? prevlast : K.key(r > 0 ? r - 1 : 0)); });
   __syncwarp();
   // binarized rows feeding the matrix-free logistic pass: a run of r > 1 equal keys leaves r - 1 repeat
   // events (the column of its class) at the tail of the row's slots, in sorted order (while sbuf holds the ids)
   auto repeat_events = [&]() {
     uint32_t extra = 0;
-#pragma unroll
-    for (int r = 0; r < E; r++) {
-      if ((cls >> r) & 1) {
-        const MaskT bbelow = bnd & (((MaskT)1 << r) - 1);
-        const int st = bbelow ? (int)lane * E + (sizeof(MaskT) == 4 ? 31 - __clz((uint32_t)bbelow) : 63 - __clzll(bbelow))
-                              : start0;
-        const uint32_t cnt = (uint32_t)((int)lane * E + r - st);
-        if (cnt > 1) {
-          const MaskT below = cls & (((MaskT)1 << r) - 1);
-          const int j = base + (sizeof(MaskT) == 4 ? __popc((uint32_t)below) : __popcll(below));
-          uint32_t col;
-          if (em.column(sbuf[sw(j)], col) || !em.filter) extra += cnt - 1;
-        }
-      }
-    }
+    each_run([&](int j, int, uint32_t cnt) {
+      uint32_t col;
+      if (cnt > 1 && (em.column(sbuf[sw(j)], col) || !em.filter)) extra += cnt - 1;
+    });
     uint32_t incl = extra;
 #pragma unroll
     for (int o = 1; o < 32; o <<= 1) {
@@ -263,22 +372,11 @@ __device__ __forceinline__ void emit_sorted(const uint32_t (&K)[E], unsigned lan
     if (tot == 0) return;
     uint32_t *tail = em.sid + stride - 1;
     uint32_t pos = em.ev + incl - extra;
-#pragma unroll
-    for (int r = 0; r < E; r++) {
-      if ((cls >> r) & 1) {
-        const MaskT bbelow = bnd & (((MaskT)1 << r) - 1);
-        const int st = bbelow ? (int)lane * E + (sizeof(MaskT) == 4 ? 31 - __clz((uint32_t)bbelow) : 63 - __clzll(bbelow))
-                              : start0;
-        const uint32_t cnt = (uint32_t)((int)lane * E + r - st);
-        if (cnt > 1) {
-          const MaskT below = cls & (((MaskT)1 << r) - 1);
-          const int j = base + (sizeof(MaskT) == 4 ? __popc((uint32_t)below) : __popcll(below));
-          uint32_t col;
-          if (em.column(sbuf[sw(j)], col) || !em.filter)
-            for (uint32_t x = 1; x < cnt; x++) tail[-(int64_t)(pos++)] = col;
-        }
-      }
-    }
+    each_run([&](int j, int, uint32_t cnt) {
+      uint32_t col;
+      if (cnt > 1 && (em.column(sbuf[sw(j)], col) || !em.filter))
+        for (uint32_t x = 1; x < cnt; x++) tail[-(int64_t)(pos++)] = col;
+    });
     em.ev += tot;
   };
   if (!em.filter) {
@@ -301,18 +399,7 @@ __device__ __forceinline__ void emit_sorted(const uint32_t (&K)[E], unsigned lan
     }
     __syncwarp();
     if (!em.binarize) {
-#pragma unroll
-      for (int r = 0; r < E; r++) {
-        if ((cls >> r) & 1) {
-          const MaskT below = cls & (((MaskT)1 << r) - 1), bbelow = bnd & (((MaskT)1 << r) - 1);
-          const int j = base + (sizeof(MaskT) == 4 ? __popc((uint32_t)below) : __popcll(below));
-          const int st = bbelow ? (int)lane * E + (sizeof(MaskT) == 4 ? 31 - __clz((uint32_t)bbelow) : 63 - __clzll(bbelow))
-                                : start0;
-          const uint32_t cnt = (uint32_t)((int)lane * E + r - st);
-          sbuf[sw(j)] = cnt;
-          em.stat(cnt);
-        }
-      }
+      each_run([&](int j, int, uint32_t cnt) { sbuf[sw(j)] = cnt; em.stat(cnt); });
       __syncwarp();
       for (int i = lane; i < total; i += 32) em.scnt[em.cursor + i] = sbuf[sw(i)];
       __syncwarp();
@@ -342,16 +429,7 @@ __device__ __forceinline__ void emit_sorted(const uint32_t (&K)[E], unsigned lan
   __syncwarp();
   // round 2: counts = distance to the previous boundary
   if (!em.binarize) {
-#pragma unroll
-    for (int r = 0; r < E; r++) {
-      if ((cls >> r) & 1) {
-        const MaskT below = cls & (((MaskT)1 << r) - 1), bbelow = bnd & (((MaskT)1 << r) - 1);
-        const int j = base + (sizeof(MaskT) == 4 ? __popc((uint32_t)below) : __popcll(below));
-        const int st = bbelow ? (int)lane * E + (sizeof(MaskT) == 4 ? 31 - __clz((uint32_t)bbelow) : 63 - __clzll(bbelow))
-                              : start0;
-        sbuf[sw(j)] = (uint32_t)((int)lane * E + r - st);
-      }
-    }
+    each_run([&](int j, int, uint32_t cnt) { sbuf[sw(j)] = cnt; });
     __syncwarp();
     uint32_t k2 = 0;
     for (int i0 = 0, it = 0; i0 < total; i0 += 32, it++) {
@@ -401,8 +479,10 @@ struct XWindow {
 // E = keys per lane of the register sort (0: no sorted levels, sequences of any length)
 // OPT: the strand operation when it is known at compile time (1 = revcomp, the common case), -1 = P.op
 // EV: binarized rows that also leave their table-level class bitmap and repeat events (XParams::events)
-template <int E, int OPT, bool EV>
+// PK: revcomp with N <= PACK_MAX: the sorted levels take the 16-bit network (warp_sort16)
+template <int E, int OPT, bool EV, bool PK>
 __global__ void __launch_bounds__(ext_threads(E), 2) extract_kernel(const XParams P) {
+  static_assert(!PK || (E >= 2 && OPT == 1), "the 16-bit sort keys need revcomp and two keys per lane");
   constexpr int EE = E > 0 ? E : 1;
   extern __shared__ __align__(16) uint32_t smem[];
   const unsigned lane = lane_id();
@@ -895,16 +975,25 @@ __global__ void __launch_bounds__(ext_threads(E), 2) extract_kernel(const XParam
     // ---- sorted levels: one register sort of the canonical codes per level ---------------------------
     if (has_sort) {
       for (int k = P.s_lo; k <= N; k++) {
-        uint32_t K[EE];
-#pragma unroll
-        for (int r = 0; r < EE; r++) {
-          const uint32_t f = FWL[r];
+        auto key = [&](uint32_t f) -> uint32_t {
           uint32_t c = (f >> 4) >> (2 * (N - k));
           if (two && !single_sorted) c = min(c, kmer_op(c, k, op));
-          K[r] = (int)(f & 15u) >= k ? c : SENT;
+          return (int)(f & 15u) >= k ? c : SENT;
+        };
+        if constexpr (PK) {
+          // 16-bit keys, two to a register (the low 16 bits of SENT are the sentinel 0xFFFF)
+          uint32_t K2[E / 2];
+#pragma unroll
+          for (int q = 0; q < E / 2; q++) K2[q] = __byte_perm(key(FWL[q]), key(FWL[q + E / 2]), 0x5410);
+          warp_sort16<E>(K2, lane);
+          emit_sorted<E>(Keys16<E>{K2}, lane, tab, em, P.level_off[k], EV ? 1 : 0, P.stride);
+        } else {
+          uint32_t K[EE];
+#pragma unroll
+          for (int r = 0; r < EE; r++) K[r] = key(FWL[r]);
+          warp_sort<EE>(K, lane);
+          emit_sorted<EE>(Keys32<EE>{K}, lane, tab, em, P.level_off[k], EV ? 1 : 0, P.stride);
         }
-        warp_sort<EE>(K, lane);
-        emit_sorted<EE>(K, lane, tab, em, P.level_off[k], EV ? 1 : 0, P.stride);
       }
     }
     // row statistics (exact integers): what the step size and the fixed-point scale of the gradient need
@@ -944,17 +1033,17 @@ __global__ void __launch_bounds__(ext_threads(E), 2) extract_kernel(const XParam
   if (mk) flush_marks();
 }
 
-template <int E, int OPT, bool EV>
+template <int E, int OPT, bool EV, bool PK>
 void launch_extract_op(const XParams &P) {
   // warps per block: the choice that keeps the most warps resident per SM (the block shares one
   // bitmap of observed classes, every warp brings its own working set)
-  KL_CUDA(cudaFuncSetAttribute((extract_kernel<E, OPT, EV>), cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
+  KL_CUDA(cudaFuncSetAttribute((extract_kernel<E, OPT, EV, PK>), cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024));
   int best_wpb = 0, best_per_sm = 0;
   for (int wpb = ext_threads(E) / 32; wpb >= 1; wpb--) {
     size_t smem = ((size_t)P.obs_words + (size_t)wpb * P.warp_words) * sizeof(uint32_t);
     if (smem > (size_t)227 * 1024) continue;
     int per_sm = 0;
-    KL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (extract_kernel<E, OPT, EV>), 32 * wpb, smem));
+    KL_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, (extract_kernel<E, OPT, EV, PK>), 32 * wpb, smem));
     if (per_sm * wpb > best_per_sm * best_wpb) { best_wpb = wpb; best_per_sm = per_sm; }
   }
   KL_REQUIRE(best_wpb > 0, "sequence too long for the shared-memory working set of one warp");
@@ -964,17 +1053,24 @@ void launch_extract_op(const XParams &P) {
   int64_t need = (P.n - P.row0 + wpb - 1) / wpb;
   if (blocks > need) blocks = need;
   if (blocks < 1) blocks = 1;
-  KL_LAUNCH((extract_kernel<E, OPT, EV>), (unsigned)blocks, 32 * wpb, smem, P);
+  KL_LAUNCH((extract_kernel<E, OPT, EV, PK>), (unsigned)blocks, 32 * wpb, smem, P);
 }
 
 template <int E>
 void launch_extract(const XParams &P) {
+  if constexpr (E >= 2) {
+    if (P.op == 1 && P.N <= PACK_MAX) {
+      if (P.events) launch_extract_op<E, 1, true, true>(P);
+      else launch_extract_op<E, 1, false, true>(P);
+      return;
+    }
+  }
   if (P.events) {
-    if (P.op == 1) launch_extract_op<E, 1, true>(P);
-    else launch_extract_op<E, -1, true>(P);
+    if (P.op == 1) launch_extract_op<E, 1, true, false>(P);
+    else launch_extract_op<E, -1, true, false>(P);
   } else {
-    if (P.op == 1) launch_extract_op<E, 1, false>(P);
-    else launch_extract_op<E, -1, false>(P);
+    if (P.op == 1) launch_extract_op<E, 1, false, false>(P);
+    else launch_extract_op<E, -1, false, false>(P);
   }
 }
 
