@@ -145,6 +145,14 @@ int kmerlr_matrix_rows(kmerlr_handle h, int64_t *rowptr, int32_t *col, double *v
 int kmerlr_matrix_set_labels(kmerlr_handle h, const uint8_t *labels, int64_t n);
 int kmerlr_matrix_from_csr(int64_t n, int64_t m, const int64_t *rowptr, const int32_t *col,
                            const double *val, int flags, kmerlr_handle *out);
+/* filterCvGroup (kmerLr_crossvalidation.go:95): rows[0..nrows) of matrix h (any order, repeats allowed: the bootstrap
+ * samples of an ensemble) as a new matrix: same columns, same class numbering, labels carried if h has labels.  The
+ * new handle stays valid after h is freed.  Its len(data.Data) is nrows (kmerlr_matrix_rows_global), so the 1/n of
+ * the loss and L1Reg = lambda n follow the subset.  It keeps every view h has: padded rows straight from the
+ * extraction stay padded, compact rows stay compact, and the matrix-free view of h carries over (it shares h's packed
+ * sequences).  KMERLR_ERR_ARG: nrows <= 0, an index outside [0, n), a null rows or out, and a SHARDED matrix (the
+ * indices of a shard cannot be checked against the rows of the other ranks: take the subset before sharding). */
+int kmerlr_matrix_subset(kmerlr_handle h, const int64_t *rows, int64_t nrows, kmerlr_handle *out);
 /* per column (all ranks): sum of the values, sum of squares, largest value, number of stored entries --
  * what TransformFull.Fit computes its offsets / scales from (kmerLr_transform.go:59-252); count and
  * binarized matrices only.  The transform itself is a reparameterisation of theta on the host side. */

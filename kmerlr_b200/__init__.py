@@ -7,5 +7,5 @@ from .api import (  # noqa: F401
     comm_init_torch, comm_unique_id, compile_test_data, compile_data, compile_training_data, compute_class_weights,
     featureSelector, flatten, from_csr, import_fasta, from_dense, genomicKmerLr, init, last_device_ms, launch_count,
     logisticRegression, option, select_data, shutdown, wiggle_records, saveWindowPredictionsWiggle, class_name, export_kmers,
-    KmerRegularizationPath, Trace,
+    KmerRegularizationPath, Trace, CrossValidation, crossvalidation, cv_groups, cv_scatter,
 )

@@ -21,6 +21,7 @@ SYMBOLS = [
     "kmerlr_sequences_create", "kmerlr_sequences_from_fasta", "kmerlr_sequences_info", "kmerlr_sequences_names",
     "kmerlr_sequences_regions", "kmerlr_sequences_bases", "kmerlr_extract_resident", "kmerlr_extract", "kmerlr_matrix_info", "kmerlr_matrix_rows_global",
     "kmerlr_matrix_classes", "kmerlr_column_moments", "kmerlr_pair_moments", "kmerlr_matrix_transform", "kmerlr_matrix_rows", "kmerlr_matrix_set_labels", "kmerlr_matrix_from_csr",
+    "kmerlr_matrix_subset",
     "kmerlr_free", "kmerlr_coeff_dim", "kmerlr_coeff_ind2sub", "kmerlr_coeff_sub2ind", "kmerlr_linear_pdf",
     "kmerlr_logpdf", "kmerlr_gradient", "kmerlr_loss", "kmerlr_class_weights", "kmerlr_select", "kmerlr_select_from_gradient", "kmerlr_reduce",
     "kmerlr_step_size", "kmerlr_proxgrad", "kmerlr_proxgrad_accel", "kmerlr_coordinate", "kmerlr_window_slots", "kmerlr_score_windows", "kmerlr_predict_windows",
@@ -89,6 +90,7 @@ def lib():
     L.kmerlr_matrix_transform.argtypes = [h, vp, vp, i64, ph]
     L.kmerlr_matrix_set_labels.argtypes = [h, vp, i64]
     L.kmerlr_matrix_from_csr.argtypes = [i64, i64, vp, vp, vp, C.c_int, ph]
+    L.kmerlr_matrix_subset.argtypes = [h, vp, i64, ph]
     L.kmerlr_free.argtypes = [h]
     L.kmerlr_coeff_dim.restype = i64
     L.kmerlr_coeff_dim.argtypes = [i64]

@@ -271,6 +271,20 @@ class KmerDataSet:
         check(lib().kmerlr_class_weights(self.h, _p(cw)))
         return cw
 
+    def subset(self, rows):
+        """filterCvGroup (kmerLr_crossvalidation.go:95): rows[0..len) of this data set (any order, repeats allowed) as a
+        new data set in HBM with the same columns and class numbering; Labels are carried, n_global = len(rows).  It
+        stays valid after this data set is freed."""
+        idx = np.ascontiguousarray(rows, dtype=np.int64).reshape(-1)
+        h = C.c_uint64()
+        check(lib().kmerlr_matrix_subset(self.h, _p(idx), len(idx), h))
+        r = KmerDataSet(h.value)
+        if self.Labels is not None:
+            r.Labels = self.Labels[idx]
+        if getattr(self, "_kmers", None) is not None:
+            r._kmers = self._kmers
+        return r
+
 
 def from_csr(n, m, rowptr, col, val, sharded=False):
     rowptr = np.ascontiguousarray(rowptr, dtype=np.int64)
@@ -733,6 +747,79 @@ class KmerLrEstimator:
             self.estimate_loop(data, n, balance, transform)
             out.append((self.active_idx.copy(), self.Theta.copy()))
         return out
+
+
+# ---------------------------------------------------------------------------------------------------
+# cross-validation (kmerLr_crossvalidation.go:56-211)
+# ---------------------------------------------------------------------------------------------------
+def cv_groups(n, k):
+    """getCvGroups (kmerLr_crossvalidation.go:56) without its math/rand shuffle: row i goes to fold i mod k.  Go's
+    generator cannot be reproduced here (SURVEY §2), so a caller that needs the reference's folds passes its fold ids
+    to crossvalidation instead."""
+    if k < 1:
+        raise KmerLrError(_lib.ERR_ARG, "cv_groups: k must be at least 1")
+    return np.arange(n, dtype=np.int64) % k
+
+
+def cv_scatter(fold_ids, held_out):
+    """the held-out results of every fold back at the rows' original positions: held_out[f] lists fold f's rows in
+    ascending row order (the order crossvalidation takes its test subset in), folds in ascending order of their id"""
+    fold_ids = np.asarray(fold_ids)
+    out = np.zeros(len(fold_ids))
+    for f, v in zip(np.unique(fold_ids), held_out):
+        out[np.nonzero(fold_ids == f)[0]] = v
+    return out
+
+
+class CrossValidation:
+    """what crossvalidation returns.  Folds: the fold ids in ascending order; Models[f][j] = (active_idx, Theta,
+    Transform) of fold f's estimator after target LambdaAuto[j]; Predictions[j] = the held-out LogPdf of every row
+    under the model of target j that was fitted without the row's fold, at the row's original position (the
+    reference's CV .table); Loss[f][j] = the held-out Loss of fold f at target j (its _loss.table)."""
+
+    def __init__(self, folds, models, predictions, loss):
+        self.Folds, self.Models, self.Predictions, self.Loss = folds, models, predictions, loss
+
+
+def crossvalidation(data, fold_ids, make_estimator, LambdaAuto, balance=False, transform_kind=None):
+    """crossvalidation / learn_cv (kmerLr_crossvalidation.go:167-211) on one resident data set with labels.  Every
+    fold is a row subset of `data` (same columns and class numbering): its training rows are all rows of the other
+    folds.  Per fold, one after the other: make_estimator() gives a fresh KmerLrEstimator; the transform of
+    `transform_kind` is fitted on the training rows (TransformFull.Fit); Estimate runs over LambdaAuto, warm-started
+    from target to target; after each target the held-out rows are reduced to the model's features (SelectData) and
+    scored (LogPdf, and Loss with the estimator's class weights and no penalty), kmerLr_classifier.go:107-147.  The
+    tables are written by the caller."""
+    fold_ids = np.asarray(fold_ids, dtype=np.int64).reshape(-1)
+    if len(fold_ids) != data.n:
+        raise KmerLrError(_lib.ERR_ARG, "crossvalidation: one fold id per row is needed")
+    folds = np.unique(fold_ids)
+    if len(folds) < 2:
+        raise KmerLrError(_lib.ERR_ARG, "crossvalidation: at least two folds are needed")
+    models, held_out, losses = [], [], []
+    for f in folds:
+        train, test = data.subset(np.nonzero(fold_ids != f)[0]), data.subset(np.nonzero(fold_ids == f)[0])
+        try:
+            est = make_estimator()
+            transform = TransformFull().Fit(train, transform_kind, est.Cooccurrence) if transform_kind else None
+            fm, fp, fl = [], [], []
+            for n in LambdaAuto:
+                est.Estimate(train, [n], balance, transform)
+                fm.append((est.active_idx.copy(), est.Theta.copy(), est.Transform))
+                sel = select_data(test, np.concatenate([[0], est.active_idx]))
+                try:
+                    lr = logisticRegression(est.Theta, est.ClassWeights, 0.0, False, est.Transform)
+                    fp.append(lr.LogPdf(sel))
+                    fl.append(lr.Loss(sel))
+                finally:
+                    sel.free()
+            models.append(fm)
+            held_out.append(fp)
+            losses.append(fl)
+        finally:
+            train.free()
+            test.free()
+    predictions = [cv_scatter(fold_ids, [p[j] for p in held_out]) for j in range(len(LambdaAuto))]
+    return CrossValidation(folds, models, predictions, losses)
 
 
 # ---------------------------------------------------------------------------------------------------

@@ -383,6 +383,14 @@ int kmerlr_matrix_from_csr(int64_t n, int64_t m, const int64_t *rowptr, const in
   });
 }
 
+// filterCvGroup (kmerLr_crossvalidation.go:95)
+int kmerlr_matrix_subset(kmerlr_handle h, const int64_t *rows, int64_t nrows, kmerlr_handle *out) {
+  return guarded([&] {
+    KL_REQUIRE(out, "matrix_subset: null argument");
+    *out = register_object(matrix_subset(*lookup<Matrix>(h, "matrix"), rows, nrows));
+  });
+}
+
 int kmerlr_column_moments(kmerlr_handle h, double *sum, double *sumsq, double *absmax, int64_t *count) {
   return guarded([&] {
     KL_REQUIRE(sum && sumsq && absmax && count, "null argument");

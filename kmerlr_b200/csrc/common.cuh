@@ -226,6 +226,11 @@ struct SeqSet : Object {
   // for every other set
   std::string names;
   std::vector<int64_t> name_off;
+  // a row subset's set (subset.cu): len / blk are gathered from the set `words`, whose packed words they point into
+  // (bits2 / inv16 stay empty here).  Its rows need not tile the words, so only the matrix-free logistic pass reads
+  // it; it is never handed out as a handle.  nullptr: the set owns its words.
+  std::shared_ptr<const SeqSet> words;
+  const SeqSet &word_owner() const { return words ? *words : *this; }
 };
 
 enum ValType : int { VAL_ONE = 0, VAL_U32 = 1, VAL_F64 = 2 };
@@ -413,6 +418,8 @@ void ensure_sliced(Matrix &M);
 bool ensure_packed(Matrix &M);      // false: the entries do not fit (real values, large counts, > 1 024 columns)
 bool ensure_blockview(Matrix &M, int grid);   // false: rows per block / counts do not fit the packed word
 std::shared_ptr<Matrix> matrix_reduce(Matrix &M, const int64_t *sel, int64_t nsel);
+// subset.cu
+std::shared_ptr<Matrix> matrix_subset(Matrix &M, const int64_t *rows, int64_t nrows);
 double matrix_maxsq(Matrix &M);
 double matrix_vmax(Matrix &M);
 // logistic.cu

@@ -1681,7 +1681,7 @@ void launch_implicit(Matrix &M, Work &wk, const double cw[2], const PgState *st,
     if (P.c > 1) KL_LAUNCH(imp_build_TS, (unsigned)((tsup + 255) / 256), 256, 0, P, wk.T.p, st);
   }
   ImpArgs A{};
-  A.n = M.n; A.len = S.len.p; A.blk = S.blk.p; A.bits2 = S.bits2.p; A.inv16 = S.inv16.p;
+  A.n = M.n; A.len = S.len.p; A.blk = S.blk.p; A.bits2 = S.word_owner().bits2.p; A.inv16 = S.word_owner().inv16.p;
   A.T = wk.T.p; A.theta = wk.theta.p; A.labels = M.labels.p;
   A.cw0 = cw[0]; A.cw1 = cw[1]; A.inv_n = 1.0 / (double)M.n_global; A.scale = wk.scale;
   A.H = wk.H.p; A.G = wk.G.p; A.lossterm = wk.lossterm.p; A.st = st; A.scatter = scatter;
