@@ -209,7 +209,7 @@ int kmerlr_proxgrad(kmerlr_handle h, double *theta_inout, int64_t ntheta, const 
                     int64_t max_iter, double hook_state[2], int64_t *iters_out, double *delta_out);
 
 /* Accelerated proximal gradient (FISTA with gradient restart, O'Donoghue & Candes), opt-in; reduced matrices on one GPU
- * only.  Same inputs as kmerlr_proxgrad, plus the extrapolated point y (ntheta doubles) and the momentum t, carried in
+ * only (kmerlr_proxgrad_accel_full below takes every one-GPU matrix).  Same inputs as kmerlr_proxgrad, plus the extrapolated point y (ntheta doubles) and the momentum t, carried in
  * and out so that a later call resumes exactly; a fresh start is y = theta, t = 1.  The step s is kmerlr_step_size's.
  * One iteration:
  *   g = gradient at y;  theta' = y - s g, soft-thresholded at s lambda for j >= 1 (the bias is not penalised);
@@ -225,6 +225,17 @@ int kmerlr_proxgrad_accel(kmerlr_handle h, double *theta_inout, double *y_inout,
                           const double class_w[2], double lambda, double l2, double step_factor, double epsilon,
                           double epsilon_loss, int64_t max_iter, double hook_state[2], int64_t *iters_out,
                           double *delta_out, int64_t *restarts_out);
+
+/* The same accelerated iteration, arguments and outputs on every one-GPU matrix kmerlr_proxgrad takes: straight from
+ * kmerlr_extract (counts or binarized, matrix-free or stored rows), imported, reduced of any width, transformed, and
+ * row subsets -- e.g. a fixed-lambda fit on the whole feature space (estimate_fixed).  A reduced matrix of at most 1023
+ * columns (stored rows) runs the body of kmerlr_proxgrad_accel and gives its bits; any other matrix runs the
+ * launch-per-iteration path of kmerlr_proxgrad with the momentum step in its prox tail.  KMERLR_ERR_ARG: a sharded
+ * matrix; t < 1 or not finite; a null theta, y, t or class_w; a matrix without labels; an empty set. */
+int kmerlr_proxgrad_accel_full(kmerlr_handle h, double *theta_inout, double *y_inout, double *t_inout, int64_t ntheta,
+                               const double class_w[2], double lambda, double l2, double step_factor, double epsilon,
+                               double epsilon_loss, int64_t max_iter, double hook_state[2], int64_t *iters_out,
+                               double *delta_out, int64_t *restarts_out);
 
 /* ---- IRLS + coordinate-descent estimator (kmerLr_estimator_coordinate.go:31-139), reduced matrices only
  * (ntheta <= 1024: it keeps the dense Gram matrix, as the reference does), one GPU.  The reference never

@@ -664,8 +664,8 @@ class KmerLrEstimator:
         self.hook_state = np.array([np.nan, np.nan])
         self.path = []
         self.Transform = None            # the selected transform of the last estimate (r.Transform of the reference's KmerLr)
-        # Accelerated: estimate_proximal runs FISTA with gradient restart (kmerlr_proxgrad_accel; reduced matrices, one
-        # GPU).  accel_state = (handle of the data, y, t, restarts of the last call): the momentum carried between calls
+        # Accelerated: estimate_proximal runs FISTA with gradient restart (kmerlr_proxgrad_accel_full; every one-GPU
+        # matrix: reduced ones of any width, and the whole feature space of a fixed-lambda fit).  accel_state = (handle of the data, y, t, restarts of the last call): the momentum carried between calls
         # on the same reduced data, so that a run cut into slices of MaxIterations resumes exactly.
         self.Accelerated = Accelerated
         self.accel_state = None
@@ -687,9 +687,10 @@ class KmerLrEstimator:
         if st is None or st[0] != data_train.h or len(st[1]) != len(theta):
             st = (data_train.h, theta.copy(), 1.0, 0)         # fresh start: y = theta, t = 1
         y, t, restarts = st[1].copy(), C.c_double(st[2]), C.c_int64()
-        check(lib().kmerlr_proxgrad_accel(data_train.h, _p(theta), _p(y), t, len(theta), _p(self.ClassWeights),
-                                          float(lam), self.L2Reg, self.StepSizeFactor, self.Epsilon, self.EpsilonLoss,
-                                          self.MaxIterations, _p(self.hook_state), iters, delta, restarts))
+        check(lib().kmerlr_proxgrad_accel_full(data_train.h, _p(theta), _p(y), t, len(theta), _p(self.ClassWeights),
+                                               float(lam), self.L2Reg, self.StepSizeFactor, self.Epsilon,
+                                               self.EpsilonLoss, self.MaxIterations, _p(self.hook_state), iters, delta,
+                                               restarts))
         self.Theta = theta
         self.accel_state = (data_train.h, y, t.value, restarts.value)
         return iters.value, delta.value

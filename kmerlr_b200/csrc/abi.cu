@@ -513,6 +513,16 @@ int kmerlr_proxgrad_accel(kmerlr_handle h, double *theta_inout, double *y_inout,
   });
 }
 
+int kmerlr_proxgrad_accel_full(kmerlr_handle h, double *theta_inout, double *y_inout, double *t_inout, int64_t ntheta,
+                               const double class_w[2], double lambda, double l2, double step_factor, double epsilon,
+                               double epsilon_loss, int64_t max_iter, double hook_state[2], int64_t *iters_out,
+                               double *delta_out, int64_t *restarts_out) {
+  return guarded([&] {
+    proxgrad_accel_full(*lookup<Matrix>(h, "matrix"), theta_inout, y_inout, t_inout, ntheta, class_w, lambda, l2,
+                        step_factor, epsilon, epsilon_loss, max_iter, hook_state, iters_out, delta_out, restarts_out);
+  });
+}
+
 int kmerlr_coordinate(kmerlr_handle h, double *theta_inout, int64_t ntheta, const double class_w_hook[2], double l1reg,
                       double l2reg, double epsilon, double epsilon_loss, int64_t max_iter, double hook_state[2],
                       int64_t *sweeps_out, double *delta_out) {

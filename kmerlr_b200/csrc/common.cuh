@@ -436,6 +436,9 @@ void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], doub
 void proxgrad_accel(Matrix &M, double *theta, double *y, double *t, int64_t ntheta, const double cw[2], double lambda,
                     double l2, double step_factor, double epsilon, double epsilon_loss, int64_t max_iter, double hook[2],
                     int64_t *iters, double *delta, int64_t *restarts);
+void proxgrad_accel_full(Matrix &M, double *theta, double *y, double *t, int64_t ntheta, const double cw[2],
+                         double lambda, double l2, double step_factor, double epsilon, double epsilon_loss,
+                         int64_t max_iter, double hook[2], int64_t *iters, double *delta, int64_t *restarts);
 // select.cu
 void select(Matrix &M, const double cw[2], int cooc, int64_t N, double theta0, const int64_t *active_idx,
             const double *active_theta, int64_t n_active, int tie, double eps_lambda, double prev_lambda,

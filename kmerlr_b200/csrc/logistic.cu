@@ -58,6 +58,21 @@ __device__ __forceinline__ void pg_stop(PgState *st, double mx, double md, doubl
   else if (st->iter >= max_iter) st->done = 2;
 }
 
+// the accelerated solver's decision at the end of a prox step, from max |theta'|, max |theta' - theta|, the NaN flag and
+// the restart dot product (y - theta').(theta' - theta): ACCEL_STOP (eval_stopping: theta = theta', y and t stay),
+// ACCEL_RESTART (t = 1, y = theta') or ACCEL_MOMENTUM (t' = (1 + sqrt(1 + 4 t^2)) / 2, y = theta' + beta (theta' - theta),
+// beta = (t - 1) / t'; beta is written in this case only)
+enum { ACCEL_STOP = 0, ACCEL_RESTART = 1, ACCEL_MOMENTUM = 2 };
+__device__ __forceinline__ int accel_decide(PgStateAccel *st, double mx, double md, double nn, double dot, double eps,
+                                            long long max_iter, double *beta) {
+  pg_stop(st, mx, md, nn, eps, max_iter);
+  if (st->done == 1) return ACCEL_STOP;
+  if (dot > 0.0) { st->t = 1.0; st->restarts += 1; return ACCEL_RESTART; }
+  const double t0 = st->t, t1 = (1.0 + sqrt(1.0 + 4.0 * (t0 * t0))) / 2.0;
+  *beta = (t0 - 1.0) / t1; st->t = t1;
+  return ACCEL_MOMENTUM;
+}
+
 __device__ __forceinline__ int64_t ind2sub(int64_t n, int64_t k1, int64_t k2) {
   return n + (n * (n - 1) / 2) - (n - k1) * ((n - k1) - 1) / 2 + k2 - k1;
 }
@@ -922,7 +937,7 @@ __device__ __forceinline__ void accel_step(PgStateAccel *st, double *y, double *
                                            double eps, long long max_iter, int replicas, double (*sh)[BT / 32]) {
   constexpr int NW = BT / 32, PER = SMALL_MAX_THETA / BT;
   __shared__ double s_beta;
-  __shared__ int s_mode;       // 0: stopped (theta = theta', y and t stay), 1: restart, 2: momentum
+  __shared__ int s_mode;
   const int t = threadIdx.x, lane = t & 31, wid = t >> 5;
   double tn[PER], dl[PER];
   double mx = 0.0, md = 0.0, nn = 0.0, dot = 0.0;
@@ -955,15 +970,7 @@ __device__ __forceinline__ void accel_step(PgStateAccel *st, double *y, double *
   __syncthreads();
   if (t == 0) {
     for (int w = 1; w < NW; w++) { mx = fmax(mx, sh[0][w]); md = fmax(md, sh[1][w]); nn = fmax(nn, sh[2][w]); dot += sh[3][w]; }
-    pg_stop(st, mx, md, nn, eps, max_iter);
-    if (st->done == 1) {
-      s_mode = 0;
-    } else if (dot > 0.0) {
-      s_mode = 1; st->t = 1.0; st->restarts += 1;
-    } else {
-      const double t0 = st->t, t1 = (1.0 + sqrt(1.0 + 4.0 * (t0 * t0))) / 2.0;
-      s_mode = 2; s_beta = (t0 - 1.0) / t1; st->t = t1;
-    }
+    s_mode = accel_decide(st, mx, md, nn, dot, eps, max_iter, &s_beta);
   }
   __syncthreads();
   const int mode = s_mode;
@@ -973,8 +980,8 @@ __device__ __forceinline__ void accel_step(PgStateAccel *st, double *y, double *
     const int64_t k = t + (int64_t)j * BT;
     if (k < ntheta) {
       xth[k] = tn[j];
-      if (mode == 1) y[k] = tn[j];
-      else if (mode == 2) y[k] = tn[j] + beta * dl[j];
+      if (mode == ACCEL_RESTART) y[k] = tn[j];
+      else if (mode == ACCEL_MOMENTUM) y[k] = tn[j] + beta * dl[j];
     }
   }
 }
@@ -1548,6 +1555,99 @@ __global__ void __launch_bounds__(256) small_p2p_tail_kernel(PgState *st, const 
 
 constexpr int PROX_BLOCKS = 256;
 
+// ---- the accelerated step on the full feature space (FISTA with gradient restart, the iteration of accel_step) ------
+// Two launches in place of prox_update: prox_accel computes theta' and takes the decision, accel_momentum applies it to
+// every coefficient.  The point the pass evaluates (y) sits where ISTA keeps theta, so the pass, its tables and
+// pass_tail's L1 partials see F(y) unchanged.
+struct AccelDecision {
+  int mode;          // ACCEL_STOP / ACCEL_RESTART / ACCEL_MOMENTUM; -1 before the first decision
+  double beta;
+};
+
+// theta' = prox(y - s g) into xnew; per-block max |theta'|, max |theta' - theta|, NaN flag and the restart dot product
+// (y - theta').(theta' - theta), the dot summed per thread in index order, then a fixed tree, then the block partials
+// in block order by the block that finishes last -- the same bits on every run.  That block takes the decision
+// (accel_decide) and leaves it in *dec.  `ticket` is zero on entry and left zero.
+__global__ void __launch_bounds__(256) prox_accel(PgStateAccel *st, const double *__restrict__ y,
+                                                  const double *__restrict__ theta, double *__restrict__ xnew,
+                                                  const unsigned long long *__restrict__ G, double inv_scale,
+                                                  double inv_scale0, int64_t ntheta, double step, double lambda,
+                                                  double *__restrict__ part, double eps, long long max_iter,
+                                                  AccelDecision *dec, unsigned int *ticket) {
+  if (st->done) return;
+  __shared__ double shx[256], shd[256], shn[256], sho[256];
+  double mx = 0.0, md = 0.0, nn = 0.0, dot = 0.0;
+  for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < ntheta; k += (int64_t)gridDim.x * blockDim.x) {
+    const double g = (double)(long long)G[k] * (k == 0 ? inv_scale0 : inv_scale);
+    const double yk = y[k];
+    double t1 = yk - step * g;
+    if (k > 0) t1 = soft_threshold(t1, step * lambda);
+    xnew[k] = t1;
+    const double dl = t1 - theta[k];
+    if (isnan(t1)) nn = 1.0;
+    mx = fmax(mx, fabs(t1));
+    md = fmax(md, fabs(dl));
+    dot += (yk - t1) * dl;
+  }
+  shx[threadIdx.x] = mx; shd[threadIdx.x] = md; shn[threadIdx.x] = nn; sho[threadIdx.x] = dot;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if ((int)threadIdx.x < o) {
+      shx[threadIdx.x] = fmax(shx[threadIdx.x], shx[threadIdx.x + o]);
+      shd[threadIdx.x] = fmax(shd[threadIdx.x], shd[threadIdx.x + o]);
+      shn[threadIdx.x] = fmax(shn[threadIdx.x], shn[threadIdx.x + o]);
+      sho[threadIdx.x] += sho[threadIdx.x + o];
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) {
+    double *p = part + 4 * blockIdx.x;
+    p[0] = shx[0]; p[1] = shd[0]; p[2] = shn[0]; p[3] = sho[0];
+  }
+  if (!last_block(ticket)) return;
+  // the partials of the grid (gridDim.x <= 256, written by other blocks: read in L2)
+  const int nb = (int)gridDim.x, i = (int)threadIdx.x;
+  const bool on = i < nb;
+  shx[i] = on ? __ldcg(part + 4 * i) : 0.0; shd[i] = on ? __ldcg(part + 4 * i + 1) : 0.0;
+  shn[i] = on ? __ldcg(part + 4 * i + 2) : 0.0; sho[i] = on ? __ldcg(part + 4 * i + 3) : 0.0;
+  __syncthreads();
+  if (i == 0) {
+    double d = 0.0;
+    for (int b = 0; b < nb; b++) d += sho[b];
+    sho[0] = d;
+  }
+  for (int o = 128; o > 0; o >>= 1) {
+    if (i < o) {
+      shx[i] = fmax(shx[i], shx[i + o]); shd[i] = fmax(shd[i], shd[i + o]); shn[i] = fmax(shn[i], shn[i + o]);
+    }
+    __syncthreads();
+  }
+  if (i == 0) {
+    *ticket = 0u;
+    double beta = 0.0;
+    dec->mode = accel_decide(st, shx[0], shd[0], shn[0], sho[0], eps, max_iter, &beta);
+    dec->beta = beta;
+  }
+}
+
+// applies the decision of prox_accel: stop: theta = theta' (y stays); restart: y = theta = theta'; momentum:
+// y = theta' + beta (theta' - theta), theta = theta'.  Once the state is stopped the later launches of a batch find
+// done == 1 and a decision that is no longer theirs: a restart or momentum step is not applied again, a stop writes the
+// same theta' again.
+__global__ void __launch_bounds__(256) accel_momentum(const PgStateAccel *st, const AccelDecision *dec,
+                                                      double *__restrict__ y, double *__restrict__ theta,
+                                                      const double *__restrict__ xnew, int64_t ntheta) {
+  const int mode = dec->mode;
+  if (mode < 0 || (st->done == 1 && mode != ACCEL_STOP)) return;
+  const double beta = dec->beta;
+  for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < ntheta; k += (int64_t)gridDim.x * blockDim.x) {
+    const double t1 = xnew[k];
+    if (mode == ACCEL_MOMENTUM) y[k] = t1 + beta * (t1 - theta[k]);
+    else if (mode == ACCEL_RESTART) y[k] = t1;
+    theta[k] = t1;
+  }
+}
+
 struct Work {
   DevBuf<double> theta, w, lossterm, g, red, scalars, gathered, blockmax;
   DevBuf<unsigned long long> G, H;     // H: forward-code tables of the matrix-free pass
@@ -1945,7 +2045,16 @@ static void proxgrad_run(Matrix &M, double *theta, double *y, double *t_acc, int
   // reduced matrices: long batches between host round trips.  The choice of the path uses quantities that are
   // the same on every rank (a rank with an empty shard must issue the same collectives as the others)
   const bool small = ntheta <= SMALL_MAX_THETA && !use_implicit(M);
-  KL_INVARIANT(!accel || (small && !M.sharded));
+  KL_INVARIANT(!accel || !M.sharded);
+  // the accelerated step on the full feature space: theta', the prox step's block partials and its decision
+  DevBuf<double> xnew, accel_part;
+  DevBuf<AccelDecision> decision;
+  if (accel && !small) {
+    xnew.alloc((size_t)ntheta);
+    accel_part.alloc(4 * PROX_BLOCKS);
+    decision.alloc(1);
+    KL_CUDA(cudaMemsetAsync(decision.p, 0xFF, sizeof(AccelDecision), ctx().stream));      // mode -1: none yet
+  }
   // the kernels of reduced matrices accumulate the columns and the bias with their own scales (set_scale), as the
   // full-space pass does: the same integers G as fused_kernel
   // the passes of a batch are ONE cooperative launch (grid barriers instead of launches); sharded matrices
@@ -2121,9 +2230,15 @@ static void proxgrad_run(Matrix &M, double *theta, double *y, double *t_acc, int
                     PROX_BLOCKS, inv_n, epsilon_loss);
         }
         // the loss-only pass (number max_iter) follows the last prox step: the state is stopped (done != 0) by then
-        if (scatter)
+        if (scatter && accel) {
+          KL_LAUNCH(prox_accel, PROX_BLOCKS, 256, 0, st.p, wk.theta.p, wk.theta.p + ntheta, xnew.p, wk.G.p, wk.inv_scale,
+                    wk.inv_scale0, ntheta, step, lambda, accel_part.p, epsilon, (long long)max_iter, decision.p,
+                    wk.tickets.p + 2);
+          KL_LAUNCH(accel_momentum, PROX_BLOCKS, 256, 0, st.p, decision.p, wk.theta.p, wk.theta.p + ntheta, xnew.p, ntheta);
+        } else if (scatter) {
           KL_LAUNCH(prox_update, PROX_BLOCKS, 256, 0, st.p, wk.theta.p, wk.G.p, wk.inv_scale, wk.inv_scale0, ntheta, step, lambda,
                     wk.blockmax.p, epsilon, (long long)max_iter, wk.tickets.p + 2);
+        }
       });
     }
     // theta comes down with the state: a batch is usually the last one, and then no second round trip is needed
@@ -2161,19 +2276,36 @@ void proxgrad(Matrix &M, double *theta, int64_t ntheta, const double cw[2], doub
                iters, delta, nullptr);
 }
 
+// the arguments both accelerated entries refuse (`who` names the entry in the messages)
+static void accel_check(const char *who, Matrix &M, const double *theta, const double *y, const double *t, int64_t ntheta,
+                        const double cw[2]) {
+  const std::string w(who);
+  KL_REQUIRE(theta && y && t && cw, w + ": null argument (theta, y, t and class_w are required)");
+  KL_REQUIRE(std::isfinite(*t) && *t >= 1.0, w + ": the momentum t must be finite and >= 1 (1 = fresh start)");
+  check_theta(M, ntheta, 0);
+  KL_REQUIRE(M.has_labels, w + ": the matrix has no labels (kmerlr_matrix_set_labels)");
+  KL_REQUIRE(M.n_global > 0, w + ": empty data set");
+}
+
 void proxgrad_accel(Matrix &M, double *theta, double *y, double *t, int64_t ntheta, const double cw[2], double lambda,
                     double l2, double step_factor, double epsilon, double epsilon_loss, int64_t max_iter, double hook[2],
                     int64_t *iters, double *delta, int64_t *restarts) {
   require_ready();
-  KL_REQUIRE(theta && y && t && cw, "proxgrad_accel: null argument (theta, y, t and class_w are required)");
-  KL_REQUIRE(std::isfinite(*t) && *t >= 1.0, "proxgrad_accel: the momentum t must be finite and >= 1 (1 = fresh start)");
-  check_theta(M, ntheta, 0);
-  KL_REQUIRE(M.has_labels, "proxgrad_accel: the matrix has no labels (kmerlr_matrix_set_labels)");
-  KL_REQUIRE(M.n_global > 0, "proxgrad_accel: empty data set");
+  accel_check("proxgrad_accel", M, theta, y, t, ntheta, cw);
   KL_REQUIRE(!M.sharded, "proxgrad_accel: sharded matrices are not supported (one GPU, reduced matrices only)");
   KL_REQUIRE(ntheta <= SMALL_MAX_THETA && !use_implicit(M),
              "proxgrad_accel: reduced matrices only (at most 1023 columns, stored rows; not a matrix straight from "
              "kmerlr_extract)");
+  proxgrad_run(M, theta, y, t, ntheta, cw, lambda, l2, step_factor, epsilon, epsilon_loss, max_iter, hook, iters, delta,
+               restarts);
+}
+
+void proxgrad_accel_full(Matrix &M, double *theta, double *y, double *t, int64_t ntheta, const double cw[2],
+                         double lambda, double l2, double step_factor, double epsilon, double epsilon_loss,
+                         int64_t max_iter, double hook[2], int64_t *iters, double *delta, int64_t *restarts) {
+  require_ready();
+  KL_REQUIRE(!M.sharded, "proxgrad_accel_full: sharded matrices are not supported (one GPU)");
+  accel_check("proxgrad_accel_full", M, theta, y, t, ntheta, cw);
   proxgrad_run(M, theta, y, t, ntheta, cw, lambda, l2, step_factor, epsilon, epsilon_loss, max_iter, hook, iters, delta,
                restarts);
 }
