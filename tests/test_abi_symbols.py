@@ -55,6 +55,38 @@ def test_pure_host_entry_points():
     assert sorted(seen) == list(range(1, ci.Dim()))
     from kmerlr_b200 import _lib
     L = _lib.lib()
+    # Sub2Ind decodes a pair index with a floating-point sqrt.  A float64 restatement of that formula is exact at every
+    # index up to m = 20 000 and at the row edges up to m ~ 9.5e7; it first fails near m = 2e8, a pair space far
+    # larger than fits in device memory.  Every index of C4 (m = 2 772), then the row edges and random indices of
+    # m = 65 536 and 10^6.
+    import ctypes as C
+    import numpy as np
+    a_, b_ = C.c_int64(), C.c_int64()
+    sub2ind, ind2sub = L.kmerlr_coeff_sub2ind, L.kmerlr_coeff_ind2sub
+
+    def pair_of(m, j):
+        sub2ind(m, j - 1, a_, b_)
+        return a_.value, b_.value
+
+    m = 2772
+    for a in range(m - 1):
+        first = ind2sub(m, a, a + 1)
+        for b in range(a + 1, m):
+            assert pair_of(m, first + b - a - 1) == (a, b)
+        assert ind2sub(m, a, m - 1) == first + m - a - 2
+    assert ind2sub(m, m - 2, m - 1) == L.kmerlr_coeff_dim(m) - 1 == 3843378
+    rng = np.random.default_rng(0)
+    for m in (65536, 10 ** 6):
+        dim = L.kmerlr_coeff_dim(m)
+        assert dim == (m + 1) * m // 2 + 1
+        assert pair_of(m, m + 1) == (0, 1) and pair_of(m, dim - 1) == (m - 2, m - 1)
+        for a in range(m - 1):
+            first = m + m * (m - 1) // 2 - (m - a) * (m - a - 1) // 2 + 1
+            assert ind2sub(m, a, a + 1) == first
+            assert pair_of(m, first) == (a, a + 1) and pair_of(m, first + m - a - 2) == (a, m - 1)
+        for j in rng.integers(m + 1, dim, 20000):
+            a, b = pair_of(m, int(j))
+            assert 0 <= a < b < m and ind2sub(m, a, b) == j
     assert L.kmerlr_window_slots(300, 200, 10) == 11 and L.kmerlr_window_slots(200, 200, 10) == 0
 
 
