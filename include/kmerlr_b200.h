@@ -237,6 +237,31 @@ int kmerlr_proxgrad_accel_full(kmerlr_handle h, double *theta_inout, double *y_i
                                double epsilon_loss, int64_t max_iter, double hook_state[2], int64_t *iters_out,
                                double *delta_out, int64_t *restarts_out);
 
+/* ---- proximal gradient over the pair-feature space (cooccurrence = 1), one GPU ----
+ * Minimises F(theta) = the mean weighted log-loss of the pair-mode linear predictor (kmerlr_linear_pdf with
+ * cooccurrence = 1) + lambda sum_{j>=1} |theta_j| over ALL ntheta = kmerlr_coeff_dim(m) coefficients: what
+ * kmerlr_proxgrad / kmerlr_proxgrad_accel_full minimise on the explicit expansion kmerlr_reduce(h, 0 .. Dim-1), without
+ * building its pair columns.  (kmerlr_loss keeps the reference's L1 bound of m + 1 in pair mode; the solver's hook
+ * sums lambda |theta_j| over every coefficient, the objective it minimises.)  The matrix is the raw one (counts,
+ * binarized, imported, row subsets, ...), not an expansion.
+ * kmerlr_step_size_pairs: kmerlr_step_size of the pair-expanded rows x~ = (v_j)_j u (v_a v_b)_{a<b},
+ * ||x~||^2 = S2 + (S2^2 - S4) / 2 with S2 = sum v^2, S4 = sum v^4 over the row -- exact integers for counts and
+ * binarized rows (the bits of kmerlr_step_size on the expansion while its sums stay below 2^53), fp64 for real values.
+ * kmerlr_proxgrad_pairs: the arguments, iteration, hook and outputs of kmerlr_proxgrad; kmerlr_proxgrad_pairs_accel:
+ * those of kmerlr_proxgrad_accel_full (theta, y and t in and out, restarts_out).  Both resume exactly from their
+ * outputs.  Each pass gives z, w and the gradient with the kernels and the order of kmerlr_gradient(cooccurrence = 1)
+ * at the point it reads (theta, or y when accelerated).
+ * KMERLR_ERR_ARG (all three where it applies): a sharded matrix; ntheta != kmerlr_coeff_dim(m); a null theta, y, t or
+ * class_w; t < 1 or not finite; a matrix without labels; an empty set. */
+int kmerlr_step_size_pairs(kmerlr_handle h, double l2, double step_factor, double *step_out);
+int kmerlr_proxgrad_pairs(kmerlr_handle h, double *theta_inout, int64_t ntheta, const double class_w[2],
+                          double lambda, double l2, double step_factor, double epsilon, double epsilon_loss,
+                          int64_t max_iter, double hook_state[2], int64_t *iters_out, double *delta_out);
+int kmerlr_proxgrad_pairs_accel(kmerlr_handle h, double *theta_inout, double *y_inout, double *t_inout, int64_t ntheta,
+                                const double class_w[2], double lambda, double l2, double step_factor, double epsilon,
+                                double epsilon_loss, int64_t max_iter, double hook_state[2], int64_t *iters_out,
+                                double *delta_out, int64_t *restarts_out);
+
 /* ---- IRLS + coordinate-descent estimator (kmerLr_estimator_coordinate.go:31-139), reduced matrices only
  * (ntheta <= 1024: it keeps the dense Gram matrix, as the reference does), one GPU.  The reference never
  * calls it and its theta slices alias (:89-91); built with the slices de-aliased, like kmerlr_proxgrad.

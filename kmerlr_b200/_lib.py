@@ -24,7 +24,7 @@ SYMBOLS = [
     "kmerlr_matrix_subset",
     "kmerlr_free", "kmerlr_coeff_dim", "kmerlr_coeff_ind2sub", "kmerlr_coeff_sub2ind", "kmerlr_linear_pdf",
     "kmerlr_logpdf", "kmerlr_gradient", "kmerlr_loss", "kmerlr_class_weights", "kmerlr_select", "kmerlr_select_from_gradient", "kmerlr_reduce",
-    "kmerlr_step_size", "kmerlr_proxgrad", "kmerlr_proxgrad_accel", "kmerlr_proxgrad_accel_full", "kmerlr_coordinate", "kmerlr_window_slots", "kmerlr_score_windows", "kmerlr_predict_windows",
+    "kmerlr_step_size", "kmerlr_proxgrad", "kmerlr_proxgrad_accel", "kmerlr_proxgrad_accel_full", "kmerlr_step_size_pairs", "kmerlr_proxgrad_pairs", "kmerlr_proxgrad_pairs_accel", "kmerlr_coordinate", "kmerlr_window_slots", "kmerlr_score_windows", "kmerlr_predict_windows",
     "kmerlr_score_windows_resident", "kmerlr_wiggle_records", "kmerlr_save_wiggle", "kmerlr_export_kmers", "kmerlr_class_name",
     "kmerlr_export_path", "kmerlr_export_trace",
 ]
@@ -111,6 +111,9 @@ def lib():
     L.kmerlr_proxgrad.argtypes = [h, vp, i64, vp, dbl, dbl, dbl, dbl, dbl, i64, vp, pi64, pdbl]
     L.kmerlr_proxgrad_accel.argtypes = [h, vp, vp, pdbl, i64, vp, dbl, dbl, dbl, dbl, dbl, i64, vp, pi64, pdbl, pi64]
     L.kmerlr_proxgrad_accel_full.argtypes = [h, vp, vp, pdbl, i64, vp, dbl, dbl, dbl, dbl, dbl, i64, vp, pi64, pdbl, pi64]
+    L.kmerlr_step_size_pairs.argtypes = [h, dbl, dbl, pdbl]
+    L.kmerlr_proxgrad_pairs.argtypes = [h, vp, i64, vp, dbl, dbl, dbl, dbl, dbl, i64, vp, pi64, pdbl]
+    L.kmerlr_proxgrad_pairs_accel.argtypes = [h, vp, vp, pdbl, i64, vp, dbl, dbl, dbl, dbl, dbl, i64, vp, pi64, pdbl, pi64]
     L.kmerlr_coordinate.argtypes = [h, vp, i64, vp, dbl, dbl, dbl, dbl, i64, vp, pi64, pdbl]
     L.kmerlr_window_slots.restype = i64
     L.kmerlr_window_slots.argtypes = [i64, i64, i64]

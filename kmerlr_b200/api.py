@@ -665,7 +665,8 @@ class KmerLrEstimator:
         self.path = []
         self.Transform = None            # the selected transform of the last estimate (r.Transform of the reference's KmerLr)
         # Accelerated: estimate_proximal runs FISTA with gradient restart (kmerlr_proxgrad_accel_full; every one-GPU
-        # matrix: reduced ones of any width, and the whole feature space of a fixed-lambda fit).  accel_state = (handle of the data, y, t, restarts of the last call): the momentum carried between calls
+        # matrix: reduced ones of any width, and the whole feature space of a fixed-lambda fit; with Cooccurrence and a
+        # Theta of every pair coefficient of the raw matrix, kmerlr_proxgrad_pairs_accel).  accel_state = (handle of the data, y, t, restarts of the last call): the momentum carried between calls
         # on the same reduced data, so that a run cut into slices of MaxIterations resumes exactly.
         self.Accelerated = Accelerated
         self.accel_state = None
@@ -674,23 +675,26 @@ class KmerLrEstimator:
         """estimate_proximal (kmerLr_estimator_proximal.go:78-120) on the (reduced) data set."""
         theta = np.ascontiguousarray(self.Theta, dtype=np.float64).copy()
         iters, delta = C.c_int64(), C.c_double()
+        # pair mode on the whole data set (estimate_fixed): theta holds every pair coefficient of the raw matrix
+        pairs = bool(self.Cooccurrence) and len(theta) == lib().kmerlr_coeff_dim(data_train.m) != data_train.m + 1
         if self.Accelerated:
-            return self._estimate_accelerated(data_train, lam, theta, iters, delta)
-        check(lib().kmerlr_proxgrad(data_train.h, _p(theta), len(theta), _p(self.ClassWeights), float(lam),
+            return self._estimate_accelerated(data_train, lam, theta, iters, delta, pairs)
+        entry = lib().kmerlr_proxgrad_pairs if pairs else lib().kmerlr_proxgrad
+        check(entry(data_train.h, _p(theta), len(theta), _p(self.ClassWeights), float(lam),
                                     self.L2Reg, self.StepSizeFactor, self.Epsilon, self.EpsilonLoss,
                                     self.MaxIterations, _p(self.hook_state), iters, delta))
         self.Theta = theta
         return iters.value, delta.value
 
-    def _estimate_accelerated(self, data_train, lam, theta, iters, delta):
+    def _estimate_accelerated(self, data_train, lam, theta, iters, delta, pairs=False):
         st = self.accel_state
         if st is None or st[0] != data_train.h or len(st[1]) != len(theta):
             st = (data_train.h, theta.copy(), 1.0, 0)         # fresh start: y = theta, t = 1
         y, t, restarts = st[1].copy(), C.c_double(st[2]), C.c_int64()
-        check(lib().kmerlr_proxgrad_accel_full(data_train.h, _p(theta), _p(y), t, len(theta), _p(self.ClassWeights),
-                                               float(lam), self.L2Reg, self.StepSizeFactor, self.Epsilon,
-                                               self.EpsilonLoss, self.MaxIterations, _p(self.hook_state), iters, delta,
-                                               restarts))
+        entry = lib().kmerlr_proxgrad_pairs_accel if pairs else lib().kmerlr_proxgrad_accel_full
+        check(entry(data_train.h, _p(theta), _p(y), t, len(theta), _p(self.ClassWeights), float(lam), self.L2Reg,
+                    self.StepSizeFactor, self.Epsilon, self.EpsilonLoss, self.MaxIterations, _p(self.hook_state), iters,
+                    delta, restarts))
         self.Theta = theta
         self.accel_state = (data_train.h, y, t.value, restarts.value)
         return iters.value, delta.value

@@ -523,6 +523,36 @@ int kmerlr_proxgrad_accel_full(kmerlr_handle h, double *theta_inout, double *y_i
   });
 }
 
+int kmerlr_step_size_pairs(kmerlr_handle h, double l2, double step_factor, double *step_out) {
+  return guarded([&] {
+    KL_REQUIRE(step_out, "step_size_pairs: null argument");
+    auto M = lookup<Matrix>(h, "matrix");
+    KL_REQUIRE(!M->sharded, "step_size_pairs: sharded matrices are not supported (one GPU)");
+    KL_REQUIRE(M->n_global > 0, "step_size_pairs: empty data set");
+    double L = 0.25 * (matrix_maxsq_pairs(*M) + 1.0) + l2 / (double)M->n_global;
+    *step_out = 1.0 / (2.0 * L + std::fmin(2.0 * l2, L)) * step_factor;
+  });
+}
+
+int kmerlr_proxgrad_pairs(kmerlr_handle h, double *theta_inout, int64_t ntheta, const double class_w[2], double lambda,
+                          double l2, double step_factor, double epsilon, double epsilon_loss, int64_t max_iter,
+                          double hook_state[2], int64_t *iters_out, double *delta_out) {
+  return guarded([&] {
+    proxgrad_pairs(*lookup<Matrix>(h, "matrix"), theta_inout, ntheta, class_w, lambda, l2, step_factor, epsilon,
+                   epsilon_loss, max_iter, hook_state, iters_out, delta_out);
+  });
+}
+
+int kmerlr_proxgrad_pairs_accel(kmerlr_handle h, double *theta_inout, double *y_inout, double *t_inout, int64_t ntheta,
+                                const double class_w[2], double lambda, double l2, double step_factor, double epsilon,
+                                double epsilon_loss, int64_t max_iter, double hook_state[2], int64_t *iters_out,
+                                double *delta_out, int64_t *restarts_out) {
+  return guarded([&] {
+    proxgrad_pairs_accel(*lookup<Matrix>(h, "matrix"), theta_inout, y_inout, t_inout, ntheta, class_w, lambda, l2,
+                         step_factor, epsilon, epsilon_loss, max_iter, hook_state, iters_out, delta_out, restarts_out);
+  });
+}
+
 int kmerlr_coordinate(kmerlr_handle h, double *theta_inout, int64_t ntheta, const double class_w_hook[2], double l1reg,
                       double l2reg, double epsilon, double epsilon_loss, int64_t max_iter, double hook_state[2],
                       int64_t *sweeps_out, double *delta_out) {

@@ -351,6 +351,9 @@ struct Matrix : Object {
   double maxsq = 0.0;
   bool has_vmax = false;
   double vmax = 0.0;
+  // cached max_i ||x~_i||^2 of the pair-expanded rows x~ = (v_j)_j u (v_a v_b)_{a<b} (pair mode's step size)
+  bool has_maxsq_pairs = false;
+  double maxsq_pairs = 0.0;
   // matrix-free view (count matrices produced by extract() without an explicit feature list)
   std::shared_ptr<Implicit> imp;
   // the same two numbers over this rank's rows, when the kernel that wrote the rows computed them
@@ -375,6 +378,10 @@ std::shared_ptr<T> lookup(uint64_t h, const char *what) {
 void exclusive_scan_i64(const int64_t *in, int64_t *out, int64_t n);            // out[n] = total
 void exclusive_scan_u32_to_i64(const uint32_t *in, int64_t *out, int64_t n);    // out[n] = total
 void exclusive_scan_u32(const uint32_t *in, uint32_t *out, int64_t n);          // out[n] = total
+// the same scan queued on the stream with a caller-owned workspace of exclusive_scan_workspace(n) words: no
+// allocation and no synchronisation (a solver's iteration scans without a host round trip)
+int64_t exclusive_scan_workspace(int64_t n);
+void exclusive_scan_u32_async(const uint32_t *in, uint32_t *out, int64_t n, int64_t *workspace);
 // extract.cu
 std::shared_ptr<SeqSet> sequences_create(const uint8_t *seq, const int64_t *off, int64_t n);
 // host sequences that arrive in chunks of whole rows: feed(c) copies chunk c on the copy stream and packs it on the
@@ -421,6 +428,7 @@ std::shared_ptr<Matrix> matrix_reduce(Matrix &M, const int64_t *sel, int64_t nse
 // subset.cu
 std::shared_ptr<Matrix> matrix_subset(Matrix &M, const int64_t *rows, int64_t nrows);
 double matrix_maxsq(Matrix &M);
+double matrix_maxsq_pairs(Matrix &M);   // max_i ||x~_i||^2 of the pair-expanded rows (one GPU)
 double matrix_vmax(Matrix &M);
 // logistic.cu
 void linear_pdf(Matrix &M, const double *theta, int64_t ntheta, int cooc, double *out_host, bool logpdf);
@@ -439,6 +447,12 @@ void proxgrad_accel(Matrix &M, double *theta, double *y, double *t, int64_t nthe
 void proxgrad_accel_full(Matrix &M, double *theta, double *y, double *t, int64_t ntheta, const double cw[2],
                          double lambda, double l2, double step_factor, double epsilon, double epsilon_loss,
                          int64_t max_iter, double hook[2], int64_t *iters, double *delta, int64_t *restarts);
+void proxgrad_pairs(Matrix &M, double *theta, int64_t ntheta, const double cw[2], double lambda, double l2,
+                    double step_factor, double epsilon, double epsilon_loss, int64_t max_iter, double hook[2],
+                    int64_t *iters, double *delta);
+void proxgrad_pairs_accel(Matrix &M, double *theta, double *y, double *t, int64_t ntheta, const double cw[2],
+                          double lambda, double l2, double step_factor, double epsilon, double epsilon_loss,
+                          int64_t max_iter, double hook[2], int64_t *iters, double *delta, int64_t *restarts);
 // select.cu
 void select(Matrix &M, const double cw[2], int cooc, int64_t N, double theta0, const int64_t *active_idx,
             const double *active_theta, int64_t n_active, int tie, double eps_lambda, double prev_lambda,

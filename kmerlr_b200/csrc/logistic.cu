@@ -82,6 +82,8 @@ struct PairTerm {
   uint32_t a, b;
   double theta;
 };
+// at most this many non-zero pair coefficients go to the rows kernel as a list; more take the O(q^2) walk
+constexpr int64_t PAIR_TERMS_MAX = 8192;
 // value of column c in the row [a, b) (columns ascending), 0 when absent
 template <typename VT>
 __device__ __forceinline__ double row_value(const uint32_t *__restrict__ col, const VT *__restrict__ val, int64_t a, int64_t b,
@@ -107,14 +109,21 @@ __device__ __forceinline__ double row_weight(double z, const uint8_t &y, const d
 // rows pass: MODE 0 = z only, 1 = log sigma(z), 2 = w_i and loss term.
 // cooc = 1: pair terms over all pairs of entries of the row (O(q^2) gathers of theta); cooc = 2: over the list of
 // non-zero pair coefficients (`terms`, sorted by coefficient index): two lookups per term and row -- an L1-regularised
-// theta has a handful of them, and 3.84 M coefficients at C4
-template <typename VT, int MODE>
+// theta has a handful of them, and 3.84 M coefficients at C4.
+// DEV_TERMS: the list and its length were built on the device (pair_terms_emit): `cooc` and `nterms` are read from
+// *dev_nterms -- the list when it holds at most PAIR_TERMS_MAX terms, the O(q^2) walk otherwise (collect_pair_terms'
+// rule, taken without a round trip to the host)
+template <typename VT, int MODE, bool DEV_TERMS = false>
 __global__ void rows_kernel(const Rows R, const uint32_t *__restrict__ col,
                             const VT *__restrict__ val, int64_t n, int64_t m, const double *__restrict__ theta,
                             int cooc, const uint8_t *__restrict__ labels, double cw0, double cw1, double inv_n,
                             double *__restrict__ out, double *__restrict__ lossterm, const PgState *st,
-                            const PairTerm *__restrict__ terms, int nterms) {
+                            const PairTerm *__restrict__ terms, int nterms, const int *__restrict__ dev_nterms) {
   if (st && st->done == 1) return;
+  if constexpr (DEV_TERMS) {
+    nterms = *dev_nterms;
+    cooc = nterms <= PAIR_TERMS_MAX ? 2 : 1;
+  }
   int64_t row = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (row >= n) return;
   unsigned lane = lane_id();
@@ -878,14 +887,18 @@ __global__ void __launch_bounds__(256) pass_tail(PgState *st, const ImpParams P,
 // theta <- prox(theta - s g), eval_stopping (kmerLr_estimator_proximal.go:30-52,88-98): a grid-wide update with
 // per-block max |theta|, max |delta| and NaN flag; the block that finishes last takes the decision.  `ticket` is
 // zero on entry and left zero.
+// PAIRS (pair mode): the coefficients k >= m1 = m + 1 are pairs and take g from the fp64 pair gradient gpair[k]
+// (pairs_gradient); the fixed-point G holds the m + 1 single-feature words only.
+template <bool PAIRS = false>
 __global__ void prox_update(PgState *st, double *__restrict__ theta, const unsigned long long *__restrict__ G,
                             double inv_scale, double inv_scale0, int64_t ntheta, double step, double lambda,
-                            double *__restrict__ blockmax, double eps, long long max_iter, unsigned int *ticket) {
+                            double *__restrict__ blockmax, double eps, long long max_iter, unsigned int *ticket,
+                            const double *__restrict__ gpair, int64_t m1) {
   if (st->done) return;
   __shared__ double shx[256], shd[256], shn[256];
   double mx = 0.0, md = 0.0, nn = 0.0;
   for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < ntheta; k += (int64_t)gridDim.x * blockDim.x) {
-    double g = (double)(long long)G[k] * (k == 0 ? inv_scale0 : inv_scale);
+    double g = PAIRS && k >= m1 ? gpair[k] : (double)(long long)G[k] * (k == 0 ? inv_scale0 : inv_scale);
     double t0 = theta[k], t1 = t0 - step * g;
     if (k > 0) t1 = soft_threshold(t1, step * lambda);
     theta[k] = t1;
@@ -1567,18 +1580,20 @@ struct AccelDecision {
 // theta' = prox(y - s g) into xnew; per-block max |theta'|, max |theta' - theta|, NaN flag and the restart dot product
 // (y - theta').(theta' - theta), the dot summed per thread in index order, then a fixed tree, then the block partials
 // in block order by the block that finishes last -- the same bits on every run.  That block takes the decision
-// (accel_decide) and leaves it in *dec.  `ticket` is zero on entry and left zero.
+// (accel_decide) and leaves it in *dec.  `ticket` is zero on entry and left zero.  PAIRS: as prox_update's.
+template <bool PAIRS = false>
 __global__ void __launch_bounds__(256) prox_accel(PgStateAccel *st, const double *__restrict__ y,
                                                   const double *__restrict__ theta, double *__restrict__ xnew,
                                                   const unsigned long long *__restrict__ G, double inv_scale,
                                                   double inv_scale0, int64_t ntheta, double step, double lambda,
                                                   double *__restrict__ part, double eps, long long max_iter,
-                                                  AccelDecision *dec, unsigned int *ticket) {
+                                                  AccelDecision *dec, unsigned int *ticket,
+                                                  const double *__restrict__ gpair, int64_t m1) {
   if (st->done) return;
   __shared__ double shx[256], shd[256], shn[256], sho[256];
   double mx = 0.0, md = 0.0, nn = 0.0, dot = 0.0;
   for (int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; k < ntheta; k += (int64_t)gridDim.x * blockDim.x) {
-    const double g = (double)(long long)G[k] * (k == 0 ? inv_scale0 : inv_scale);
+    const double g = PAIRS && k >= m1 ? gpair[k] : (double)(long long)G[k] * (k == 0 ? inv_scale0 : inv_scale);
     const double yk = y[k];
     double t1 = yk - step * g;
     if (k > 0) t1 = soft_threshold(t1, step * lambda);
@@ -1648,6 +1663,39 @@ __global__ void __launch_bounds__(256) accel_momentum(const PgStateAccel *st, co
   }
 }
 
+// ---- pair mode on the device: the list of non-zero pair coefficients of the point the pass reads -----------------
+// flags[i] = [p[m1 + i] != 0] over the npairs pair coefficients (-0.0 counts as zero, as in collect_pair_terms)
+__global__ void pair_nz_flags(const PgState *st, const double *__restrict__ p, int64_t m1, int64_t npairs,
+                              uint32_t *__restrict__ flags) {
+  if (st->done == 1) return;
+  for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < npairs; i += (int64_t)gridDim.x * blockDim.x)
+    flags[i] = p[m1 + i] != 0.0 ? 1u : 0u;
+}
+
+// pos = the exclusive scan of the flags (pos[npairs] = their sum): terms[pos[i]] = (a, b, p[m + 1 + i]) for every
+// non-zero pair i with pos[i] < PAIR_TERMS_MAX -- coefficient order, the list collect_pair_terms builds on the host --
+// and *count = the number of non-zero pairs, capped at PAIR_TERMS_MAX + 1 (the rows kernel then walks all pairs)
+__global__ void pair_terms_emit(const PgState *st, const double *__restrict__ p, int64_t m, const uint32_t *__restrict__ pos,
+                                int64_t npairs, PairTerm *__restrict__ terms, int *__restrict__ count) {
+  if (st->done == 1) return;
+  const int64_t i0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i0 == 0) { const uint32_t c = pos[npairs]; *count = c > PAIR_TERMS_MAX ? (int)PAIR_TERMS_MAX + 1 : (int)c; }
+  for (int64_t i = i0; i < npairs; i += (int64_t)gridDim.x * blockDim.x) {
+    const uint32_t q = pos[i];
+    if (q >= PAIR_TERMS_MAX) break;                 // (pos ascends with i)
+    const double v = p[m + 1 + i];
+    if (v == 0.0) continue;
+    // pair (a, b), a < b: the pairs with first index < a number a (2m - a - 1) / 2
+    auto first = [m](int64_t a) { return a * (2 * m - a - 1) / 2; };
+    const double h = (double)(2 * m - 1);
+    int64_t a = (int64_t)((h - sqrt(h * h - 8.0 * (double)i)) / 2.0);
+    if (a < 0) a = 0;
+    while (a > 0 && first(a) > i) a--;
+    while (a + 1 < m && first(a + 1) <= i) a++;
+    terms[q] = PairTerm{(uint32_t)a, (uint32_t)(a + 1 + (i - first(a))), v};
+  }
+}
+
 struct Work {
   DevBuf<double> theta, w, lossterm, g, red, scalars, gathered, blockmax;
   DevBuf<unsigned long long> G, H;     // H: forward-code tables of the matrix-free pass
@@ -1687,7 +1735,6 @@ template <> const double *csc_val<double>(const Matrix &M) { return M.cval_f64.p
 inline unsigned warp_grid(int64_t items, int threads) { return (unsigned)((items * 32 + threads - 1) / threads); }
 
 // the non-zero pair coefficients of a host theta, in coefficient order; empty optional = too many (dense theta)
-constexpr int64_t PAIR_TERMS_MAX = 8192;
 struct PairTerms {
   bool sparse = false;
   DevBuf<PairTerm> dev;
@@ -1720,7 +1767,7 @@ void launch_rows(const Matrix &M, const double *theta, int cooc, const double cw
   const bool sparse = cooc && T && T->sparse;
   KL_LAUNCH((rows_kernel<VT, MODE>), warp_grid(M.n, 256), 256, 0, M.rows(), M.col.p, csr_val<VT>(M), M.n, M.m,
             theta, sparse ? 2 : cooc, M.labels.p, cw ? cw[0] : 1.0, cw ? cw[1] : 1.0, inv_n, out, lossterm, st,
-            sparse ? T->dev.p : (const PairTerm *)nullptr, sparse ? T->n : 0);
+            sparse ? T->dev.p : (const PairTerm *)nullptr, sparse ? T->n : 0, (const int *)nullptr);
 }
 
 // fixed-point scales: sum_i |w_i v_ic| <= max(cw) * max|v| for a column, <= max(cw) for the bias, each kept below
@@ -1898,6 +1945,56 @@ void launch_pass_tail(const Matrix &M, Work &wk, PgState *st, int64_t n, int64_t
   wk.F = nullptr;
 }
 
+// pair coefficients of the gradient from the weights wk.w into wk.g[m + 1, Dim) (m > 1; the CSC view exists)
+template <typename VT>
+void launch_pairs_gradient(const Matrix &M, Work &wk) {
+  const int ntile = (int)((M.m + PAIR_T - 1) / PAIR_T);
+  const size_t smem = (size_t)PAIR_CH * PAIR_T * sizeof(double) + (size_t)8 * PAIR_CH * (sizeof(double) + sizeof(unsigned short));
+  KL_CUDA(cudaFuncSetAttribute(pairs_gradient<VT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  KL_LAUNCH((pairs_gradient<VT>), (unsigned)((int64_t)ntile * (ntile + 1) / 2), 256, smem, M.colptr.p, M.crow.p,
+            csc_val<VT>(M), M.m, M.n, ntile, wk.w.p, wk.g.p);
+}
+
+// pair mode's solver scratch: the non-zero flags of the pair coefficients, their scan, the scan's workspace, the
+// term list and its length
+struct PairScratch {
+  DevBuf<uint32_t> flags, pos;
+  DevBuf<int64_t> tiles;
+  DevBuf<PairTerm> terms;
+  DevBuf<int> count;
+  void alloc(int64_t npairs) {
+    flags.alloc((size_t)(npairs > 0 ? npairs : 1));
+    pos.alloc((size_t)npairs + 1);
+    tiles.alloc((size_t)exclusive_scan_workspace(npairs));
+    terms.alloc((size_t)PAIR_TERMS_MAX);
+    count.alloc(1);
+    count.zero();                 // (no pair coefficients at m <= 1: the list stays empty)
+  }
+};
+
+// One pass of the pair-mode solver at the point p (ntheta = Dim coefficients, on the device): the term list of p, then
+// the kernels and the order of kmerlr_gradient with cooccurrence = 1 -- rows_kernel (w and the loss terms), and with
+// scatter the fixed-point single-feature words of G (scatter_w) and the fp64 pair gradient in wk.g (pairs_gradient).
+// The same launches whatever the number of terms, and no host round trip.
+template <typename VT>
+void launch_pair_pass(Matrix &M, Work &wk, PairScratch &ps, const double *p, int64_t ntheta, const double cw[2],
+                      const PgState *st, int scatter) {
+  const int64_t m1 = M.m + 1, npairs = ntheta - m1;
+  if (npairs > 0) {
+    const unsigned grid = (unsigned)std::min<int64_t>((npairs + 255) / 256, 65535);
+    KL_LAUNCH(pair_nz_flags, grid, 256, 0, st, p, m1, npairs, ps.flags.p);
+    exclusive_scan_u32_async(ps.flags.p, ps.pos.p, npairs, ps.tiles.p);
+    KL_LAUNCH(pair_terms_emit, grid, 256, 0, st, p, M.m, ps.pos.p, npairs, ps.terms.p, ps.count.p);
+  }
+  KL_LAUNCH((rows_kernel<VT, 2, true>), warp_grid(M.n, 256), 256, 0, M.rows(), M.col.p, csr_val<VT>(M), M.n, M.m, p, 1,
+            M.labels.p, cw[0], cw[1], 1.0 / (double)M.n_global, wk.w.p, wk.lossterm.p, st, ps.terms.p, 0, ps.count.p);
+  if (!scatter) return;
+  KL_CUDA(cudaMemsetAsync(wk.G.p, 0, (size_t)m1 * sizeof(unsigned long long), ctx().stream));
+  KL_LAUNCH((scatter_w<VT>), warp_grid(M.n, 256), 256, 0, M.rows(), M.col.p, csr_val<VT>(M), M.n, wk.w.p, wk.scale,
+            wk.scale0, wk.G.p);
+  if (M.m > 1) launch_pairs_gradient<VT>(M, wk);
+}
+
 void check_theta(const Matrix &M, int64_t ntheta, int cooc) {
   if (cooc) KL_INVARIANT(ntheta == kmerlr_coeff_dim(M.m));
   else KL_INVARIANT(ntheta == M.m + 1);
@@ -1958,11 +2055,7 @@ void gradient(Matrix &M, const double *theta, int64_t ntheta, const double cw[2]
                   wk.scale, wk.scale0, wk.G.p);
       if (M.sharded) comm_allreduce_sum_i64((int64_t *)wk.G.p, M.m + 1);
       if (M.m > 1) {
-        const int ntile = (int)((M.m + PAIR_T - 1) / PAIR_T);
-        const size_t smem = (size_t)PAIR_CH * PAIR_T * sizeof(double) + (size_t)8 * PAIR_CH * (sizeof(double) + sizeof(unsigned short));
-        KL_CUDA(cudaFuncSetAttribute(pairs_gradient<VT>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        KL_LAUNCH((pairs_gradient<VT>), (unsigned)((int64_t)ntile * (ntile + 1) / 2), 256, smem, M.colptr.p, M.crow.p,
-                  csc_val<VT>(M), M.m, M.n, ntile, wk.w.p, wk.g.p);
+        launch_pairs_gradient<VT>(M, wk);
         if (M.sharded) {
           // pair entries: every rank sums the per-rank values in rank order
           comm_allgather_f64(wk.g.p, wk.gathered.p, ntheta);
@@ -2010,14 +2103,17 @@ double loss(Matrix &M, const double *theta, int64_t ntheta, const double cw[2], 
 }
 
 // the body of proxgrad and proxgrad_accel: they differ in the kernels' ACCEL instantiation and in y and the
-// accelerated state, which travel with theta and the iteration state (y == nullptr: ISTA)
+// accelerated state, which travel with theta and the iteration state (y == nullptr: ISTA).  pairs: theta has all
+// Dim = kmerlr_coeff_dim(m) coefficients of pair mode (proxgrad_pairs*): the pair pass, the step of the pair-expanded
+// rows, the L1 term over every coefficient and the prox step over both gradients
 static void proxgrad_run(Matrix &M, double *theta, double *y, double *t_acc, int64_t ntheta, const double cw[2],
                          double lambda, double l2, double step_factor, double epsilon, double epsilon_loss,
-                         int64_t max_iter, double hook[2], int64_t *iters, double *delta, int64_t *restarts) {
+                         int64_t max_iter, double hook[2], int64_t *iters, double *delta, int64_t *restarts,
+                         bool pairs = false) {
   const bool accel = y != nullptr;
-  Trace tr(accel ? "proxgrad_accel" : "proxgrad");
+  Trace tr(pairs ? (accel ? "proxgrad_pairs_accel" : "proxgrad_pairs") : (accel ? "proxgrad_accel" : "proxgrad"));
   // estimate_step_size (kmerLr_estimator_proximal.go:54-76)
-  double L = 0.25 * (matrix_maxsq(M) + 1.0) + l2 / (double)M.n_global;
+  double L = 0.25 * ((pairs ? matrix_maxsq_pairs(M) : matrix_maxsq(M)) + 1.0) + l2 / (double)M.n_global;
   double step = 1.0 / (2.0 * L + std::fmin(2.0 * l2, L)) * step_factor;
   Work wk; alloc_work(M, ntheta, wk);
   set_scale(M, wk, cw);
@@ -2044,7 +2140,10 @@ static void proxgrad_run(Matrix &M, double *theta, double *y, double *t_acc, int
   const double inv_n = 1.0 / (double)M.n_global;
   // reduced matrices: long batches between host round trips.  The choice of the path uses quantities that are
   // the same on every rank (a rank with an empty shard must issue the same collectives as the others)
-  const bool small = ntheta <= SMALL_MAX_THETA && !use_implicit(M);
+  // (never in pair mode: the reduced-matrix kernels know no pair terms)
+  const bool small = !pairs && ntheta <= SMALL_MAX_THETA && !use_implicit(M);
+  PairScratch ps;
+  if (pairs) { ensure_csc(M); ps.alloc(ntheta - (M.m + 1)); }
   KL_INVARIANT(!accel || !M.sharded);
   // the accelerated step on the full feature space: theta', the prox step's block partials and its decision
   DevBuf<double> xnew, accel_part;
@@ -2217,9 +2316,11 @@ static void proxgrad_run(Matrix &M, double *theta, double *y, double *t_acc, int
       }
       dispatch_vt(M, [&](auto *tag) {
         using VT = typename std::remove_pointer<decltype(tag)>::type;
-        launch_fused<VT>(M, wk, cw, st.p, scatter);
-        // columns, loss and L1 partials; one GPU: the loss sum and the hook in the same launch
-        launch_pass_tail(M, wk, st.p, M.n, M.m + 1, lambda, M.sharded ? 0 : 1, epsilon_loss);
+        if (pairs) launch_pair_pass<VT>(M, wk, ps, wk.theta.p, ntheta, cw, st.p, scatter);
+        else launch_fused<VT>(M, wk, cw, st.p, scatter);
+        // columns, loss and L1 partials (of every coefficient: ntheta is m + 1 outside pair mode); one GPU: the loss
+        // sum and the hook in the same launch
+        launch_pass_tail(M, wk, st.p, M.n, ntheta, lambda, M.sharded ? 0 : 1, epsilon_loss);
         if (M.sharded) {
           // ONE collective per iteration: gradient words + the loss sums of the ranks
           unsigned long long *slots = wk.G.p + M.m + 1;
@@ -2231,13 +2332,23 @@ static void proxgrad_run(Matrix &M, double *theta, double *y, double *t_acc, int
         }
         // the loss-only pass (number max_iter) follows the last prox step: the state is stopped (done != 0) by then
         if (scatter && accel) {
-          KL_LAUNCH(prox_accel, PROX_BLOCKS, 256, 0, st.p, wk.theta.p, wk.theta.p + ntheta, xnew.p, wk.G.p, wk.inv_scale,
-                    wk.inv_scale0, ntheta, step, lambda, accel_part.p, epsilon, (long long)max_iter, decision.p,
-                    wk.tickets.p + 2);
+          if (pairs)
+            KL_LAUNCH(prox_accel<true>, PROX_BLOCKS, 256, 0, st.p, wk.theta.p, wk.theta.p + ntheta, xnew.p, wk.G.p,
+                      wk.inv_scale, wk.inv_scale0, ntheta, step, lambda, accel_part.p, epsilon, (long long)max_iter,
+                      decision.p, wk.tickets.p + 2, wk.g.p, M.m + 1);
+          else
+            KL_LAUNCH(prox_accel<>, PROX_BLOCKS, 256, 0, st.p, wk.theta.p, wk.theta.p + ntheta, xnew.p, wk.G.p,
+                      wk.inv_scale, wk.inv_scale0, ntheta, step, lambda, accel_part.p, epsilon, (long long)max_iter,
+                      decision.p, wk.tickets.p + 2, (const double *)nullptr, (int64_t)0);
           KL_LAUNCH(accel_momentum, PROX_BLOCKS, 256, 0, st.p, decision.p, wk.theta.p, wk.theta.p + ntheta, xnew.p, ntheta);
         } else if (scatter) {
-          KL_LAUNCH(prox_update, PROX_BLOCKS, 256, 0, st.p, wk.theta.p, wk.G.p, wk.inv_scale, wk.inv_scale0, ntheta, step, lambda,
-                    wk.blockmax.p, epsilon, (long long)max_iter, wk.tickets.p + 2);
+          if (pairs)
+            KL_LAUNCH(prox_update<true>, PROX_BLOCKS, 256, 0, st.p, wk.theta.p, wk.G.p, wk.inv_scale, wk.inv_scale0, ntheta,
+                      step, lambda, wk.blockmax.p, epsilon, (long long)max_iter, wk.tickets.p + 2, wk.g.p, M.m + 1);
+          else
+            KL_LAUNCH(prox_update<>, PROX_BLOCKS, 256, 0, st.p, wk.theta.p, wk.G.p, wk.inv_scale, wk.inv_scale0, ntheta,
+                      step, lambda, wk.blockmax.p, epsilon, (long long)max_iter, wk.tickets.p + 2,
+                      (const double *)nullptr, (int64_t)0);
         }
       });
     }
@@ -2308,6 +2419,39 @@ void proxgrad_accel_full(Matrix &M, double *theta, double *y, double *t, int64_t
   accel_check("proxgrad_accel_full", M, theta, y, t, ntheta, cw);
   proxgrad_run(M, theta, y, t, ntheta, cw, lambda, l2, step_factor, epsilon, epsilon_loss, max_iter, hook, iters, delta,
                restarts);
+}
+
+// the arguments the pair-mode entries refuse (`who` names the entry in the messages; y == t == nullptr: ISTA)
+static void pairs_check(const char *who, Matrix &M, const double *theta, const double *y, const double *t, bool accel,
+                        int64_t ntheta, const double cw[2]) {
+  const std::string w(who);
+  KL_REQUIRE(!M.sharded, w + ": sharded matrices are not supported (one GPU)");
+  KL_REQUIRE(theta && cw && (!accel || (y && t)),
+             w + (accel ? ": null argument (theta, y, t and class_w are required)" : ": null argument (theta and class_w are required)"));
+  if (accel) KL_REQUIRE(std::isfinite(*t) && *t >= 1.0, w + ": the momentum t must be finite and >= 1 (1 = fresh start)");
+  KL_REQUIRE(ntheta == kmerlr_coeff_dim(M.m),
+             w + ": ntheta must be kmerlr_coeff_dim(m) = " + std::to_string(kmerlr_coeff_dim(M.m)) + " (every pair coefficient)");
+  KL_REQUIRE(ntheta - (M.m + 1) < ((int64_t)1 << 32), w + ": more than 2^32 pair coefficients");
+  KL_REQUIRE(M.has_labels, w + ": the matrix has no labels (kmerlr_matrix_set_labels)");
+  KL_REQUIRE(M.n_global > 0, w + ": empty data set");
+}
+
+void proxgrad_pairs(Matrix &M, double *theta, int64_t ntheta, const double cw[2], double lambda, double l2,
+                    double step_factor, double epsilon, double epsilon_loss, int64_t max_iter, double hook[2],
+                    int64_t *iters, double *delta) {
+  require_ready();
+  pairs_check("proxgrad_pairs", M, theta, nullptr, nullptr, false, ntheta, cw);
+  proxgrad_run(M, theta, nullptr, nullptr, ntheta, cw, lambda, l2, step_factor, epsilon, epsilon_loss, max_iter, hook,
+               iters, delta, nullptr, true);
+}
+
+void proxgrad_pairs_accel(Matrix &M, double *theta, double *y, double *t, int64_t ntheta, const double cw[2],
+                          double lambda, double l2, double step_factor, double epsilon, double epsilon_loss,
+                          int64_t max_iter, double hook[2], int64_t *iters, double *delta, int64_t *restarts) {
+  require_ready();
+  pairs_check("proxgrad_pairs_accel", M, theta, y, t, true, ntheta, cw);
+  proxgrad_run(M, theta, y, t, ntheta, cw, lambda, l2, step_factor, epsilon, epsilon_loss, max_iter, hook, iters, delta,
+               restarts, true);
 }
 
 }  // namespace kl

@@ -216,6 +216,38 @@ __global__ void row_sqnorm_max(const Rows R, const VT *__restrict__ val, int64_t
   if (lane == 0) atomicMax(out, (unsigned long long)__double_as_longlong(s));
 }
 
+// max_i ||x~_i||^2 of the pair-expanded rows x~ = (v_j)_j u (v_a v_b)_{a<b}: ||x~||^2 = S2 + (S2^2 - S4) / 2 with
+// S2 = sum v^2 and S4 = sum v^4 over the row, one warp per row.  Integer values (u32 counts, binarized rows) whose S2 is
+// below 2^32 take exact 64-bit integer sums (then S2^2 < 2^64), rounded to a double once: the bits of the explicit
+// expansion's row_sqnorm_max whenever its sums are exact (below 2^53).  Real values, and larger integer rows, in fp64
+// (S2^2 is rounded before the subtraction, so that a row of one entry gives S2 exactly).
+template <typename VT>
+__global__ void row_sqnorm_pairs_max(const Rows R, const VT *__restrict__ val, int64_t n, unsigned long long *__restrict__ out) {
+  int64_t row = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (row >= n) return;
+  unsigned lane = lane_id();
+  int64_t a, b;
+  R.range(row, a, b);
+  constexpr bool INT = std::is_same<VT, uint32_t>::value;
+  double d2 = 0.0, d4 = 0.0;
+  unsigned long long i2 = 0ull, i4 = 0ull;
+  for (int64_t p = a + lane; p < b; p += 32) {
+    const double v = val ? (double)val[p] : 1.0, v2 = v * v;
+    d2 += v2; d4 += v2 * v2;
+    if (INT) { const unsigned long long u = val ? (unsigned long long)val[p] : 1ull, u2 = u * u; i2 += u2; i4 += u2 * u2; }
+  }
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) {
+    d2 += __shfl_xor_sync(0xffffffffu, d2, o); d4 += __shfl_xor_sync(0xffffffffu, d4, o);
+    i2 += __shfl_xor_sync(0xffffffffu, i2, o); i4 += __shfl_xor_sync(0xffffffffu, i4, o);
+  }
+  if (lane != 0) return;
+  double s;
+  if (INT && d2 < 4294967296.0) s = (double)(i2 + (i2 * i2 - i4) / 2ull);   // (v < 2^16 everywhere: no product wraps)
+  else s = d2 + 0.5 * (__dmul_rn(d2, d2) - d4);
+  atomicMax(out, (unsigned long long)__double_as_longlong(s));
+}
+
 template <typename VT>
 __global__ void abs_max(const VT *__restrict__ val, int64_t nnz, unsigned long long *__restrict__ out) {
   double mx = 0.0;
@@ -915,6 +947,25 @@ static void ensure_stats(Matrix &M) {
 double matrix_maxsq(Matrix &M) {
   ensure_stats(M);
   return M.maxsq;
+}
+
+double matrix_maxsq_pairs(Matrix &M) {
+  KL_INVARIANT(!M.sharded);
+  if (M.has_maxsq_pairs) return M.maxsq_pairs;
+  matrix_compact(M);
+  DevBuf<unsigned long long> d(1);
+  d.zero();
+  if (M.n > 0) {
+    unsigned wgrid = (unsigned)((M.n * 32 + 127) / 128);
+    if (M.vt == VAL_F64) KL_LAUNCH((row_sqnorm_pairs_max<double>), wgrid, 128, 0, M.rows(), M.val_f64.p, M.n, d.p);
+    else KL_LAUNCH((row_sqnorm_pairs_max<uint32_t>), wgrid, 128, 0, M.rows(), M.vt == VAL_U32 ? M.val_u32.p : nullptr, M.n, d.p);
+  }
+  unsigned long long bits = 0;
+  d.download(&bits, 1);
+  sync_stream();
+  memcpy(&M.maxsq_pairs, &bits, sizeof(double));
+  M.has_maxsq_pairs = true;
+  return M.maxsq_pairs;
 }
 
 double matrix_vmax(Matrix &M) {

@@ -99,18 +99,32 @@ __global__ void scan_tiles(const TIn *__restrict__ in, int64_t n, const int64_t 
   if (blockIdx.x == 0 && threadIdx.x == 0) out[n] = (TOut)tile_off[nt];
 }
 
+int64_t tile_count(int64_t n) {
+  const int64_t nt = (n + SCAN_TILE - 1) / SCAN_TILE;
+  return nt == 0 ? 1 : nt;
+}
+
+template <typename TIn, typename TOut>
+void scan_launch(const TIn *in, TOut *out, int64_t n, int64_t *tiles) {
+  const int64_t nt = tile_count(n);
+  KL_LAUNCH((scan_tile_sums<TIn>), (unsigned)nt, SCAN_THREADS, 0, in, n, tiles);
+  KL_LAUNCH(scan_tile_offsets, 1, 1024, 0, tiles, nt);
+  KL_LAUNCH((scan_tiles<TIn, TOut>), (unsigned)nt, SCAN_THREADS, 0, in, n, tiles, out, nt);
+}
+
 template <typename TIn, typename TOut>
 void scan_impl(const TIn *in, TOut *out, int64_t n) {
-  int64_t nt = (n + SCAN_TILE - 1) / SCAN_TILE;
-  if (nt == 0) nt = 1;
-  DevBuf<int64_t> tiles((size_t)nt + 1);
-  KL_LAUNCH((scan_tile_sums<TIn>), (unsigned)nt, SCAN_THREADS, 0, in, n, tiles.p);
-  KL_LAUNCH(scan_tile_offsets, 1, 1024, 0, tiles.p, nt);
-  KL_LAUNCH((scan_tiles<TIn, TOut>), (unsigned)nt, SCAN_THREADS, 0, in, n, tiles.p, out, nt);
+  DevBuf<int64_t> tiles((size_t)tile_count(n) + 1);
+  scan_launch(in, out, n, tiles.p);
   sync_stream();  // tiles is freed on return
 }
 
 }  // namespace
+
+int64_t exclusive_scan_workspace(int64_t n) { return tile_count(n) + 1; }
+void exclusive_scan_u32_async(const uint32_t *in, uint32_t *out, int64_t n, int64_t *workspace) {
+  scan_launch<uint32_t, uint32_t>(in, out, n, workspace);
+}
 
 void exclusive_scan_i64(const int64_t *in, int64_t *out, int64_t n) { scan_impl<int64_t, int64_t>(in, out, n); }
 void exclusive_scan_u32_to_i64(const uint32_t *in, int64_t *out, int64_t n) { scan_impl<uint32_t, int64_t>(in, out, n); }
